@@ -2,7 +2,7 @@
 """Benchmark of the AdaptivePnP_SCI hot path on B200 - headline: two-stage online-adaptive ADMM reconstruction,
 512x512x8 Bayer, FastDVDnet (BASELINE.json configs[3]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5] [--dump-outputs DIR]
 
 Contract (see the task statement): W untimed warm-up steps, exactly K timed steps bracketed by a barrier +
 torch.cuda.synchronize() on both sides, CUDA-event timing, max over ranks, rank 0 prints ONE JSON line.
@@ -367,6 +367,35 @@ def hbm_kernel_table(H, W, B, dev, pk):
     return rows
 
 
+# what the timed call returns, in order, per configuration (non-array members of the returned tuple are not named):
+# config 1 the stage-1 Bayer cube [H,W,B]; config 2 the gray denoiser output and theta [H,W,B]; configs 3-5 the planar device
+# tensors xhat [B,3,H,W] and theta [B,H,W] (config 5: rank 0's row strip)
+OUTPUT_NAMES = {1: ("x_bayer",), 2: ("xhat", "theta"), 3: ("xhat", "theta"), 4: ("xhat", "theta"), 5: ("xhat", "theta")}
+DUMP_LIMIT_BYTES = 63 * 1024 * 1024          # array data; the .npy headers stay well inside the last of 64 MB
+
+
+def dump_outputs(d, names, out):
+    """DIR/<name>.npy of every named output of one step.  Above 63 MB of data in all, every array is replaced by the same
+    fixed strided sample of its flattened elements (every s-th, s = ceil(total / 63 MB)), so two runs stay comparable."""
+    arrays = []
+    for name, a in zip(names, out):
+        if isinstance(a, np.ndarray):
+            a = torch.from_numpy(a)
+        arrays.append((name, a.detach()))
+    total = sum(a.numel() * (8 if a.dtype == torch.float64 else 4) for _, a in arrays)
+    stride = -(-total // DUMP_LIMIT_BYTES)
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays:
+        if a.dtype != torch.float64:
+            a = a.float()
+        a = a.contiguous()
+        if stride > 1:
+            a = a.view(-1)[::stride]
+        np.save(os.path.join(d, name + ".npy"), a.cpu().numpy())
+        sys.stderr.write("bench: %s/%s.npy %s%s\n" % (d, name, tuple(a.shape),
+                                                         " (every %d-th element)" % stride if stride > 1 else ""))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -377,7 +406,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-eager", action="store_true")
     ap.add_argument("--no-delta-psnr", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, for output-by-output comparison "
+                         "of two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -524,6 +558,8 @@ def main():
         step_device()
     clocks = ClockSampler(local_rank) if rank == 0 else None
     ms, launches, out = timed(step_device, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, OUTPUT_NAMES[c], out)
     if clocks is not None and world == 1 and ms < 1000.0:
         # a timed region shorter than nvidia-smi's start-up (config 1: a few ms per step) would end without a sample: keep the
         # SAME step running under the sampler for about a second more (untimed) so that the line still carries clocks under load
