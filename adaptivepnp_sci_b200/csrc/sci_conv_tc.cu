@@ -1274,6 +1274,10 @@ int conv_fwd_tc_launch(const sci_conv_desc* d, void* stream) {
     }
     const int grid = min(p.num_tiles, SCI_NUM_SMS);
     p.pdl = (d->pdl && env_int("SCI_CONV_PDL", 1)) ? 1 : 0;
+    if (env_int("SCI_CONV_VERBOSE", 0))
+        fprintf(stderr, "conv v1 plan: %dx%d Cin %d -> %d stride %d half %d ps %d | tps %d stages %d lo_chunk0 %d ks_last %d wsplit %d "
+                "emit_lo %d pdl %d tiles %d\n", d->H, d->W, d->Cin, d->Cout, d->stride, (int)half, p.ps, p.tps, p.stages, p.lo_chunk0,
+                p.ks_last, p.wsplit, p.emit_lo, p.pdl, p.num_tiles);
     if (p.pdl) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = sci_stream(stream);
@@ -1478,11 +1482,11 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     }
     const int grid = min(p.num_tiles, SCI_NUM_SMS);
     const int threads = 128 + 128 * epi_wg;
+    p.pdl = (d->pdl && env_int("SCI_CONV_PDL", 1)) ? 1 : 0;
     if (env_int("SCI_CONV_VERBOSE", 0))
         fprintf(stderr, "conv v2 plan: %dx%d Cin %d -> %d cols (+%d) half %d ps %d mode %d | resident %d stages %d R %d stack %d epi_wg %d out_bufs %d "
-                "rb %d/%d smem %zu KB tiles %d\n", d->H, d->W, d->Cin, ncols, col0, (int)half, p.ps, mode, p.resident, p.stages, p.R, p.stack,
-                epi_wg, p.out_bufs, rb_in, rb_out, smem / 1024, p.num_tiles);
-    p.pdl = (d->pdl && env_int("SCI_CONV_PDL", 1)) ? 1 : 0;
+                "rb %d/%d smem %zu KB tiles %d split %d ks_last %d pdl %d\n", d->H, d->W, d->Cin, ncols, col0, (int)half, p.ps, mode, p.resident,
+                p.stages, p.R, p.stack, epi_wg, p.out_bufs, rb_in, rb_out, smem / 1024, p.num_tiles, p.split, p.ks_last, p.pdl);
     if (p.pdl) {
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(grid); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = sci_stream(stream);
@@ -1662,6 +1666,9 @@ int conv_wgrad_tc_launch(const sci_wgrad_desc* d, void* stream) {
     }
     const int groups = 3 * p.m_tiles;
     const int gx = max(1, min(p.num_tiles, (2 * SCI_NUM_SMS) / groups));
+    if (env_int("SCI_CONV_VERBOSE", 0))
+        fprintf(stderr, "wgrad v1 plan: %dx%d Cin %d Cout %d stride %d | m_tiles %d grid %d groups %d tiles %d\n", d->H, d->W, d->Cin, d->Cout,
+                d->stride, p.m_tiles, gx, groups, p.num_tiles);
     conv_wgrad_tc_kernel<<<dim3(gx, groups), TC_THREADS, smem, sci_stream(stream)>>>(tmZ, tmX, p);
     SCI_CHECK_LAUNCH("conv tc wgrad");
     return SCI_OK;
@@ -1865,6 +1872,9 @@ int conv_wgrad2_tc_launch(const sci_wgrad_desc* d, void* stream) {
     }
     const int groups = 3 * p.m_tiles;
     const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS / groups));
+    if (env_int("SCI_CONV_VERBOSE", 0))
+        fprintf(stderr, "wgrad v2 plan: %dx%d Cin %d Cout %d stride %d | swap %d fuse %d m_tiles %d accs %d stages %d grid %d groups %d tiles %d\n",
+                d->H, d->W, d->Cin, d->Cout, d->stride, p.swap, p.fuse, p.m_tiles, p.accs, p.stages, gx, groups, p.num_tiles);
     conv_wgrad2_tc_kernel<<<dim3(gx, groups), TC_THREADS, smem, sci_stream(stream)>>>(tmZ, tmX, p);
     SCI_CHECK_LAUNCH("conv tc wgrad v2");
     return SCI_OK;
@@ -2049,6 +2059,9 @@ int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream) {
         if (dev >= 0 && dev < 64) attr_set[dev] = true;
     }
     const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS));
+    if (env_int("SCI_CONV_VERBOSE", 0))
+        fprintf(stderr, "wgrad v3 plan: %dx%d Cin %d Cout %d stride 1 | p_is_dz %d cp %d cq %d stages %d grid %d tiles %d\n", d->H, d->W,
+                d->Cin, d->Cout, p.p_is_dz, cp, cq, p.stages, gx, p.num_tiles);
     conv_wgrad3_tc_kernel<<<gx, TC_THREADS, smem, sci_stream(stream)>>>(tmP, tmQ, p);
     SCI_CHECK_LAUNCH("conv tc wgrad v3");
     return SCI_OK;
