@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <atomic>
+
 #include "sci_b200.h"
 
 #define SCI_NUM_SMS 148   // B200: 2 dies x 74 SMs
@@ -24,6 +26,28 @@ static inline int sci_fail(int code, const char* what, cudaError_t e = cudaSucce
          if (e__ != cudaSuccess) return sci_fail(SCI_ELAUNCH, what, e__); } while (0)
 
 static inline cudaStream_t sci_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// Raises `kernel`'s dynamic shared-memory limit to `bytes` the first time it is launched on the current device.  Later
+// calls cost a cudaGetDevice and a scan of the few kernels seen so far: no driver call and no lock on the launch path.
+// Kernels beyond the table, and devices >= 64, simply set the attribute on every call.
+static inline cudaError_t sci_smem_limit(const void* kernel, int bytes) {
+    constexpr int SLOTS = 32;
+    static std::atomic<const void*> kernels[SLOTS];
+    static std::atomic<uint64_t> devices[SLOTS];       // bit d: the attribute is set on device d
+    int dev = 0;
+    cudaGetDevice(&dev);
+    const uint64_t bit = (dev >= 0 && dev < 64) ? 1ull << dev : 0;
+    int i = 0;
+    for (; i < SLOTS; ++i) {
+        const void* k = kernels[i].load(std::memory_order_acquire);
+        if (k == nullptr && kernels[i].compare_exchange_strong(k, kernel)) break;
+        if (k == kernel) break;
+    }
+    if (i < SLOTS && (devices[i].load(std::memory_order_acquire) & bit)) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess && i < SLOTS) devices[i].fetch_or(bit, std::memory_order_release);
+    return e;
+}
 
 static inline int sci_ceil_div(long a, long b) { return (int)((a + b - 1) / b); }
 

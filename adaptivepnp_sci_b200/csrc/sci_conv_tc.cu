@@ -14,7 +14,7 @@
 //     warps 4-7 = epilogue (tcgen05.ld -> scale/shift/ReLU/skip-add/PixelShuffle/TF32 round -> global).
 //   * pipelines: smem ring (full/empty mbarriers) between TMA and MMA; two TMEM accumulator stages
 //     (tmem_full/tmem_empty) between MMA and epilogue, so the epilogue of tile i overlaps the MMAs of i+1.
-// Weight-gradient kernel (conv_wgrad_tc_kernel): see the comment above its definition.
+// Weight-gradient kernels (conv_wgrad2_tc_kernel, conv_wgrad3_tc_kernel): see the comments above their definitions.
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include <stdlib.h>
@@ -126,7 +126,8 @@ __device__ __forceinline__ void tc_mma_elect(uint32_t d_tmem, uint64_t adesc, ui
 }
 // K-major SWIZZLE_128B descriptor split into its 32-bit halves: the low word carries the start address (>> 4) and
 // LBO = 16 B, the high word (SBO = 1024 B, version 1, layout SWIZZLE_128B) never changes.  Advancing an operand by whole
-// 16-byte units inside the tile is then ONE 32-bit add on the low word.
+// 16-byte units inside the tile is then ONE 32-bit add on the low word.  The base-offset field stays 0: measured on B200,
+// the swizzle XOR is taken from the ABSOLUTE shared-memory address bits, so an advanced descriptor reads what TMA wrote.
 constexpr uint32_t DESC_HI_K128 = 0x40004040u;
 // K-major SWIZZLE_64B (64-byte operand rows = 32 fp16 channels): SBO = 8 rows x 64 B = 512 B, layout type 4
 constexpr uint32_t DESC_HI_K64 = 0x80004020u;
@@ -433,7 +434,7 @@ constexpr int A2_STAGE = 17 * 1024;               // row box rounded up to the 1
 struct Fwd2Params {
     const float* scale; const float* shift; const float* residual; float* y;
     int N, H, W, Cin, Cout, relu, ps, round_tf32;
-    int tiles_w, num_tiles, k_chunks, stages, acc_stride, tmem_cols, resident, desc_mode, tma_store, out_bufs;
+    int tiles_w, num_tiles, k_chunks, stages, acc_stride, tmem_cols, resident, out_bufs;
     const float* planar_in1; float* planar_out;   // fused network output: out[n][c][h][w] = in1[n][c][h][w] - conv[c], c < 3
     int pdl;          // launched with programmatic stream serialization: see griddepcontrol below
     int col0, Ctot;   // this launch computes GEMM columns [col0, col0 + Cout) of a layer with Ctot columns (Cout = 256 layers run as two halves)
@@ -460,16 +461,6 @@ struct Fwd2Params {
     uint32_t desc_hi;
 };
 
-__device__ __forceinline__ uint64_t umma_desc_off(uint32_t saddr, int mode) {
-    // K-major SWIZZLE_128B descriptor whose start is advanced by whole 128-byte rows inside the 1024-byte swizzle
-    // period.  Measured on B200: the swizzle XOR is taken from the ABSOLUTE shared-memory address bits, so the plain
-    // descriptor (base-offset field 0) reads exactly what TMA wrote; setting the base-offset field to
-    // (start >> 7) & 7 (mode 1, kept for experiments) gives wrong results.
-    uint64_t d = umma_desc(saddr, 16, 1024);
-    if (mode == 1) d |= (uint64_t)((saddr >> 7) & 7u) << 49;
-    return d;
-}
-
 // Epilogue organisation (round 2).  The ncu source view of the full-resolution layers showed the four epilogue warps
 // - one per SM sub-partition - busy >90 % of the time at IPC 0.25 (407 instructions per 32-channel chunk, every one
 // waiting for its predecessor) while the MMA warp sat on the tmem_empty barrier: the 12->90 layer was bound by its
@@ -478,7 +469,7 @@ __device__ __forceinline__ uint64_t umma_desc_off(uint32_t saddr, int mode) {
 //     second group shares the quarters and takes every second (row, chunk) unit): two warps per scheduler hide each
 //     other's latencies;
 //   * MODE selects the epilogue at compile time (0 = TMA store, 1 = TMA store + skip-add, 2 = fused planar network
-//     output, 3 = direct stores) instead of run-time flags per element; scale / shift come from shared memory as float4;
+//     output, 4 = data gradient with the fused activation backward) instead of run-time flags per element; scale / shift come from shared memory as float4;
 //   * the planar mode fetches the in1 values of ALL its rows before it waits for the accumulator (the per-row prefetch
 //     left the HBM latency of those loads exposed: 46 % of the epilogue's samples in the 32->3 layer).
 //   * HALF: fp16 storage and operands (kind::f16, fp32 accumulation): the same 11-bit significand as TF32 - the products
@@ -802,7 +793,7 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             // operands from global memory are requested while the MMAs of this tile are still running
             float4 rr[8];
             float pin[PIN_ROWS][3];
-            if (!HALF && (MODE == 1 || MODE == 3)) {
+            if (!HALF && MODE == 1) {
 #pragma unroll
                 for (int j = 0; j < 8; ++j) rr[j] = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (p.residual && valid && g < units) {
@@ -1059,7 +1050,7 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                         continue;
                     }
                     unit(t, c0, v);
-                    if (MODE == 1 || MODE == 3) {
+                    if (MODE == 1) {
                         float4 rn[8];
 #pragma unroll
                         for (int j = 0; j < 8; ++j) rn[j] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1080,40 +1071,31 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
                         for (int j = 0; j < 32; ++j) v[j] = rna_tf32(v[j]);
                     }
-                    if (MODE == 3) {
-                        if (valid) {
-                            float* yp = p.y + out_offset(ho, c0);
-#pragma unroll
-                            for (int j = 0; j < 32; j += 4)
-                                *reinterpret_cast<float4*>(yp + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-                        }
-                    } else {
-                        // coalesced path: the warp's 32 pixels x 32 channels go through a 128B-swizzled 4 KB staging tile and
-                        // leave as ONE TMA store (box {32 ch, 32 px}; PixelShuffle = element stride 2 on the pixel axis of a map
-                        // over the up-sampled tensor); out-of-image pixels are clipped by TMA
-                        const uint32_t sbuf = sbuf0 + (p.out_bufs == 2 ? (st_cnt & 1) * tile_b : 0u);
-                        if (lane == 0) {
-                            if (p.out_bufs == 2) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-                            else                 asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                        }
-                        __syncwarp();
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4) {
-                            const uint32_t a = sbuf + (uint32_t)lane * 128u + (uint32_t)(((j >> 2) ^ (lane & 7)) << 4);
-                            asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v[j]), "f"(v[j + 1]), "f"(v[j + 2]), "f"(v[j + 3]) : "memory");
-                        }
-                        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                        __syncwarp();
-                        if (lane == 0) {
-                            const int cg = p.col0 + c0;
-                            int cx = cg, cw = wt * 128 + q * 32, chh = ho;
-                            if (p.ps) { const int qq = cg / Cq; cx = cg % Cq; cw = 2 * cw + (qq & 1); chh = 2 * ho + (qq >> 1); }
-                            asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
-                                         ::"l"(&tmY), "r"(sbuf), "r"(cx), "r"(cw), "r"(chh), "r"(n) : "memory");
-                            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                        }
-                        ++st_cnt;
+                    // coalesced path: the warp's 32 pixels x 32 channels go through a 128B-swizzled 4 KB staging tile and
+                    // leave as ONE TMA store (box {32 ch, 32 px}; PixelShuffle = element stride 2 on the pixel axis of a map
+                    // over the up-sampled tensor); out-of-image pixels are clipped by TMA
+                    const uint32_t sbuf = sbuf0 + (p.out_bufs == 2 ? (st_cnt & 1) * tile_b : 0u);
+                    if (lane == 0) {
+                        if (p.out_bufs == 2) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+                        else                 asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
                     }
+                    __syncwarp();
+#pragma unroll
+                    for (int j = 0; j < 32; j += 4) {
+                        const uint32_t a = sbuf + (uint32_t)lane * 128u + (uint32_t)(((j >> 2) ^ (lane & 7)) << 4);
+                        asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(a), "f"(v[j]), "f"(v[j + 1]), "f"(v[j + 2]), "f"(v[j + 3]) : "memory");
+                    }
+                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                    __syncwarp();
+                    if (lane == 0) {
+                        const int cg = p.col0 + c0;
+                        int cx = cg, cw = wt * 128 + q * 32, chh = ho;
+                        if (p.ps) { const int qq = cg / Cq; cx = cg % Cq; cw = 2 * cw + (qq & 1); chh = 2 * ho + (qq >> 1); }
+                        asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
+                                     ::"l"(&tmY), "r"(sbuf), "r"(cx), "r"(cw), "r"(chh), "r"(n) : "memory");
+                        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+                    }
+                    ++st_cnt;
                 }
             }
             }
@@ -1143,13 +1125,17 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 }
 
 // ---------------------------------------------------------------------------------------------------
-// host side: TMA descriptors through the driver entry point (no libcuda link dependency)
+// host side: TMA descriptors through the driver entry point (no libcuda link dependency), launches
 // ---------------------------------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-EncodeTiledFn get_encode_fn() {
+// cuTensorMapEncodeTiled of a rank-`rank` fp32 / fp16 tensor: dims, box and element strides innermost first, byte strides
+// of dims 1 .. rank-1.  `what` names the tensor in the error message.
+int encode_map(CUtensorMap* tm, const char* what, const void* base, bool half, int rank, const cuuint64_t* dims,
+               const cuuint64_t* strides, const cuuint32_t* box, const cuuint32_t* estr, CUtensorMapSwizzle swz,
+               CUtensorMapL2promotion l2 = CU_TENSOR_MAP_L2_PROMOTION_L2_256B) {
     static EncodeTiledFn fn = nullptr;
     if (!fn) {
         void* p = nullptr;
@@ -1158,48 +1144,62 @@ EncodeTiledFn get_encode_fn() {
             q == cudaDriverEntryPointSuccess)
             fn = reinterpret_cast<EncodeTiledFn>(p);
     }
-    return fn;
+    if (!fn) return sci_fail(SCI_ELAUNCH, "cuTensorMapEncodeTiled entry point not available");
+    const CUresult r = fn(tm, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank,
+                          const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, l2,
+                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        char msg[96];
+        snprintf(msg, sizeof(msg), "cuTensorMapEncodeTiled(%s) failed with CUresult %d", what, (int)r);
+        return sci_fail(SCI_ELAUNCH, msg);
+    }
+    return SCI_OK;
 }
 
-// NHWC activation tensor [N][H][W][C], box = {32 ch, TILE_W*stride, TILE_H*stride, 1} traversed with element stride `stride`
+// NHWC activation tensor [N][H][W][C], box = {32 ch, box_w*stride, box_h*stride, 1} traversed with element stride `stride`
 int make_act_map(CUtensorMap* tm, const float* x, int N, int H, int W, int C, int stride, int box_w, int box_h,
                  CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B, bool half = false, bool row64 = false) {
-    EncodeTiledFn fn = get_encode_fn();
-    if (!fn) return sci_fail(SCI_ELAUNCH, "cuTensorMapEncodeTiled entry point not available");
     const cuuint64_t esz = half ? 2 : 4;
     const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
     const cuuint64_t strides[3] = {(cuuint64_t)C * esz, (cuuint64_t)W * C * esz, (cuuint64_t)H * W * C * esz};
     const cuuint32_t box[4] = {(cuuint32_t)(row64 ? 32 : (half ? 64 : KCH)), (cuuint32_t)(box_w * stride), (cuuint32_t)(box_h * stride), 1};
     const cuuint32_t estr[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
-    CUresult r = fn(tm, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(x), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        char msg[96];
-        snprintf(msg, sizeof(msg), "cuTensorMapEncodeTiled(activations) failed with CUresult %d", (int)r);
-        return sci_fail(SCI_ELAUNCH, msg);
-    }
-    return SCI_OK;
+    return encode_map(tm, "activations", x, half, 4, dims, strides, box, estr, swz);
 }
 
 // packed weights [taps][Cout][Cin] (taps = 9, or 18 with the hi/remainder split), box = {32 ch, Cout, 1}
 int make_weight_map(CUtensorMap* tm, const float* w, int Cout, int Cin, int taps, int box_rows = 0, bool half = false,
                     bool row64 = false) {
-    EncodeTiledFn fn = get_encode_fn();
-    if (!fn) return sci_fail(SCI_ELAUNCH, "cuTensorMapEncodeTiled entry point not available");
     const cuuint64_t esz = half ? 2 : 4;
     const cuuint64_t dims[3] = {(cuuint64_t)Cin, (cuuint64_t)Cout, (cuuint64_t)taps};
     const cuuint64_t strides[2] = {(cuuint64_t)Cin * esz, (cuuint64_t)Cout * Cin * esz};
     const cuuint32_t box[3] = {(cuuint32_t)(row64 ? 32 : (half ? 64 : KCH)), (cuuint32_t)(box_rows ? box_rows : Cout), 1};
     const cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(tm, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(w), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, row64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        char msg[96];
-        snprintf(msg, sizeof(msg), "cuTensorMapEncodeTiled(weights) failed with CUresult %d", (int)r);
-        return sci_fail(SCI_ELAUNCH, msg);
+    return encode_map(tm, "weights", w, half, 3, dims, strides, box, estr,
+                      row64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B);
+}
+
+// Launches `kernel` with up to 220 KB of dynamic shared memory.  pdl: with programmatic stream serialization, so that
+// its prologue may overlap the tail of the previous kernel on the stream (the kernel waits with griddepcontrol.wait
+// before it reads that kernel's results).
+template <typename... Params, typename... Args>
+int launch(void (*kernel)(Params...), dim3 grid, int threads, size_t smem, void* stream, bool pdl, const char* what,
+           const Args&... args) {
+    cudaError_t e = sci_smem_limit((const void*)kernel, 220 * 1024);
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, what, e);
+    if (pdl) {
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = grid; cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = sci_stream(stream);
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        at[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = at; cfg.numAttrs = 1;
+        e = cudaLaunchKernelEx(&cfg, kernel, args...);
+    } else {
+        kernel<<<grid, threads, smem, sci_stream(stream)>>>(args...);
+        e = cudaGetLastError();
     }
-    return SCI_OK;
+    return e == cudaSuccess ? SCI_OK : sci_fail(SCI_ELAUNCH, what, e);
 }
 
 int next_pow2_cols(int c) { int v = 32; while (v < c) v <<= 1; return v; }
@@ -1209,10 +1209,24 @@ int env_int(const char* name, int dflt) {
     return v ? atoi(v) : dflt;
 }
 
+// bytes per operand row: fp16 tensors with 32 channels use 64-byte rows (SWIZZLE_64B); everything else one 128-byte row
+// per pixel and channel chunk
+int operand_row_bytes(const sci_conv_desc* d) {
+    return (d->half_io && d->Cin == 32 && env_int("SCI_CONV_SW64", 1)) ? 64 : 128;
+}
+
+// K steps (32 bytes: 8 fp32 / 16 fp16 channels each) of the LAST channel chunk that can hold non-zero channels when only
+// the first `used` of the Cin channels can: the zero-padded rest is not multiplied.  `used` must reach into the last chunk
+// to shorten it.
+int ks_last(int Cin, int used, int rb_in, int esz) {
+    const int kch = rb_in / esz, step = 32 / esz, rest = used - (Cin / kch - 1) * kch;
+    return rest <= 0 ? rb_in / 32 : min(rb_in / 32, (rest + step - 1) / step);
+}
+
 int conv_fwd_tc_launch(const sci_conv_desc* d, void* stream) {
     const bool half = d->half_io != 0;
     const int esz = half ? 2 : 4;
-    const int rb_in = (half && d->Cin == 32 && env_int("SCI_CONV_SW64", 1)) ? 64 : 128;
+    const int rb_in = operand_row_bytes(d);
     const int kch = rb_in / esz;
     if (d->Cin % kch != 0 || d->Cout % 16 != 0 || d->Cout > 256)
         return sci_fail(SCI_EUNSUPPORTED, "conv tc: needs Cin % 32 == 0 (fp16: % 64), Cout % 16 == 0, Cout <= 256");
@@ -1230,11 +1244,7 @@ int conv_fwd_tc_launch(const sci_conv_desc* d, void* stream) {
     p.wsplit = d->w_split ? 1 : 0;
     p.emit_lo = d->emit_lo ? 1 : 0;
     p.Cstore = (half && d->Cout_store) ? d->Cout_store : d->Cout;
-    {
-        const int step = half ? 16 : 8, used = (d->K_used > 0 && d->K_used <= d->Cin && !d->w_split) ? d->K_used : d->Cin;
-        p.ks_last = min(rb_in / 32, max(1, (used - (d->Cin / kch - 1) * kch + step - 1) / step));
-        if (used <= (d->Cin / kch - 1) * kch) p.ks_last = rb_in / 32;      // K_used must reach into the last chunk to shorten it
-    }
+    p.ks_last = ks_last(d->Cin, (d->K_used > 0 && d->K_used <= d->Cin && !d->w_split) ? d->K_used : d->Cin, rb_in, esz);
     if (p.emit_lo && (d->pixel_shuffle || d->residual || !d->round_tf32))
         return sci_fail(SCI_EUNSUPPORTED, "conv tc: emit_lo needs round_tf32 and no pixel_shuffle / residual");
     p.tiles_w = (p.Wo + TILE_W - 1) / TILE_W; p.tiles_h = (p.Ho + TILE_H - 1) / TILE_H;
@@ -1263,37 +1273,14 @@ int conv_fwd_tc_launch(const sci_conv_desc* d, void* stream) {
     rc = make_weight_map(&tmB, d->w, d->Cout, d->Cin, 9 * (1 + p.wsplit), 0, half, rb_in == 64);
     if (rc) return rc;
     const size_t smem = (size_t)p.stages * stage_bytes + 1024;
-    static bool attr_set[64][2] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev][half ? 1 : 0]) {
-        cudaError_t e = half ? cudaFuncSetAttribute(conv_fwd_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024)
-                             : cudaFuncSetAttribute(conv_fwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "conv tc: smem attribute", e);
-        if (dev >= 0 && dev < 64) attr_set[dev][half ? 1 : 0] = true;
-    }
     const int grid = min(p.num_tiles, SCI_NUM_SMS);
     p.pdl = (d->pdl && env_int("SCI_CONV_PDL", 1)) ? 1 : 0;
     if (env_int("SCI_CONV_VERBOSE", 0))
         fprintf(stderr, "conv v1 plan: %dx%d Cin %d -> %d stride %d half %d ps %d | tps %d stages %d lo_chunk0 %d ks_last %d wsplit %d "
                 "emit_lo %d pdl %d tiles %d\n", d->H, d->W, d->Cin, d->Cout, d->stride, (int)half, p.ps, p.tps, p.stages, p.lo_chunk0,
                 p.ks_last, p.wsplit, p.emit_lo, p.pdl, p.num_tiles);
-    if (p.pdl) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(grid); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = sci_stream(stream);
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        cudaError_t e = half ? cudaLaunchKernelEx(&cfg, conv_fwd_tc_kernel<true>, tmA, tmB, p)
-                             : cudaLaunchKernelEx(&cfg, conv_fwd_tc_kernel<false>, tmA, tmB, p);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "conv tc fwd (PDL launch)", e);
-        return SCI_OK;
-    }
-    if (half) conv_fwd_tc_kernel<true><<<grid, TC_THREADS, smem, sci_stream(stream)>>>(tmA, tmB, p);
-    else      conv_fwd_tc_kernel<false><<<grid, TC_THREADS, smem, sci_stream(stream)>>>(tmA, tmB, p);
-    SCI_CHECK_LAUNCH("conv tc fwd");
-    return SCI_OK;
+    return launch(half ? conv_fwd_tc_kernel<true> : conv_fwd_tc_kernel<false>, dim3(grid), TC_THREADS, smem, stream, p.pdl,
+                  "conv tc fwd", tmA, tmB, p);
 }
 
 
@@ -1310,8 +1297,7 @@ bool fwd2_eligible(const sci_conv_desc* d) {
 int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncols) {
     const bool half = d->half_io != 0;
     const int esz = half ? 2 : 4;
-    // fp16 tensors with 32 channels use 64-byte operand rows (SWIZZLE_64B); everything else one 128-byte row per pixel and chunk
-    const int rb_in = (half && d->Cin == 32 && env_int("SCI_CONV_SW64", 1)) ? 64 : 128;
+    const int rb_in = operand_row_bytes(d);
     const int kch = rb_in / esz;                     // channels per operand row
     if (d->Cin % kch != 0) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: Cin % 32 (fp32) / % 64 or == 32 (fp16)");
     if (((uintptr_t)d->x | (uintptr_t)d->w | (uintptr_t)d->y | (uintptr_t)d->residual) & 15)
@@ -1336,13 +1322,9 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     p.desc_hi = rb_in == 64 ? DESC_HI_K64 : DESC_HI_K128;
     const int a_stage = p.a_stage;
     const int b_bytes = p.Cout * rb_in;
-    p.tma_store = ((half || env_int("SCI_CONV_TMA_STORE", 1)) && !p.planar_out) ? 1 : 0;
+    const bool tma_store = !p.planar_out;            // every epilogue but the planar one leaves through TMA stores
     p.Cstore = cout_store;
-    {
-        const int step = half ? 16 : 8, used = (d->K_used > 0 && d->K_used <= d->Cin) ? d->K_used : d->Cin;
-        p.ks_last = min(rb_in / 32, max(1, (used - (p.k_chunks - 1) * kch + step - 1) / step));
-        if (used <= (p.k_chunks - 1) * kch) p.ks_last = rb_in / 32;
-    }
+    p.ks_last = ks_last(d->Cin, (d->K_used > 0 && d->K_used <= d->Cin) ? d->K_used : d->Cin, rb_in, esz);
     p.ucols = 32;
     if (half) {
         const int cq = p.ps ? d->Cout / 4 : ncols;             // columns that belong to one stored pixel row
@@ -1360,10 +1342,10 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
         p.ucols = 32;
         p.ks_last = 4;
     }
-    int mode = p.planar_out ? 2 : (!p.tma_store ? 3 : (d->residual ? 1 : 0));
+    int mode = p.planar_out ? 2 : (d->residual ? 1 : 0);
     p.mask_y = d->mask_y; p.col_s1 = d->col_s1; p.col_s2 = d->col_s2; p.mask_relu = d->mask_relu;
     if (d->mask_y) {
-        if (half || p.planar_out || !p.tma_store || (d->pixel_shuffle ? d->Cout / 4 : d->Cout) > 128 || (d->col_s2 && !d->col_s1))
+        if (half || p.planar_out || (d->pixel_shuffle ? d->Cout / 4 : d->Cout) > 128 || (d->col_s2 && !d->col_s1))
             return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: fused activation backward needs the fp32 TMA-store path and <= 128 stored channels");
         mode = 4;
     }
@@ -1380,16 +1362,16 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     const int epi_first = epi_env ? (epi_env == 1 ? 1 : 2) : ((half || p.k_chunks <= 1 || d->residual || d->mask_y) ? 2 : 1);
     for (epi_wg = epi_first; epi_wg >= 1; --epi_wg) {
         for (p.out_bufs = ((epi_wg == 2 || d->mask_y) ? 1 : 2); p.out_bufs >= 1; --p.out_bufs) {
-            out_stage = p.tma_store ? 4 * epi_wg * p.out_bufs * tile_b : 0;
+            out_stage = tma_store ? 4 * epi_wg * p.out_bufs * tile_b : 0;
             budget = total_budget - out_stage;
             p.resident = (w_bytes + 3 * a_stage <= budget) ? 1 : 0;
             const int sb = a_stage + (p.resident ? 0 : 3 * b_bytes);
             const int st = (budget - (p.resident ? w_bytes : 0)) / sb;
-            const bool would_be_resident = w_bytes + 3 * a_stage <= total_budget - (p.tma_store ? 4 * epi_wg * tile_b : 0);
+            const bool would_be_resident = w_bytes + 3 * a_stage <= total_budget - (tma_store ? 4 * epi_wg * tile_b : 0);
             if ((p.resident || !would_be_resident) && st >= 3) break;
             if (p.out_bufs == 1) break;
         }
-        const bool resident_with_one = w_bytes + 3 * a_stage <= total_budget - (p.tma_store ? 4 * tile_b : 0);
+        const bool resident_with_one = w_bytes + 3 * a_stage <= total_budget - (tma_store ? 4 * tile_b : 0);
         // fp16 chains: the MMAs are twice as fast, so the epilogue decides more often - two warpgroups even where that costs
         // the weights their residency (64->128 + PixelShuffle: 0.215 ms resident with one group, 0.135 ms streamed with two)
         if (epi_wg == 1 || epi_env == 2 || half || p.resident || !resident_with_one) break;
@@ -1425,29 +1407,18 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     p.tiles_h = (p.H + p.R - 1) / p.R;
     p.num_tiles = p.tiles_w * p.tiles_h * p.N;
     p.tmem_cols = next_pow2_cols(2 * p.R * p.acc_stride);
-    p.desc_mode = env_int("SCI_CONV_DESC_MODE", 0);
     p.dbg = env_int("SCI_CONV_DBG", 0);
     CUtensorMap tmA, tmB;
-    // activation map with a {32 ch, 130 px, 1 row, 1 image} box
-    {
-        EncodeTiledFn fn = get_encode_fn();
-        if (!fn) return sci_fail(SCI_ELAUNCH, "cuTensorMapEncodeTiled entry point not available");
-        // fp16: the channel extent is the STORED one; a box that sticks out of it (e.g. channels 64..127 of a 96-channel tensor)
-        // is zero-filled by TMA, matching the zero rows of the packed weights
-        const cuuint64_t dims[4] = {(cuuint64_t)cin_store, (cuuint64_t)d->W, (cuuint64_t)d->H, (cuuint64_t)d->N};
-        const cuuint64_t strides[3] = {(cuuint64_t)cin_store * esz, (cuuint64_t)d->W * cin_store * esz, (cuuint64_t)d->H * d->W * cin_store * esz};
-        const cuuint32_t box[4] = {(cuuint32_t)kch, ROW_PX, 1, 1};
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = fn(&tmA, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(d->x), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, rb_in == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return sci_fail(SCI_ELAUNCH, "cuTensorMapEncodeTiled(row box) failed");
-    }
-    int rc = make_weight_map(&tmB, d->w, d->Cout, d->Cin, 9, ncols, half, rb_in == 64);
+    // activation map with a {kch ch, 130 px, 1 row, 1 image} box.  fp16: the channel extent is the STORED one; a box that
+    // sticks out of it (e.g. channels 64..127 of a 96-channel tensor) is zero-filled by TMA, matching the zero rows of the
+    // packed weights
+    int rc = make_act_map(&tmA, d->x, d->N, d->H, d->W, cin_store, 1, ROW_PX, 1,
+                          rb_in == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, half, rb_in == 64);
+    if (rc) return rc;
+    rc = make_weight_map(&tmB, d->w, d->Cout, d->Cin, 9, ncols, half, rb_in == 64);
     if (rc) return rc;
     CUtensorMap tmY = tmA;
-    if (p.tma_store) {
-        EncodeTiledFn fn = get_encode_fn();
+    if (tma_store) {
         // plain layers: [N][H][W][Cout], box {32 ch, 32 px}.  PixelShuffle layers: the map covers the up-sampled tensor
         // [N][2H][2W][Cout/4]; the 32 pixels of a warp land on every second column (element stride 2).
         const int ps = d->pixel_shuffle ? 1 : 0;
@@ -1456,30 +1427,23 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
         const cuuint64_t strides[3] = {oc * esz, ow * oc * esz, oh * ow * oc * esz};
         const cuuint32_t box[4] = {(cuuint32_t)(rb_out / esz), (cuuint32_t)(32 << ps), 1, 1};
         const cuuint32_t estr[4] = {1, (cuuint32_t)(1 << ps), 1, 1};
-        CUresult r = fn(&tmY, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, d->y, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        rb_out == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return sci_fail(SCI_ELAUNCH, "cuTensorMapEncodeTiled(output) failed");
+        rc = encode_map(&tmY, "output", d->y, half, 4, dims, strides, box, estr,
+                        rb_out == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE);
+        if (rc) return rc;
     }
     const size_t smem = (size_t)(p.resident ? w_bytes : 0) + (size_t)p.stages * stage_bytes + out_stage + 1024;
     if (smem > 220 * 1024) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: shared memory budget exceeded");
     typedef void (*Fwd2Kernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const Fwd2Params);
+    // indexed by MODE (there is no MODE 3; MODE 4 exists for fp32 only)
     static const Fwd2Kernel kernels[2][2][5] = {
-        {{conv_fwd2_tc_kernel<1, 0, false>, conv_fwd2_tc_kernel<1, 1, false>, conv_fwd2_tc_kernel<1, 2, false>, conv_fwd2_tc_kernel<1, 3, false>,
+        {{conv_fwd2_tc_kernel<1, 0, false>, conv_fwd2_tc_kernel<1, 1, false>, conv_fwd2_tc_kernel<1, 2, false>, nullptr,
           conv_fwd2_tc_kernel<1, 4, false>},
-         {conv_fwd2_tc_kernel<2, 0, false>, conv_fwd2_tc_kernel<2, 1, false>, conv_fwd2_tc_kernel<2, 2, false>, conv_fwd2_tc_kernel<2, 3, false>,
+         {conv_fwd2_tc_kernel<2, 0, false>, conv_fwd2_tc_kernel<2, 1, false>, conv_fwd2_tc_kernel<2, 2, false>, nullptr,
           conv_fwd2_tc_kernel<2, 4, false>}},
         {{conv_fwd2_tc_kernel<1, 0, true>, conv_fwd2_tc_kernel<1, 1, true>, conv_fwd2_tc_kernel<1, 2, true>, nullptr, nullptr},
          {conv_fwd2_tc_kernel<2, 0, true>, conv_fwd2_tc_kernel<2, 1, true>, conv_fwd2_tc_kernel<2, 2, true>, nullptr, nullptr}}};
     const Fwd2Kernel kern = kernels[half ? 1 : 0][epi_wg - 1][mode];
-    if (!kern) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2 fp16: direct-store epilogue not built");
-    static bool attr_set[64][2][2][5] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev][half ? 1 : 0][epi_wg - 1][mode]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "conv tc v2: smem attribute", e);
-        if (dev >= 0 && dev < 64) attr_set[dev][half ? 1 : 0][epi_wg - 1][mode] = true;
-    }
+    if (!kern) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: epilogue not built");
     const int grid = min(p.num_tiles, SCI_NUM_SMS);
     const int threads = 128 + 128 * epi_wg;
     p.pdl = (d->pdl && env_int("SCI_CONV_PDL", 1)) ? 1 : 0;
@@ -1487,204 +1451,29 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
         fprintf(stderr, "conv v2 plan: %dx%d Cin %d -> %d cols (+%d) half %d ps %d mode %d | resident %d stages %d R %d stack %d epi_wg %d out_bufs %d "
                 "rb %d/%d smem %zu KB tiles %d split %d ks_last %d pdl %d\n", d->H, d->W, d->Cin, ncols, col0, (int)half, p.ps, mode, p.resident,
                 p.stages, p.R, p.stack, epi_wg, p.out_bufs, rb_in, rb_out, smem / 1024, p.num_tiles, p.split, p.ks_last, p.pdl);
-    if (p.pdl) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(grid); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = sci_stream(stream);
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmY, p);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "conv tc fwd v2 (PDL launch)", e);
-        return SCI_OK;
-    }
-    kern<<<grid, threads, smem, sci_stream(stream)>>>(tmA, tmB, tmY, p);
-    SCI_CHECK_LAUNCH("conv tc fwd v2");
-    return SCI_OK;
+    return launch(kern, dim3(grid), threads, smem, stream, p.pdl, "conv tc fwd v2", tmA, tmB, tmY, p);
 }
 
 // ---------------------------------------------------------------------------------------------------
-// weight-gradient kernel (conv_wgrad_tc_kernel)
+// weight-gradient kernel, version 2 (conv_wgrad2_tc_kernel): operand orientation and tap fusion chosen per layer
 //   dW[tap][co][ci] += oscale[co] * sum_pixels dz[p][co] * x[p (+) tap][ci]
-//   GEMM view: D[128 co][Cin] += A^T B over K = pixels, both operands MN-major (channels contiguous; TMA swizzle
-//   128B_ATOM_32B <-> UMMA SWIZZLE_128B_BASE32B, the only MN-major layout tcgen05 accepts for TF32):
-//     A = dz tile  [64 pixels][Cout_tile]  = Cout_tile/32 TMA boxes {32 ch, 8 px, 8 rows, 1 image}
-//     B = x  tile  [64 pixels][Cin]        = Cin/32 TMA boxes at the tap-shifted (and, for stride-2 layers,
-//                                            element-strided) coordinates; out-of-image pixels are zero-filled
-//   One CTA owns a filter row (3 taps -> 3 TMEM accumulators of Cin columns), one 128-wide block of output
-//   channels and a strided subset of the 8x8 pixel tiles; it accumulates over all its tiles in TMEM and
-//   finishes with vectorised red.global.add into the packed gradient.
-// ---------------------------------------------------------------------------------------------------
-constexpr int WG_TILE = 8;                       // 8x8 pixels = 64 = K block
-constexpr int WG_CHUNK_BYTES = WG_TILE * WG_TILE * KCH * 4;   // 8 KB per 32-channel chunk
-constexpr int WG_STAGES = 3;
-
-struct WgradParams {
-    const float* oscale; float* dw;
-    int N, Ho, Wo, Cin, Cout, stride;
-    int tiles_w, tiles_h, num_tiles, a_chunks, b_chunks, m_tiles, tmem_cols;
-};
-
-__global__ void __launch_bounds__(TC_THREADS, 1)
-conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtensorMap tmX, const WgradParams p) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t full_bar[WG_STAGES], empty_bar[WG_STAGES], done_bar;
-    __shared__ uint32_t tmem_slot;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const int frow = blockIdx.y / p.m_tiles;          // filter row r (taps r*3 .. r*3+2)
-    const int mt = blockIdx.y % p.m_tiles;            // 128-wide block of output channels
-    const int a_chunks = min(p.a_chunks - mt * 4, 4);
-    const uint32_t a_bytes = (uint32_t)a_chunks * WG_CHUNK_BYTES, b_bytes = (uint32_t)p.b_chunks * WG_CHUNK_BYTES;
-    const uint32_t a_region = 4 * WG_CHUNK_BYTES, stage_bytes = a_region + (uint32_t)p.b_chunks * WG_CHUNK_BYTES;
-
-    if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmZ) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&tmX) : "memory");
-    }
-    if (warp == 1 && lane == 0) {
-        for (int s = 0; s < WG_STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-        mbar_init(&done_bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    if (warp == 2) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"((uint32_t)p.tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = __shfl_sync(0xffffffffu, tmem_slot, 0);
-
-    if (warp == 0) {
-        int stage = 0; uint32_t phase = 0;
-        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-            const int tw = tile % p.tiles_w, th = (tile / p.tiles_w) % p.tiles_h, n = tile / (p.tiles_w * p.tiles_h);
-            const int ow0 = tw * WG_TILE, oh0 = th * WG_TILE;
-            for (int s = 0; s < 3; ++s) {
-                mbar_wait(&empty_bar[stage], phase ^ 1u);
-                if (elect_one()) {
-                    mbar_arrive_expect_tx(&full_bar[stage], a_bytes + b_bytes);
-                    const uint32_t base = smem_base + (uint32_t)stage * stage_bytes;
-                    for (int c = 0; c < a_chunks; ++c)
-                        tma_load_4d(base + c * WG_CHUNK_BYTES, &tmZ, &full_bar[stage], (mt * 4 + c) * KCH, ow0, oh0, n);
-                    for (int c = 0; c < p.b_chunks; ++c)
-                        tma_load_4d(base + a_region + c * WG_CHUNK_BYTES, &tmX, &full_bar[stage], c * KCH,
-                                    ow0 * p.stride + s - 1, oh0 * p.stride + frow - 1, n);
-                }
-                __syncwarp();
-                if (++stage == WG_STAGES) { stage = 0; phase ^= 1u; }
-            }
-        }
-    } else if (warp == 1) {
-        // D=f32, A=B=tf32, both MN-major (bits 15/16), N = Cin, M = 128
-        const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) |
-                               ((uint32_t)(p.Cin >> 3) << 17) | ((128u >> 4) << 24);
-        // MN-major SWIZZLE_128B_BASE32B (atom = 32 channels x 4 pixels): LBO = stride between 32-channel chunks,
-        // SBO = stride between 4-pixel groups; one K=8 MMA spans two atoms
-        const uint64_t desc_hi = umma_desc(0, WG_CHUNK_BYTES, 512, 1);
-        int stage = 0; uint32_t phase = 0; uint32_t first = 1;
-        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-            for (int s = 0; s < 3; ++s) {
-                mbar_wait(&full_bar[stage], phase);
-                tc_fence_after();
-                const uint32_t a_addr = smem_base + (uint32_t)stage * stage_bytes, b_addr = a_addr + a_region;
-                const uint32_t d_tmem = tmem_base + (uint32_t)(s * p.Cin);
-#pragma unroll
-                for (int k8 = 0; k8 < WG_TILE * WG_TILE / 8; ++k8) {
-                    tc_mma_tf32_elect(d_tmem, desc_hi | (uint64_t)(((a_addr + k8 * 1024) & 0x3FFFFu) >> 4),
-                                      desc_hi | (uint64_t)(((b_addr + k8 * 1024) & 0x3FFFFu) >> 4), idesc,
-                                      (uint32_t)(!first || k8 != 0));
-                }
-                tc_commit_elect(&empty_bar[stage]);
-                if (++stage == WG_STAGES) { stage = 0; phase ^= 1u; }
-            }
-            first = 0;
-        }
-        tc_commit_elect(&done_bar);
-    } else if (warp >= 4) {
-        const int q = warp & 3;
-        const int co = mt * 128 + q * 32 + lane;
-        const bool has_work = blockIdx.x < p.num_tiles;
-        if (has_work) {
-            mbar_wait(&done_bar, 0);
-            tc_fence_after();
-            const float sc = (co < p.Cout && p.oscale) ? p.oscale[co] : 1.f;
-            for (int s = 0; s < 3; ++s) {
-                const int tap = frow * 3 + s;
-                const uint32_t t_row = tmem_base + (uint32_t)(s * p.Cin) + ((uint32_t)(q * 32) << 16);
-                for (int c0 = 0; c0 < p.Cin; c0 += 32) {
-                    float v[32];
-                    tmem_ld32(t_row + c0, v);
-                    if (co < p.Cout) {
-                        float* dst = p.dw + ((long)tap * p.Cout + co) * p.Cin + c0;
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4)
-                            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(v[j] * sc),
-                                         "f"(v[j + 1] * sc), "f"(v[j + 2] * sc), "f"(v[j + 3] * sc) : "memory");
-                    }
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 2) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols) : "memory");
-    }
-}
-
-int conv_wgrad_tc_launch(const sci_wgrad_desc* d, void* stream) {
-    if (d->Cin % KCH != 0 || d->Cout % KCH != 0 || d->Cin > 128 || d->Cout > 256)
-        return sci_fail(SCI_EUNSUPPORTED, "wgrad tc: needs Cin % 32 == 0 (<= 128), Cout % 32 == 0 (<= 256)");
-    WgradParams p;
-    p.oscale = d->oscale; p.dw = d->dw;
-    p.N = d->N; p.stride = d->stride; p.Cin = d->Cin; p.Cout = d->Cout;
-    p.Ho = (d->H - 1) / d->stride + 1; p.Wo = (d->W - 1) / d->stride + 1;
-    p.tiles_w = (p.Wo + WG_TILE - 1) / WG_TILE; p.tiles_h = (p.Ho + WG_TILE - 1) / WG_TILE;
-    p.num_tiles = p.tiles_w * p.tiles_h * p.N;
-    p.a_chunks = p.Cout / KCH; p.b_chunks = p.Cin / KCH;
-    p.m_tiles = (p.Cout + 127) / 128;
-    p.tmem_cols = next_pow2_cols(3 * p.Cin);
-    CUtensorMap tmZ, tmX;
-    int rc = make_act_map(&tmZ, d->dz, d->N, p.Ho, p.Wo, d->Cout, 1, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
-    if (rc) return rc;
-    rc = make_act_map(&tmX, d->x, d->N, d->H, d->W, d->Cin, d->stride, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
-    if (rc) return rc;
-    const size_t stage_bytes = (size_t)4 * WG_CHUNK_BYTES + (size_t)p.b_chunks * WG_CHUNK_BYTES;
-    const size_t smem = WG_STAGES * stage_bytes + 1024;
-    static bool attr_set[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(conv_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "wgrad tc: smem attribute", e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
-    const int groups = 3 * p.m_tiles;
-    const int gx = max(1, min(p.num_tiles, (2 * SCI_NUM_SMS) / groups));
-    if (env_int("SCI_CONV_VERBOSE", 0))
-        fprintf(stderr, "wgrad v1 plan: %dx%d Cin %d Cout %d stride %d | m_tiles %d grid %d groups %d tiles %d\n", d->H, d->W, d->Cin, d->Cout,
-                d->stride, p.m_tiles, gx, groups, p.num_tiles);
-    conv_wgrad_tc_kernel<<<dim3(gx, groups), TC_THREADS, smem, sci_stream(stream)>>>(tmZ, tmX, p);
-    SCI_CHECK_LAUNCH("conv tc wgrad");
-    return SCI_OK;
-}
-
-
-// ---------------------------------------------------------------------------------------------------
-// weight-gradient kernel, version 2: operand orientation and tap fusion chosen per layer
-//   The version-1 launch list (profiles/) showed the full-resolution 32-channel layers at 0.73-0.89 ms each: with
-//   M = Cout = 32 of 128 rows used, three quarters of every MMA were wasted and each tap reloaded the dz tile.
+//   GEMM view: D[128][N] += A^T B over K = pixels, both operands MN-major (channels contiguous; TMA swizzle
+//   128B_ATOM_32B <-> UMMA SWIZZLE_128B_BASE32B, the only MN-major layout tcgen05 accepts for TF32), built from TMA boxes
+//   {32 ch, 8 px, 8 rows, 1 image} of dz and of x at the tap-shifted (and, for stride-2 layers, element-strided)
+//   coordinates; out-of-image pixels are zero-filled.  One CTA group owns a filter row and one 128-wide M block, each
+//   CTA a strided subset of the 8x8 pixel tiles; it accumulates in TMEM and finishes with red.global.add into the
+//   packed gradient.  The launch list of a first version with M = Cout fixed (profiles/) showed the full-resolution
+//   32-channel layers at 0.73-0.89 ms each: with M = 32 of 128 rows used, three quarters of every MMA were wasted and
+//   each tap reloaded the dz tile.  Hence
 //   * swap = 0: M side = dz (Cout), N side = x.  swap = 1: M side = x (Cin), N side = dz (Cout) - chosen when that
 //     fills the 128 MMA rows better.
 //   * fuse = 1: the three horizontal taps of the filter row are ONE operand (their 32-channel chunks are simply
 //     consecutive chunks of the MN-major operand), so one MMA per 8 pixels covers all three taps and the unshifted
 //     operand is loaded once per tile instead of once per tap.
 // ---------------------------------------------------------------------------------------------------
+constexpr int WG_TILE = 8;                       // 8x8 pixels = 64 = K block
+constexpr int WG_CHUNK_BYTES = WG_TILE * WG_TILE * KCH * 4;   // 8 KB per 32-channel chunk
+
 struct Wgrad2Params {
     const float* oscale; float* dw;
     int N, Ho, Wo, Cin, Cout, stride;
@@ -1862,22 +1651,12 @@ int conv_wgrad2_tc_launch(const sci_wgrad_desc* d, void* stream) {
     rc = make_act_map(&tmX, d->x, d->N, d->H, d->W, d->Cin, d->stride, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (rc) return rc;
     const size_t smem = p.stages * stage_bytes + 1024;
-    static bool attr_set[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(conv_wgrad2_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "wgrad tc v2: smem attribute", e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
     const int groups = 3 * p.m_tiles;
     const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS / groups));
     if (env_int("SCI_CONV_VERBOSE", 0))
         fprintf(stderr, "wgrad v2 plan: %dx%d Cin %d Cout %d stride %d | swap %d fuse %d m_tiles %d accs %d stages %d grid %d groups %d tiles %d\n",
                 d->H, d->W, d->Cin, d->Cout, d->stride, p.swap, p.fuse, p.m_tiles, p.accs, p.stages, gx, groups, p.num_tiles);
-    conv_wgrad2_tc_kernel<<<dim3(gx, groups), TC_THREADS, smem, sci_stream(stream)>>>(tmZ, tmX, p);
-    SCI_CHECK_LAUNCH("conv tc wgrad v2");
-    return SCI_OK;
+    return launch(conv_wgrad2_tc_kernel, dim3(gx, groups), TC_THREADS, smem, stream, false, "conv tc wgrad v2", tmZ, tmX, p);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -2050,21 +1829,11 @@ int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream) {
     rc = make_act_map(&tmQ, Q, d->N, d->H, d->W, cq, 1, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (rc) return rc;
     const size_t smem = p.stages * stage_bytes + 2048 + 1024;
-    static bool attr_set[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(conv_wgrad3_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "wgrad tc v3: smem attribute", e);
-        if (dev >= 0 && dev < 64) attr_set[dev] = true;
-    }
     const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS));
     if (env_int("SCI_CONV_VERBOSE", 0))
         fprintf(stderr, "wgrad v3 plan: %dx%d Cin %d Cout %d stride 1 | p_is_dz %d cp %d cq %d stages %d grid %d tiles %d\n", d->H, d->W,
                 d->Cin, d->Cout, p.p_is_dz, cp, cq, p.stages, gx, p.num_tiles);
-    conv_wgrad3_tc_kernel<<<gx, TC_THREADS, smem, sci_stream(stream)>>>(tmP, tmQ, p);
-    SCI_CHECK_LAUNCH("conv tc wgrad v3");
-    return SCI_OK;
+    return launch(conv_wgrad3_tc_kernel, dim3(gx), TC_THREADS, smem, stream, false, "conv tc wgrad v3", tmP, tmQ, p);
 }
 
 int check_conv_desc(const sci_conv_desc* d) {
@@ -2115,7 +1884,7 @@ extern "C" int sci_conv3x3_wgrad(const sci_wgrad_desc* d, int impl, void* stream
         if (d->Cin % 32 != 0 || d->Cout % 32 != 0 || d->Cin > 128 || d->Cout > 256)
             return sci_fail(SCI_EUNSUPPORTED, "wgrad tc: needs Cin % 32 == 0 (<= 128), Cout % 32 == 0 (<= 256)");
         if (wgrad3_eligible(d)) return conv_wgrad3_tc_launch(d, stream);
-        return env_int("SCI_WGRAD_V2", 1) ? conv_wgrad2_tc_launch(d, stream) : conv_wgrad_tc_launch(d, stream);
+        return conv_wgrad2_tc_launch(d, stream);
     }
     return sci_fail(SCI_EINVAL, "wgrad: unknown impl");
 }

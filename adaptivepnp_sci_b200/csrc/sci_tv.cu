@@ -18,8 +18,6 @@
 // rewrites the few channels that did.  No host involvement, 3 launches.
 //
 // Compiled with --fmad=false: the fp32 arithmetic mirrors numpy's separate ops.
-#include <stdlib.h>
-
 #include "sci_common.cuh"
 
 namespace {
@@ -28,165 +26,16 @@ constexpr int TV_TW = 64, TV_TH = 32;      // output tile (full-res pixels)
 constexpr int TV_HALO = 8;                 // 4 half-res pixels
 constexpr int TV_RW = TV_TW + 2 * TV_HALO; // 80
 constexpr int TV_RH = TV_TH + 2 * TV_HALO; // 48
-constexpr int TV_NPIX = TV_RW * TV_RH;     // 3840
-constexpr int TV_ROWGROUPS = 4;            // 80 columns x 4 row groups
-constexpr int TV_THREADS = TV_RW * TV_ROWGROUPS;   // 320
+constexpr int TV_THREADS = 320;            // 40 column pairs x 8 row groups
 constexpr int TV_MAX_UPD = 4;              // out_1..out_4 are the candidate results
-#ifndef TV_UNROLL
-#define TV_UNROLL 4                        // row-loop unrolling: independent pixels in flight hide the sqrt / divide latency
-#endif
-constexpr int TV_UNROLL_N = TV_UNROLL;
 
 // workspace: double epart[B][4 iters][2 kinds][4 phases][nblk], then int nstop[B*4]
 __host__ __device__ inline size_t tv_epart_count(int B, int nblk) { return (size_t)B * 4 * 2 * 4 * nblk; }
 
-// is_fix = 0: main pass (all channels run to n_iter_max, energies recorded)
-// is_fix = 1: fix-up pass (only channels with nstop < last are rewritten)
-__global__ void __launch_bounds__(TV_THREADS) tv_chambolle_kernel(
-    const float* __restrict__ x, const float* __restrict__ b, float c_b, float* __restrict__ theta,
-    float* __restrict__ b_out, float s_b, int clip, int H, int W, float tau, float tw, int last_iter,
-    double* __restrict__ epart, const int* __restrict__ nstop, int is_fix) {
-    extern __shared__ float smem[];
-    float* sf = smem;                 // f = x + c_b*b
-    float* so = sf + TV_NPIX;         // current iterate out_i
-    float* sp0 = so + TV_NPIX;        // dual variable, row direction
-    float* sp1 = sp0 + TV_NPIX;       // dual variable, column direction
-    __shared__ double sred[TV_THREADS / 32][16][2];   // 10 warps
-    __shared__ int s_stop[4];
-
-    const int t = blockIdx.z;
-    const int nblk = gridDim.x * gridDim.y, blk = blockIdx.y * gridDim.x + blockIdx.x;
-    if (threadIdx.x < 4) s_stop[threadIdx.x] = is_fix ? nstop[t * 4 + threadIdx.x] : last_iter;
-    __syncthreads();
-    if (is_fix && s_stop[0] >= last_iter && s_stop[1] >= last_iter && s_stop[2] >= last_iter && s_stop[3] >= last_iter)
-        return;
-
-    const long plane = (long)H * W;
-    const float* xp = x + t * plane;
-    const float* bp = b ? b + t * plane : nullptr;
-    const int gr0 = blockIdx.y * TV_TH - TV_HALO, gc0 = blockIdx.x * TV_TW - TV_HALO;
-
-    // thread -> fixed column cx of the 80-wide region, rows ry, ry+4, ... (no per-pixel
-    // div/mod, column predicates hoisted out of the row loops)
-    const int cx = threadIdx.x % TV_RW, ry = threadIdx.x / TV_RW;
-    const bool t_active = true;
-    const int gc = gc0 + cx;
-    const bool col_in = gc >= 0 && gc < W;
-    const bool col_interior = cx >= TV_HALO && cx < TV_HALO + TV_TW && gc < W;
-    const bool col_has_left = gc >= 2 && cx >= 2;            // neighbour (c-2) exists in the image and in the tile
-    const bool col_has_right = gc + 2 < W && cx + 2 < TV_RW;
-
-    if (t_active) {
-        for (int rr = ry; rr < TV_RH; rr += TV_ROWGROUPS) {
-            const int gr = gr0 + rr, i = rr * TV_RW + cx;
-            float v = 0.f;
-            if (col_in && gr >= 0 && gr < H) {
-                v = xp[(long)gr * W + gc];
-                if (bp) v = v + c_b * bp[(long)gr * W + gc];
-            }
-            sf[i] = v; so[i] = v; sp0[i] = 0.f; sp1[i] = 0.f;
-        }
-    }
-    __syncthreads();
-
-    // energy accumulators: [iteration 0..3][row parity] for (sum d^2, sum |g|); the column parity is fixed per thread
-    double e_d[TV_MAX_UPD][2], e_n[TV_MAX_UPD][2];
-#pragma unroll
-    for (int k = 0; k < TV_MAX_UPD; ++k) { e_d[k][0] = e_d[k][1] = e_n[k][0] = e_n[k][1] = 0.0; }
-    const int cpar = gc & 1;
-
-#pragma unroll
-    for (int it = 0; it <= TV_MAX_UPD; ++it) {
-        if (it > last_iter) break;
-        // ---- phase A: d = -div p, out = f + d (it > 0); write the result of the channels stopping here
-        if (it > 0) {
-            if (t_active) {
-#pragma unroll TV_UNROLL_N
-                for (int rr = ry; rr < TV_RH; rr += TV_ROWGROUPS) {
-                    const int gr = gr0 + rr, i = rr * TV_RW + cx;
-                    float d = -(sp0[i] + sp1[i]);
-                    if (gr >= 2 && rr >= 2) d += sp0[i - 2 * TV_RW];
-                    if (col_has_left) d += sp1[i - 2];
-                    const float o = sf[i] + d;
-                    so[i] = o;
-                    if (col_interior && rr >= TV_HALO && rr < TV_HALO + TV_TH && gr < H) {
-                        const int rpar = gr & 1;
-                        if (it < TV_MAX_UPD && !is_fix) {
-                            const double dd = (double)(d * d);
-                            if (rpar) e_d[it][1] += dd; else e_d[it][0] += dd;
-                        }
-                        const int stop = s_stop[rpar * 2 + cpar];
-                        if (it == stop && (!is_fix || stop < last_iter)) {
-                            const long g = (long)gr * W + gc;
-                            float th = o;
-                            if (clip) th = fminf(fmaxf(th, 0.f), 1.f);
-                            theta[t * plane + g] = th;
-                            if (bp) b_out[t * plane + g] = bp[g] + s_b * (xp[g] - th);
-                        }
-                    }
-                }
-            }
-            __syncthreads();
-        }
-        if (it == TV_MAX_UPD || it == last_iter) break;   // the last dual update never shapes the result
-        // ---- phase B: forward differences, energy, dual update
-        if (t_active) {
-#pragma unroll TV_UNROLL_N
-            for (int rr = ry; rr < TV_RH; rr += TV_ROWGROUPS) {
-                const int gr = gr0 + rr, i = rr * TV_RW + cx;
-                const bool in_img = col_in && gr >= 0 && gr < H;
-                const float o = so[i];
-                float g0 = 0.f, g1 = 0.f;
-                if (in_img && gr + 2 < H && rr + 2 < TV_RH) g0 = so[i + 2 * TV_RW] - o;
-                if (in_img && col_has_right) g1 = so[i + 2] - o;
-                const float nrm = sqrtf(g0 * g0 + g1 * g1);
-                if (col_interior && rr >= TV_HALO && rr < TV_HALO + TV_TH && gr < H && !is_fix) {
-                    if (gr & 1) e_n[it][1] += (double)nrm; else e_n[it][0] += (double)nrm;
-                }
-                const float inv = 1.0f / (nrm * tw + 1.0f);          // one IEEE division shared by both components
-                sp0[i] = in_img ? (sp0[i] - tau * g0) * inv : 0.f;
-                sp1[i] = in_img ? (sp1[i] - tau * g1) * inv : 0.f;
-            }
-        }
-        __syncthreads();
-    }
-
-    if (is_fix) return;
-    // ---- deterministic per-block energy partials: warp shuffle (keeping lane parity = column parity), then
-    //      a fixed-order sum over the 8 warps
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-    for (int k = 0; k < TV_MAX_UPD; ++k)
-#pragma unroll
-        for (int rp = 0; rp < 2; ++rp) {
-            double a = e_d[k][rp], c = e_n[k][rp];
-#pragma unroll
-            for (int o = 16; o >= 2; o >>= 1) {
-                a += __shfl_xor_sync(0xffffffffu, a, o);
-                c += __shfl_xor_sync(0xffffffffu, c, o);
-            }
-            if (lane < 2) {      // lane parity == thread parity == column parity offset
-                sred[wid][(k * 2 + rp) * 2 + 0][lane] = a;
-                sred[wid][(k * 2 + rp) * 2 + 1][lane] = c;
-            }
-        }
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        // thread -> (k, rp, kind, lane_par)
-        const int lp = threadIdx.x & 1, kind = (threadIdx.x >> 1) & 1, rp = (threadIdx.x >> 2) & 1, k = threadIdx.x >> 3;
-        double s = 0.0;
-        for (int w8 = 0; w8 < TV_THREADS / 32; ++w8) s += sred[w8][(k * 2 + rp) * 2 + kind][lp];
-        // lane parity lp == column parity: cx = threadIdx.x % 80 keeps the parity of threadIdx.x, gc0 is even
-        const int cp = (gc0 + lp) & 1;
-        const int phase = rp * 2 + cp;
-        epart[((((size_t)t * 4 + k) * 2 + kind) * 4 + phase) * nblk + blk] = s;
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------
-// Version 2 of the tile kernel (same maths, same interface, bit-identical interior results).  ncu on version 1
-// (profiles/ncu_r1_prof_tv_chambolle.csv): issue slots 65 % busy, DRAM 2 % — instruction-bound, and most instructions were
-// boundary predicates and address arithmetic.  Here
+// The tile kernel.  ncu on an earlier, straightforward form (one thread per column, profiles/ncu_r1_prof_tv_chambolle.csv)
+// found it instruction-bound: issue slots 65 % busy, DRAM 2 %, and most instructions were boundary predicates and address
+// arithmetic.  Hence
 //   * the four shared-memory arrays carry a 2-pixel zero border, so tile-edge neighbours need no predicate (halo pixels
 //     may then hold garbage one ring deeper per iteration, which the 8-pixel halo already budgets for);
 //   * image borders are handled by per-row / per-thread select masks (dual variables outside the image stay exactly 0);
@@ -200,6 +49,8 @@ constexpr int TV2_PAIRS = TV_RW / 2;               // 40 column pairs
 constexpr int TV2_RG = TV_THREADS / TV2_PAIRS;     // 8 row groups
 constexpr int TV2_RPT = TV_RH / TV2_RG;            // 6 rows per thread
 
+// is_fix = 0: main pass (all channels run to n_iter_max, energies recorded)
+// is_fix = 1: fix-up pass (only channels with nstop < last are rewritten)
 __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
     const float* __restrict__ x, const float* __restrict__ b, float c_b, float* __restrict__ theta,
     float* __restrict__ b_out, float s_b, int clip, int H, int W, float tau, float tw, int last_iter,
@@ -421,18 +272,9 @@ extern "C" int sci_tv_chambolle2d(const float* x, const float* b, float c_b, flo
     const int nblk = grid.x * grid.y;
     double* epart = reinterpret_cast<double*>(workspace);
     int* nstop = reinterpret_cast<int*>(epart + tv_epart_count(B, nblk));
-    const char* v2env = getenv("SCI_TV_V2");
-    const bool v2 = !(v2env && v2env[0] == '0');
-    auto kern = v2 ? tv_chambolle2_kernel : tv_chambolle_kernel;
-    const size_t smem = v2 ? (size_t)4 * TV2_N * sizeof(float) : (size_t)4 * TV_NPIX * sizeof(float);
-    static bool attr_set[64][2] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr_set[dev][v2]) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "tv: smem attribute", e);
-        if (dev >= 0 && dev < 64) attr_set[dev][v2] = true;
-    }
+    const size_t smem = (size_t)4 * TV2_N * sizeof(float);
+    const cudaError_t e = sci_smem_limit((const void*)tv_chambolle2_kernel, (int)smem);
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "tv: smem attribute", e);
     const int last_iter = n_iter_max - 1;              // index of the last iterate (4 for n_iter_max=5)
     const float tau = 0.25f;                            // 1/(2*ndim), ndim = 2
     const float tw = (float)(0.25 / (double)weight);    // python-double tau/weight, cast at the fp32 multiply
@@ -440,13 +282,13 @@ extern "C" int sci_tv_chambolle2d(const float* x, const float* b, float c_b, flo
         // n_iter_max = 1 returns the input unchanged
         return sci_fail(SCI_EUNSUPPORTED, "tv: n_iter_max = 1 is the identity; not routed through the kernel");
     }
-    kern<<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nullptr, 0);
+    tv_chambolle2_kernel<<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nullptr, 0);
     SCI_CHECK_LAUNCH("tv main pass");
     const int nch = B * 4;
     tv_decide_kernel<<<nch, TV_DEC_THREADS, 0, st>>>(epart, nblk, (double)weight, (double)eps,
                                                      (double)(H / 2) * (double)(W / 2), last_iter, nstop, nstop_out);
     SCI_CHECK_LAUNCH("tv decide");
-    kern<<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nstop, 1);
+    tv_chambolle2_kernel<<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nstop, 1);
     SCI_CHECK_LAUNCH("tv fix-up pass");
     return SCI_OK;
 }

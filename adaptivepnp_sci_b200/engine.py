@@ -178,19 +178,7 @@ class ConvLayer:
         self.dwpk = None
         self.first = first       # network input layer: on the TF32 path its input arrives as hi + remainder copies
 
-    def refresh_fwd(self, tf32):
-        c = self.conv
-        if self.bn is not None:
-            bn = self.bn
-            call("sci_bn_fold", ptr(bn.weight.data), ptr(bn.bias.data), ptr(bn.running_mean), ptr(bn.running_var),
-                 float(bn.eps), ptr(self.scale), ptr(self.shift), self.Co, self.Co_pad, stream())
-        elif c.bias is not None:
-            self.shift[:self.Co].copy_(c.bias.data)
-        self.ci_dup = self.ci_half if self.dup_in else (16 if (self.first and tf32) else 0)
-        call("sci_conv_pack_weights", ptr(c.weight.data), ptr(self.wpk), self.Co, self.Ci, self.groups, self.Co_pad,
-             self.Ci_pad, int(self.ps), None, 0, (2 if (tf32 and self.wsplit) else int(tf32)), self.ci_dup, stream())
-
-    # ---- the same work as table entries of a batched launch (engine: one launch per phase instead of one per layer) ----
+    # ---- table entries of the engine's batched bookkeeping launches (one launch per phase, see _EngineBase._table) ----
     def fwd_ops(self, tf32):
         c = self.conv
         ops = []
@@ -229,24 +217,6 @@ class ConvLayer:
             ops.append(_op(6, Co=self.Co, a=self.s1, o0=bucket.grad_view(self.conv.bias)))
         return ops
 
-    def refresh_bwd(self, tf32):
-        """Data-gradient form of the weights: transposed, taps flipped, rows scaled by the folded BN scale."""
-        if self.wpk_t is None:
-            self.wpk_t = torch.empty(9 * self.Co_pad * self.Ci_pad, dtype=torch.float32, device=self.wpk.device)
-            self.s1 = torch.zeros(self.Co_pad, dtype=torch.float32, device=self.wpk.device)
-            self.s2 = torch.zeros(self.Co_pad, dtype=torch.float32, device=self.wpk.device)
-        if self.stride == 2 and self.groups == 1 and not self.ps and self.ci_dup == 0:
-            # stride-2 layers: data gradient as a sub-pixel convolution over dz at the low resolution
-            if self.wpk_t.numel() != 36 * self.Co_pad * self.Ci_pad:
-                self.wpk_t = torch.empty(36 * self.Co_pad * self.Ci_pad, dtype=torch.float32, device=self.wpk.device)
-            call("sci_conv_pack_weights_s2t", ptr(self.conv.weight.data), ptr(self.wpk_t), self.Co, self.Ci, self.Co_pad,
-                 self.Ci_pad, ptr(self.scale), int(tf32), stream())
-            self.s2t = True
-            return
-        self.s2t = False
-        call("sci_conv_pack_weights", ptr(self.conv.weight.data), ptr(self.wpk_t), self.Co, self.Ci, self.groups,
-             self.Co_pad, self.Ci_pad, int(self.ps), ptr(self.scale), 1, int(tf32), self.ci_dup, stream())
-
 
 class HalfLayer:
     """fp16 forward form of a ConvLayer (inference chains on the kind::f16 kernels, ``sci_conv_desc.half_io``).
@@ -271,11 +241,6 @@ class HalfLayer:
         self.N = base.Co_pad
         self.stride, self.relu, self.ps = base.stride, base.relu, base.ps
         self.wpk = torch.empty(9 * self.N * self.K, dtype=torch.float16, device=base.conv.weight.device)
-
-    def refresh_fwd(self, tf32):
-        c = self.base.conv
-        call("sci_conv_pack_weights_half", ptr(c.weight.data), ptr(self.wpk), self.base.Co, self.base.Ci, self.base.groups,
-             self.N, self.K, int(self.ps), self.ci_dup, stream())
 
     def fwd_ops(self, tf32):
         b = self.base
@@ -313,8 +278,6 @@ class _EngineBase:
         self._bwd_valid = False
         self.dirty = True
         self.n_launch = 0
-        self.batch = os.environ.get("SCI_BATCH_OPS", "1") != "0"
-        self.fuse_act = os.environ.get("SCI_FUSE_ACT_BWD", "1") != "0"      # activation backward in the dgrad epilogue
         self._tables = None
         self.s12_flat = None
         self.pdl_chain = False   # True inside an inference chain: weights are packed, consecutive convs may overlap (PDL)
@@ -335,11 +298,7 @@ class _EngineBase:
         if self._tables is not None and self._tables["bucket"] is not self.bucket:
             self._tables = None                                       # new parameter storage: every table entry points at the old one
         if self.dirty or self._version() != self._seen_version:
-            if self.batch:
-                self._table("fwd").run()
-            else:
-                for L in self.layers + (getattr(self, "layers_inf", None) or []):
-                    L.refresh_fwd(self.tf32)
+            self._table("fwd").run()
             self._seen_version = self._version()
             self._bwd_valid = False
             self.dirty = False
@@ -351,15 +310,11 @@ class _EngineBase:
                 L.dwpk = self.dw_flat[off:off + n]
                 off += n
         if training and not self._bwd_valid:
-            if self.batch:
-                self._table("bwd").run()
-            else:
-                for L in self.layers:
-                    L.refresh_bwd(self.tf32)
+            self._table("bwd").run()
             self._bwd_valid = True
 
     def _table(self, which):
-        """Batched bookkeeping (SCI_BATCH_OPS=0 restores one launch per layer): 'fwd' = BatchNorm folding / bias + weight
+        """Batched bookkeeping, one launch per phase: 'fwd' = BatchNorm folding / bias + weight
         packing of every layer (+ the fp16 / split inference forms), 'bwd' = data-gradient weight forms, 'grads' = packed
         weight gradients -> parameter gradients + BatchNorm / bias gradients from the column sums."""
         if self._tables is None:
@@ -384,14 +339,17 @@ class _EngineBase:
     def begin_backward(self):
         """Zero the packed weight-gradient accumulators and the per-column sums (one memset each)."""
         self.dw_flat.zero_()
-        if self.batch:
-            self.s12_flat.zero_()
+        self.s12_flat.zero_()
+
+    def param_grads(self, L):
+        """Per-layer step of the parameter gradients of L: nothing is left to do per layer, finish_param_grads() computes
+        those of every layer in one launch.  Kept so that callers which drive a backward pass layer by layer still work."""
 
     def finish_param_grads(self):
-        """Batched mode: all parameter gradients in one launch at the end of the backward pass."""
-        if self.batch:
-            self._table("grads").run()
-            self.n_launch += 1
+        """All parameter gradients in one launch at the end of the backward pass: packed dW -> torch-layout grad slots,
+        bias / BatchNorm affine grads from the column sums."""
+        self._table("grads").run()
+        self.n_launch += 1
 
     # ---- kernel wrappers ------------------------------------------------------------------------------
     def conv(self, L, x, N, H, W, y, residual=None, round_out=True, emit_lo=False, planar=None):
@@ -442,7 +400,7 @@ class _EngineBase:
 
     def can_fuse_act_bwd(self, Lp, out_channels):
         """The data-gradient kernel can apply layer Lp's activation backward in its epilogue (tensor-core fp32 path)."""
-        return (self.fuse_act and self.impl == IMPL_TC and self.batch and (Lp.relu or Lp.has_affine) and out_channels <= 128)
+        return self.impl == IMPL_TC and (Lp.relu or Lp.has_affine) and out_channels <= 128
 
     def dgrad_s2(self, L, dz, N, Ho, Wo, dx, residual=None, mask=None):
         """Stride-2 layer: dx[N,2Ho,2Wo,Ci_pad] = PixelShuffle(conv(dz[N,Ho,Wo,Co_pad], sub-pixel weights)) [+ residual]."""
@@ -470,26 +428,10 @@ class _EngineBase:
         need = L.has_affine
         if not (L.relu or need):
             return dy
-        if need and not self.batch:
-            L.s1.zero_()
-            L.s2.zero_()
         call("sci_act_bwd", ptr(dy), ptr(y) if (L.relu or L.bn is not None) else None, ptr(dy), n_pix, C, int(L.relu),
              ptr(L.s1) if need else None, ptr(L.s2) if (need and L.bn is not None) else None, stream())
         self.n_launch += 1
         return dy
-
-    def param_grads(self, L):
-        """packed dW -> torch-layout grad slot; bias / BatchNorm affine grads from the column sums."""
-        if self.batch:
-            return                                   # done for all layers at once by finish_param_grads()
-        b = self.bucket
-        call("sci_conv_unpack_wgrad", ptr(L.dwpk), ptr(b.grad_view(L.conv.weight)), L.Co, L.Ci, L.groups, L.Co_pad,
-             L.Ci_pad, int(L.ps), L.ci_dup, stream())
-        if L.bn is not None:
-            call("sci_bn_param_grad", ptr(L.s1), ptr(L.s2), ptr(L.bn.weight.data), ptr(L.bn.bias.data),
-                 ptr(b.grad_view(L.bn.weight)), ptr(b.grad_view(L.bn.bias)), L.Co, stream())
-        elif L.conv.bias is not None:
-            b.grad_view(L.conv.bias).copy_(L.s1[:L.Co])
 
     def after_step(self):
         """Parameters were updated in place by sci_adam_step (raw pointers): re-pack on next use."""
@@ -511,22 +453,20 @@ class FFDNetEngine(_EngineBase):
             # This also holds for the TRAINING forward: with plain TF32 weights there (1.75 ms instead of 3.5 ms per pass at
             # 8x512x512, tools/time_ffdnet_train.py) the Adam-normalised updates change enough to move the final
             # reconstruction by 5e-3 on the golden online loop (3.4e-4 with the split), so the split stays on.
-            layers.append(ConvLayer(c, bn, relu=not last, first=(i == 0), wsplit=(default_impl() == IMPL_TC)
-                                    and os.environ.get("SCI_FFDNET_TRAIN_WSPLIT", "1") != "0"))
+            layers.append(ConvLayer(c, bn, relu=not last, first=(i == 0), wsplit=default_impl() == IMPL_TC))
         super().__init__(module, layers)
-        # inference on the TF32 path uses "3xTF32": every activation is stored as tf32 hi + remainder and every weight
-        # as tf32 hi + remainder, which brings the conv stack to ~fp32 accuracy (FFDNet has no residual connection, so
-        # plain TF32 rounding reaches the output undamped and is then integrated by the ADMM dual variables)
-        self.layers_inf = None
-        if self.tf32 and os.environ.get("SCI_FFDNET_INF_PRODUCTS", "3") == "3":
-            self.layers_inf = [ConvLayer(c, bn, relu=(i < len(convs) - 1), first=(i == 0), wsplit=True, dup_in=(i > 0))
-                               for i, (c, bn) in enumerate(convs)]
-        # ... and since round 2 as fp16 value + fp16 remainder (x 2^11) per activation and weight on the row-reuse kernel:
-        # the same three products at the fp16 tensor rate and half the bytes (SCI_FFDNET_INF=tf32 restores the 3xTF32 chain)
+        # inference on the TF32 path keeps every activation and weight as a value + remainder pair, which brings the conv
+        # stack to ~fp32 accuracy (FFDNet has no residual connection, so plain TF32 rounding reaches the output undamped
+        # and is then integrated by the ADMM dual variables): as fp16 value + fp16 remainder (x 2^11) on the row-reuse
+        # kernel, three products at the fp16 tensor rate and half the bytes ...
         self.layers_h = None
         if self.tf32 and os.environ.get("SCI_FFDNET_INF", "half") == "half" and all(L.Co_pad <= 128 for L in layers):
             self.layers_h = [HalfLayer(L, 0, 0, split=True) for L in layers]
-            self.layers_inf = self.layers_h              # (the list prepare() re-packs)
+        # ... or, with SCI_FFDNET_INF=tf32 or a layer wider than 128 columns, as "3xTF32": tf32 hi + remainder
+        self.layers_inf = self.layers_h                  # (the list prepare() re-packs)
+        if self.tf32 and self.layers_h is None:
+            self.layers_inf = [ConvLayer(c, bn, relu=(i < len(convs) - 1), first=(i == 0), wsplit=True, dup_in=(i > 0))
+                               for i, (c, bn) in enumerate(convs)]
         self.in_nc, self.out_nc = module.in_nc, module.out_nc
         if (self.in_nc, self.out_nc) not in ((3, 3), (1, 1)):
             raise NotImplementedError("native FFDNet engine: colour (3->3) and gray (1->1) models")
@@ -606,7 +546,6 @@ class FFDNetEngine(_EngineBase):
                 dx = self.ws.get("g%d" % (i % 2), (B, h2, w2, L.Ci_pad), dev)
                 self.dgrad(L, dz, B, h2, w2, dx)
                 dy = dx
-            self.param_grads(L)
         self.finish_param_grads()
 
     def forward_nchw(self, x, sigma):
@@ -823,7 +762,6 @@ class FastDVDnetEngine(_EngineBase):
                 else:
                     Ho, Wo = Hin, Win
                     self.dgrad(Li, dz, N, Ho, Wo, dx, residual, mask=mask)
-            self.param_grads(Li)
             return dx
 
         # out = in1 - xo  ->  d xo = -dout (padded columns 0)
@@ -945,7 +883,6 @@ class DDnetEngine(_EngineBase):
                 self.dgrad_s2(Li, dz, N, Ho, Wo, dx, residual)
             else:
                 self.dgrad(Li, dz, N, Ho, Wo, dx, residual)
-        self.param_grads(Li)
         return dx
 
     def _body_backward(self, L, S, d_xo, N, H, W, want_dx, tag):

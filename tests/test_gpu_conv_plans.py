@@ -47,15 +47,14 @@ MARGIN = 1024                         # elements before and after every output (
 N_, H_, W_ = 2, 37, 300               # W: tiles of 128 + 128 + 44 pixels; H: no multiple of 2, 4 or 8
 SCI_EUNSUPPORTED = -3
 KNOBS = ("SCI_CONV_V2", "SCI_CONV_RESIDENT", "SCI_CONV_WPAIR", "SCI_CONV_ROWS", "SCI_CONV_STACK", "SCI_CONV_EPI_WG",
-         "SCI_CONV_TMA_STORE", "SCI_CONV_TPS", "SCI_CONV_SPLIT_ACC", "SCI_CONV_PDL", "SCI_WGRAD_V2", "SCI_WGRAD_V3",
-         "SCI_CONV_SW64", "SCI_CONV_IMPL", "SCI_FFDNET_INF", "SCI_FFDNET_INF_PRODUCTS", "SCI_CONV_HALF")
+         "SCI_CONV_TPS", "SCI_CONV_SPLIT_ACC", "SCI_CONV_PDL", "SCI_WGRAD_V3", "SCI_CONV_SW64", "SCI_CONV_IMPL",
+         "SCI_FFDNET_INF", "SCI_CONV_HALF")
 
 
 @pytest.fixture(autouse=True)
 def _plan_env(monkeypatch):
     """Every case starts from the planner's defaults and prints its launch plans."""
-    for k in ("SCI_CONV_DBG", "SCI_CONV_DESC_MODE"):
-        assert k not in os.environ, "%s is a timing experiment (results invalid): unset it" % k
+    assert "SCI_CONV_DBG" not in os.environ, "SCI_CONV_DBG is a timing experiment (results invalid): unset it"
     for k in KNOBS:
         monkeypatch.delenv(k, raising=False)
     monkeypatch.setenv("SCI_CONV_VERBOSE", "1")
@@ -210,11 +209,11 @@ FWD_CASES = [
     _case("v2_streamed_r1", 96, 96, dict(mode=0, resident=0, R=1, stack=0, epi_wg=1, out_bufs=2)),
     _case("v2_resident0_r1", 32, 32, dict(mode=0, resident=0, R=1), env={"SCI_CONV_RESIDENT": "0"}),
     _case("v2_streamed_r2", 128, 128, dict(mode=0, resident=0, R=2, epi_wg=1), H=601, round_tf32=1),
-    # epilogue warpgroups, direct stores (MODE 3), skip-add (MODE 1), 256 columns as two passes
+    # epilogue warpgroups, TF32-rounded stores, skip-add (MODE 1), 256 columns as two passes
     _case("v2_epi1", 32, 32, dict(mode=0, epi_wg=1, out_bufs=2, resident=1), env={"SCI_CONV_EPI_WG": "1"}),
     _case("v2_epi2", 64, 64, dict(mode=0, epi_wg=2, out_bufs=1), env={"SCI_CONV_EPI_WG": "2"}),
-    _case("v2_mode3", 64, 64, dict(mode=3, resident=1, R=4), env={"SCI_CONV_TMA_STORE": "0"}, round_tf32=1),
-    _case("v2_mode3_res", 32, 32, dict(mode=3, epi_wg=2), env={"SCI_CONV_TMA_STORE": "0"}, res=True),
+    _case("v2_r4_round", 64, 64, dict(mode=0, resident=1, R=4), round_tf32=1),
+    _case("v2_mode1_res_epi2", 32, 32, dict(mode=1, epi_wg=2), res=True),
     _case("v2_mode1_res", 32, 64, dict(mode=1, epi_wg=2), res=True, round_tf32=1),
     _case("v2_256_ps_res", 128, 256, dict(mode=1, ps=1), ps=1, relu=0, affine=False, res=True, n_plans=2),
     _case("v2_256_res", 64, 256, dict(mode=1, ps=0), res=True, n_plans=2),
@@ -679,8 +678,8 @@ WGRAD_CASES = [
     ("v2_two_m_tiles", 128, 256, 1, N_, H_, W_, {}, "wgrad v2", dict(swap=0, m_tiles=2)),
     ("v2_stride2", 64, 128, 2, N_, 37, 301, {}, "wgrad v2", dict(swap=0, fuse=1, stride=2)),
     ("v2_many_tiles", 64, 128, 1, N_, 250, 301, {}, "wgrad v2", dict(swap=0, fuse=1)),
-    ("v1", 64, 64, 1, N_, H_, W_, {"SCI_WGRAD_V2": "0", "SCI_WGRAD_V3": "0"}, "wgrad v1", dict(m_tiles=1)),
-    ("v1_stride2_two_m", 32, 256, 2, N_, 37, 301, {"SCI_WGRAD_V2": "0"}, "wgrad v1", dict(m_tiles=2, stride=2)),
+    ("v2_fuse_v3_off", 64, 64, 1, N_, H_, W_, {"SCI_WGRAD_V3": "0"}, "wgrad v2", dict(swap=0, fuse=1, m_tiles=1)),
+    ("v2_stride2_two_m", 32, 256, 2, N_, 37, 301, {}, "wgrad v2", dict(swap=0, fuse=1, m_tiles=2, stride=2)),
 ]
 
 

@@ -117,7 +117,9 @@ def test_projection(cuda, B):
     assert abs(float(sse) - want) / want < 1e-9
 
 
-@pytest.mark.parametrize("shape", [(64, 64, 2), (40, 136, 3), (256, 256, 8)])
+# (100, 76), (34, 130): ragged tiles in both directions; (256, 320): several full tiles; B = 1 .. 8 frames
+@pytest.mark.parametrize("shape", [(64, 64, 2), (40, 136, 3), (256, 256, 8), (64, 64, 8), (100, 76, 3), (256, 320, 2),
+                                   (34, 130, 1)])
 def test_tv_chambolle(cuda, shape):
     """TV prior vs the oracle restatement on ragged tile counts, incl. the early-stop decision per channel."""
     from adaptivepnp_sci_b200 import ops
@@ -125,13 +127,15 @@ def test_tv_chambolle(cuda, shape):
     H, W, B = shape
     rng = np.random.default_rng(H + W)
     yy, xx = np.mgrid[0:H // 2, 0:W // 2]
+    B += 1                                         # + one nearly flat frame
     stack = np.empty((H // 2, W // 2, B, 4), np.float32)
-    for t in range(B):
+    for t in range(B - 1):
         for ib in range(4):
             # large-amplitude channels make the energy converge fast: the reference loop stops at i=3 (sigma 8)
             # or i=1 (sigma 50); ordinary channels run all 5 iterations
             noise = (0.08, 8.0, 50.0)[(t + ib) % 3] * rng.standard_normal((H // 2, W // 2))
             stack[:, :, t, ib] = 0.5 + 0.3 * np.sin((xx + 3 * t) / 9.0) * np.cos((yy + ib) / 7.0) + noise
+    stack[:, :, B - 1] = 0.5 + 0.02 * rng.random((H // 2, W // 2, 4))
     ref, stops = tv_chambolle.denoise_tv_chambolle(stack.reshape(H // 2, W // 2, 4 * B), 0.1, n_iter_max=5,
                                                    multichannel=True, return_stops=True)
     x = _stack4_to_planar(stack, cuda)
@@ -147,11 +151,15 @@ def test_tv_chambolle(cuda, shape):
     # fused form: theta = clip(TV(x + c*b)), b' = b + s*(x - theta)
     b = 0.05 * torch.randn_like(x)
     b2 = torch.empty_like(b)
-    ops.tv_chambolle(x, b, -1.0, theta, b2, -1.0, True, ws)
+    nstop.zero_()
+    ops.tv_chambolle(x, b, -1.0, theta, b2, -1.0, True, ws, nstop_out=nstop)
     f = (x - b)
-    ref2 = tv_chambolle.denoise_tv_chambolle(_planar_to_stack4(f, H, W, B).reshape(H // 2, W // 2, 4 * B), 0.1,
-                                             n_iter_max=5, multichannel=True).reshape(H // 2, W // 2, B, 4)
-    ref2 = np.clip(ref2, 0, 1)
+    ref2, stops2 = tv_chambolle.denoise_tv_chambolle(_planar_to_stack4(f, H, W, B).reshape(H // 2, W // 2, 4 * B), 0.1,
+                                                     n_iter_max=5, multichannel=True, return_stops=True)
+    got_stops2 = nstop.cpu().numpy().reshape(B, 4)
+    assert np.array_equal(got_stops2, np.minimum(np.array(stops2).reshape(B, 4), 4)), got_stops2
+    assert (got_stops2 < 4).any()                  # the fix-up pass rewrote channels that stopped early
+    ref2 = np.clip(ref2.reshape(H // 2, W // 2, B, 4), 0, 1)
     assert _rel(_planar_to_stack4(theta, H, W, B), ref2) < REL
     want_b = (b - (x - theta)).cpu()
     assert torch.allclose(b2.cpu(), want_b, atol=1e-7, rtol=0)

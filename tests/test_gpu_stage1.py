@@ -77,29 +77,6 @@ def test_roundtrip_properties_512(cuda):
     assert float(((Ax - y).abs() * has).max()) < 1e-4
 
 
-@pytest.mark.parametrize("shape", [(64, 64, 8), (100, 76, 3), (256, 320, 2), (34, 130, 1)])
-def test_tv_kernel_generations_agree(cuda, shape, monkeypatch):
-    """The second-generation TV tile kernel (zero-bordered shared memory, column pairs) must reproduce the first one
-    exactly: same theta / b_out values and the same early-stop indices, incl. ragged tiles and image borders."""
-    from adaptivepnp_sci_b200 import ops
-    H, W, B = shape
-    g = torch.Generator().manual_seed(H * 1000 + W)
-    x = torch.rand(B, H, W, generator=g)
-    x[0] = x[0] * 0.02 + 0.5                                   # a nearly flat frame: its channels stop early
-    b = 0.05 * torch.randn(B, H, W, generator=g)
-    x, b = x.cuda(), b.cuda()
-    outs = {}
-    for v in ("0", "1"):
-        monkeypatch.setenv("SCI_TV_V2", v)
-        ws = ops.TvWorkspace(H, W, B, x.device)
-        theta, b_out = torch.empty_like(x), torch.empty_like(x)
-        nstop = torch.zeros(B * 4, dtype=torch.int32, device=x.device)
-        ops.tv_chambolle(x, b, -1.0, theta, b_out, -1.0, True, ws, nstop_out=nstop)
-        outs[v] = (theta.cpu(), b_out.cpu(), nstop.cpu())
-    assert torch.equal(outs["0"][2], outs["1"][2])
-    assert torch.equal(outs["0"][0], outs["1"][0]) and torch.equal(outs["0"][1], outs["1"][1])
-
-
 @pytest.mark.parametrize("impl", ["ref", "tc"])
 def test_stage1_deep_branches_vs_golden(cuda, impl, monkeypatch):
     """Deep branches of admm_denoise_bayer_demosaic_pre ('ffdnet_color' / 'fastdvd_color', dvp...online.py:456-503, :552)

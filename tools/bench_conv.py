@@ -26,7 +26,7 @@ def main():
     for N, H, W, Ci, Co, stride, ps in SHAPES:
         conv = torch.nn.Conv2d(Ci, Co, 3, stride=stride, padding=1, bias=False).to(dev)
         L = engine.ConvLayer(conv, None, relu=True, stride=stride, ps=ps)
-        L.refresh_fwd(True)
+        engine.OpTable(L.fwd_ops(True), dev).run()
         x = torch.rand(N, H, W, L.Ci_pad, device=dev)
         Ho, Wo = (H // stride, W // stride) if not ps else (2 * H, 2 * W)
         y = torch.empty(N, Ho, Wo, L.out_ch, device=dev)
