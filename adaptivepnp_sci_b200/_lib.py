@@ -40,6 +40,9 @@ PROTOTYPES = {
     "sci_project_stage1": [_p, _p, _p, _p, _p, _p, _l, _i, _f, _f, _p, _p, _p],
     "sci_project_stage2": [_p, _p, _p, _p, _p, _p, _l, _i, _d, _d, _p],
     "sci_tv_chambolle2d": [_p, _p, _f, _p, _p, _f, _i, _i, _i, _i, _f, _f, _i, _p, _sz, _p, _p],
+    "sci_tv_strip_main": [_p, _p, _f, _p, _p, _f, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, ctypes.c_uint, _p, _f, _f, _i,
+                          _p, _sz, _p, _p],
+    "sci_tv_strip_finish": [_p, _p, _f, _p, _p, _f, _i, _i, _i, _i, _i, _i, _p, _p, _f, _f, _i, _p, _sz, _p, _i, _p, _p],
     "sci_malvar2004": [_p, _p, _f, _p, _f, _p, _p, _i, _i, _i, _p],
     "sci_dual_update_rgb": [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p],
     "sci_dual_update_stage1": [_p, _p, _p, _p, _i, _i, _i, _i, _p, _p, _p],
@@ -67,6 +70,7 @@ PROTOTYPES = {
     "sci_p2p_open_handle": [_p, _p],
     "sci_p2p_close_handle": [_p],
     "sci_halo_send": [_p, _i, _i, _i, _i, _p, _p, _p, _p, ctypes.c_uint, _p, _p],
+    "sci_halo_send_tv": [_p, _p, _f, _i, _i, _i, _i, _p, _p, _p, _p, ctypes.c_uint, _p, _p],
     "sci_halo_assemble": [_p, _i, _i, _i, _i, _i, _p, _p, _p, _p, ctypes.c_uint, _p, _p, _p],
     "sci_fastdvd_pack_input_half": [_p, _f, _p, _i, _i, _i, _i, _p],
     "sci_conv_unpack_wgrad": [_p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
@@ -103,7 +107,7 @@ PROTOTYPES = {
     "sci_axpy": [_p, _f, _p, _p, _l, _p],
     "sci_adam_step": [_p, _p, _p, _p, _l, _d, _d, _d, _d, _i, _p],
 }
-_SPECIAL_RESTYPE = {"sci_last_error": ctypes.c_char_p, "sci_tv_workspace_bytes": _sz}
+_SPECIAL_RESTYPE = {"sci_last_error": ctypes.c_char_p, "sci_tv_workspace_bytes": _sz, "sci_tv_strip_workspace_bytes": _sz}
 
 for _name, _args in PROTOTYPES.items():
     _fn = getattr(lib, _name)
@@ -113,6 +117,8 @@ lib.sci_last_error.argtypes = []
 lib.sci_last_error.restype = ctypes.c_char_p
 lib.sci_tv_workspace_bytes.argtypes = [_i, _i, _i]
 lib.sci_tv_workspace_bytes.restype = _sz
+lib.sci_tv_strip_workspace_bytes.argtypes = [_i, _i, _i]
+lib.sci_tv_strip_workspace_bytes.restype = _sz
 
 
 class SciError(RuntimeError):
@@ -137,7 +143,8 @@ def check(rc, what):
 
 
 # kernel launches issued through the C ABI since import (bench.py reports the count inside its timed region)
-KERNELS_PER_CALL = {"sci_tv_chambolle2d": 3, "sci_version": 0, "sci_conv_tc_available": 0, "sci_host_legacy_normal": 0}
+KERNELS_PER_CALL = {"sci_tv_chambolle2d": 3, "sci_tv_strip_main": 2, "sci_tv_strip_finish": 2, "sci_version": 0,
+                    "sci_conv_tc_available": 0, "sci_host_legacy_normal": 0}
 launch_count = 0
 
 

@@ -59,6 +59,19 @@ __device__ __forceinline__ float4 ldg_stream4(const float* p) {
     return r;
 }
 
+// Flag word of the peer-to-peer halo exchange (sci_p2p.cu), read with system-scope acquire semantics, and the
+// nanosecond clock its bounded waits are measured with.
+__device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) {
+    unsigned v;
+    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
+    return t;
+}
+
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

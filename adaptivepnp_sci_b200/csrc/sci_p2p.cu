@@ -15,22 +15,14 @@
 // A slot of parity p is rewritten at exchange seq + 2, which a neighbour can only reach after it has received my data of
 // exchange seq + 1, i.e. after my assemble kernel of exchange seq has drained the slot (stream order): no write-after-read
 // hazard.  The wait is bounded (about 10 s of globaltimer): a lost neighbour sets an error word instead of hanging the GPU.
+// The TV prior's exchange (halo_send_tv_kernel) follows the same protocol; its receiver is the TV strip kernel itself
+// (sci_tv.cu), which reads the slots in place in its main and fix-up passes - the last reader before the next send.
 #include "sci_common.cuh"
 
 namespace {
 
-__device__ __forceinline__ unsigned ld_acquire_sys(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
 __device__ __forceinline__ void st_release_sys(unsigned* p, unsigned v) {
     asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
 }
 
 // blockIdx.y = side (0: my top rows -> upper neighbour, 1: my bottom rows -> lower neighbour)
@@ -54,6 +46,42 @@ __global__ void __launch_bounds__(256) halo_send_kernel(const float* __restrict_
         const unsigned total = gridDim.x * gridDim.y;
         if (atomicAdd(done, 1u) == total - 1) {
             *done = 0;                                   // ready for the next exchange (stream-ordered)
+            __threadfence_system();
+            if (up_flag) st_release_sys(up_flag, seq);
+            if (down_flag) st_release_sys(down_flag, seq);
+        }
+    }
+}
+
+// The TV prior's halo: f = x + c_b*b of the boundary rows, formed here and stored straight into the neighbours' slots
+// (the receiving TV kernel reads the slots in place, there is no assembled strip).  This file is compiled with FMA
+// contraction, so the product and the sum are written as separately rounded ops: the same bits as the TV kernel's load.
+__global__ void __launch_bounds__(256) halo_send_tv_kernel(const float* __restrict__ x, const float* __restrict__ b, float c_b,
+                                                           int planes, int rows, int W, int halo, float* up_dst, float* down_dst,
+                                                           unsigned* up_flag, unsigned* down_flag, unsigned seq, unsigned* done) {
+    const int side = blockIdx.y;
+    float* dst = side == 0 ? up_dst : down_dst;
+    if (dst != nullptr) {
+        const int r0 = side == 0 ? 0 : rows - halo;
+        const long per_plane = (long)halo * W, n2 = (long)planes * per_plane / 2;
+        for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n2; i += (long)gridDim.x * blockDim.x) {
+            const long e = i * 2, pl = e / per_plane, off = e - pl * per_plane;      // W even: a float2 stays inside a row
+            const long src = (pl * rows + r0) * W + off;
+            float2 v = *reinterpret_cast<const float2*>(x + src);
+            if (b) {
+                const float2 bb = *reinterpret_cast<const float2*>(b + src);
+                v.x = __fadd_rn(v.x, __fmul_rn(c_b, bb.x));
+                v.y = __fadd_rn(v.y, __fmul_rn(c_b, bb.y));
+            }
+            *reinterpret_cast<float2*>(dst + e) = v;                                 // store into the PEER's memory
+        }
+    }
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const unsigned total = gridDim.x * gridDim.y;
+        if (atomicAdd(done, 1u) == total - 1) {
+            *done = 0;
             __threadfence_system();
             if (up_flag) st_release_sys(up_flag, seq);
             if (down_flag) st_release_sys(down_flag, seq);
@@ -139,6 +167,20 @@ extern "C" int sci_halo_send(const float* own, int planes, int rows, int W, int 
     halo_send_kernel<<<dim3(gx, 2), 256, 0, sci_stream(stream)>>>(own, planes, rows, W, halo, up_dst, down_dst, up_flag, down_flag,
                                                                   seq, done_counter);
     SCI_CHECK_LAUNCH("halo_send");
+    return SCI_OK;
+}
+
+extern "C" int sci_halo_send_tv(const float* x, const float* b, float c_b, int planes, int rows, int W, int halo, float* up_dst,
+                                float* down_dst, unsigned* up_flag, unsigned* down_flag, unsigned seq, unsigned* done_counter,
+                                void* stream) {
+    SCI_REQUIRE(x && planes > 0 && rows > 0 && W > 0 && W % 2 == 0 && halo > 0 && halo <= rows && done_counter, "halo_send_tv");
+    SCI_REQUIRE((up_dst == nullptr) == (up_flag == nullptr) && (down_dst == nullptr) == (down_flag == nullptr),
+                "halo_send_tv: dst / flag pairs");
+    const long n2 = (long)planes * halo * W / 2;
+    const int gx = (int)max(1L, min((long)SCI_NUM_SMS * 4, (n2 + 255) / 256));
+    halo_send_tv_kernel<<<dim3(gx, 2), 256, 0, sci_stream(stream)>>>(x, b, c_b, planes, rows, W, halo, up_dst, down_dst,
+                                                                     up_flag, down_flag, seq, done_counter);
+    SCI_CHECK_LAUNCH("halo_send_tv");
     return SCI_OK;
 }
 

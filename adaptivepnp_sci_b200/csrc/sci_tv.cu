@@ -49,12 +49,28 @@ constexpr int TV2_PAIRS = TV_RW / 2;               // 40 column pairs
 constexpr int TV2_RG = TV_THREADS / TV2_PAIRS;     // 8 row groups
 constexpr int TV2_RPT = TV_RH / TV2_RG;            // 6 rows per thread
 
+// Row-strip form (sci_tv_strip_*): the launch covers local rows [0, rows) of an H_total-row image whose first row is the
+// global row row0 (even).  Border masks use global rows; the 8 rows above / below the strip are read from halo buffers
+// [B][TV_HALO][W] that already hold f = x + c_b*b (null at a true image border, where the rows are zero as in the
+// un-tiled kernel).  Rows further out than the halo may feed only pixels of the halo itself, never an own row.
+struct TvStrip {
+    int row0, H_total;
+    const float* halo_top;
+    const float* halo_bot;
+    const unsigned* flag_top;     // peer-to-peer flag words to wait for before the halo is read (null: nothing to wait for)
+    const unsigned* flag_bot;
+    unsigned seq;
+    unsigned* err;
+};
+
 // is_fix = 0: main pass (all channels run to n_iter_max, energies recorded)
 // is_fix = 1: fix-up pass (only channels with nstop < last are rewritten)
+// STRIP = false: the whole image, H rows (the TvStrip argument is unused).  STRIP = true: H is the strip's row count.
+template <bool STRIP>
 __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
     const float* __restrict__ x, const float* __restrict__ b, float c_b, float* __restrict__ theta,
     float* __restrict__ b_out, float s_b, int clip, int H, int W, float tau, float tw, int last_iter,
-    double* __restrict__ epart, const int* __restrict__ nstop, int is_fix) {
+    double* __restrict__ epart, const int* __restrict__ nstop, int is_fix, TvStrip strip) {
     extern __shared__ float smem[];
     float* sf = smem;
     float* so = sf + TV2_N;
@@ -65,14 +81,31 @@ __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
     const int t = blockIdx.z;
     const int nblk = gridDim.x * gridDim.y, blk = blockIdx.y * gridDim.x + blockIdx.x;
     if (threadIdx.x < 4) s_stop[threadIdx.x] = is_fix ? nstop[t * 4 + threadIdx.x] : last_iter;
+    if (STRIP && threadIdx.x == 0) {
+        // halo rows delivered peer to peer: a tile that reads them waits for the neighbour's sequence number (bounded, as in
+        // halo_assemble_kernel: a lost neighbour sets the error word instead of hanging the GPU)
+        const unsigned long long t0 = globaltimer_ns();
+#pragma unroll
+        for (int side = 0; side < 2; ++side) {
+            const unsigned* flag = side == 0 ? (blockIdx.y == 0 ? strip.flag_top : nullptr)
+                                             : ((int)blockIdx.y * TV_TH + TV_TH + TV_HALO > H ? strip.flag_bot : nullptr);
+            if (!flag) continue;
+            while ((int)(ld_acquire_sys(flag) - strip.seq) < 0) {
+                if (globaltimer_ns() - t0 > 10000000000ull) { atomicExch(strip.err, 1u + side); break; }
+                __nanosleep(200);
+            }
+        }
+    }
     __syncthreads();
     if (is_fix && s_stop[0] >= last_iter && s_stop[1] >= last_iter && s_stop[2] >= last_iter && s_stop[3] >= last_iter)
         return;
 
+    const int Himg = STRIP ? strip.H_total : H;                   // image height, for the border masks
+    const int goff = STRIP ? strip.row0 : 0;                      // global row of local row 0
     const long plane = (long)H * W;
     const float* xp = x + t * plane;
     const float* bp = b ? b + t * plane : nullptr;
-    const int gr0 = blockIdx.y * TV_TH - TV_HALO, gc0 = blockIdx.x * TV_TW - TV_HALO;    // both even
+    const int gr0 = goff + blockIdx.y * TV_TH - TV_HALO, gc0 = blockIdx.x * TV_TW - TV_HALO;    // both even
 
     // zero everything once (borders stay zero for the whole kernel)
     {
@@ -92,13 +125,19 @@ __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
     // ---- load f = x + c_b*b
 #pragma unroll
     for (int k = 0; k < TV2_RPT; ++k) {
-        const int gr = gr0 + ry + k * TV2_RG, i = base + k * TV2_RG * TV2_P;
+        const int gr = gr0 + ry + k * TV2_RG, lr = gr - goff, i = base + k * TV2_RG * TV2_P;
         float2 v = make_float2(0.f, 0.f);
-        if (col_in && gr >= 0 && gr < H) {
-            v = *reinterpret_cast<const float2*>(xp + (long)gr * W + gc);
-            if (bp) {
-                const float2 bb = *reinterpret_cast<const float2*>(bp + (long)gr * W + gc);
-                v.x = v.x + c_b * bb.x; v.y = v.y + c_b * bb.y;
+        if (col_in && gr >= 0 && gr < Himg) {
+            if (!STRIP || (lr >= 0 && lr < H)) {
+                v = *reinterpret_cast<const float2*>(xp + (long)lr * W + gc);
+                if (bp) {
+                    const float2 bb = *reinterpret_cast<const float2*>(bp + (long)lr * W + gc);
+                    v.x = v.x + c_b * bb.x; v.y = v.y + c_b * bb.y;
+                }
+            } else if (lr < 0) {
+                v = *reinterpret_cast<const float2*>(strip.halo_top + ((long)t * TV_HALO + lr + TV_HALO) * W + gc);
+            } else if (lr < H + TV_HALO) {
+                v = *reinterpret_cast<const float2*>(strip.halo_bot + ((long)t * TV_HALO + lr - H) * W + gc);
             }
         }
         *reinterpret_cast<float2*>(sf + i) = v;
@@ -118,7 +157,7 @@ __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
             // ---- phase A: d = -div p, out = f + d; write the result of the channels stopping here
 #pragma unroll 2
             for (int k = 0; k < TV2_RPT; ++k) {
-                const int rr = ry + k * TV2_RG, gr = gr0 + rr, i = base + k * TV2_RG * TV2_P;
+                const int rr = ry + k * TV2_RG, lr = gr0 - goff + rr, i = base + k * TV2_RG * TV2_P;
                 const float2 p0 = *reinterpret_cast<const float2*>(sp0 + i), p1 = *reinterpret_cast<const float2*>(sp1 + i);
                 const float2 pu = *reinterpret_cast<const float2*>(sp0 + i - 2 * TV2_P);
                 const float2 pl = *reinterpret_cast<const float2*>(sp1 + i - 2);
@@ -128,12 +167,12 @@ __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
                 dx += pl.x; dy += pl.y;
                 const float ox = f.x + dx, oy = f.y + dy;
                 *reinterpret_cast<float2*>(so + i) = make_float2(ox, oy);
-                if (col_interior && rr >= TV_HALO && rr < TV_HALO + TV_TH && gr < H) {
+                if (col_interior && rr >= TV_HALO && rr < TV_HALO + TV_TH && lr < H) {     // own rows only
                     if (it < TV_MAX_UPD && !is_fix) {
                         e_d[it][0] += (double)(dx * dx);
                         e_d[it][1] += (double)(dy * dy);
                     }
-                    const long g = (long)gr * W + gc;
+                    const long g = (long)lr * W + gc;
                     const bool w0 = it == stop0 && (!is_fix || stop0 < last_iter);
                     const bool w1 = it == stop1 && (!is_fix || stop1 < last_iter);
                     if (w0 || w1) {
@@ -162,15 +201,15 @@ __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
 #pragma unroll 2
         for (int k = 0; k < TV2_RPT; ++k) {
             const int rr = ry + k * TV2_RG, gr = gr0 + rr, i = base + k * TV2_RG * TV2_P;
-            const bool in_img = col_in && gr >= 0 && gr < H;
-            const bool has_dn = in_img && gr + 2 < H, has_rt = in_img && col_right;
+            const bool in_img = col_in && gr >= 0 && gr < Himg;
+            const bool has_dn = in_img && gr + 2 < Himg, has_rt = in_img && col_right;
             const float2 o = *reinterpret_cast<const float2*>(so + i);
             const float2 od = *reinterpret_cast<const float2*>(so + i + 2 * TV2_P);
             const float2 orr = *reinterpret_cast<const float2*>(so + i + 2);
             const float g0x = has_dn ? od.x - o.x : 0.f, g0y = has_dn ? od.y - o.y : 0.f;
             const float g1x = has_rt ? orr.x - o.x : 0.f, g1y = has_rt ? orr.y - o.y : 0.f;
             const float nx = sqrtf(g0x * g0x + g1x * g1x), ny = sqrtf(g0y * g0y + g1y * g1y);
-            if (col_interior && rr >= TV_HALO && rr < TV_HALO + TV_TH && gr < H && !is_fix) {
+            if (col_interior && rr >= TV_HALO && rr < TV_HALO + TV_TH && gr - goff < H && !is_fix) {
                 e_n[it][0] += (double)nx;
                 e_n[it][1] += (double)ny;
             }
@@ -207,9 +246,48 @@ __global__ void __launch_bounds__(TV_THREADS, 3) tv_chambolle2_kernel(
     }
 }
 
-// One block per channel: fixed-order (deterministic) reduction of the per-block partials, then the
-// reference's stopping rule  |E_prev - E_i| < eps * E_init  (i >= 1).
+// Fixed-order (deterministic) reduction of one channel's per-block partials: strided per-thread sums, then a tree.  The
+// channel's 8 sums (q = k*2 + kind) end in sm[0][0..7].
 constexpr int TV_DEC_THREADS = 128;
+__device__ __forceinline__ void tv_channel_sums(const double* __restrict__ epart, int nblk, int t, int phase,
+                                                double (*sm)[8]) {
+    double acc[8];
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {        // q = k*2 + kind
+        const double* p = epart + ((((size_t)t * 4 + (q >> 1)) * 2 + (q & 1)) * 4 + phase) * nblk;
+        double s = 0.0;
+        for (int j = threadIdx.x; j < nblk; j += TV_DEC_THREADS) s += p[j];
+        acc[q] = s;
+    }
+#pragma unroll
+    for (int q = 0; q < 8; ++q) sm[threadIdx.x][q] = acc[q];
+    __syncthreads();
+    for (int off = TV_DEC_THREADS / 2; off > 0; off >>= 1) {
+        if (threadIdx.x < off) {
+#pragma unroll
+            for (int q = 0; q < 8; ++q) sm[threadIdx.x][q] += sm[threadIdx.x + off][q];
+        }
+        __syncthreads();
+    }
+}
+
+// The reference's stopping rule  |E_prev - E_i| < eps * E_init  (i >= 1) on a channel's 8 energy sums.
+__device__ __forceinline__ int tv_stop_rule(const double* e, double weight, double eps, double n_pix, int last_iter) {
+    double E_init = 0.0, E_prev = 0.0;
+    int stop = last_iter;
+    for (int k = 0; k < TV_MAX_UPD && k < last_iter; ++k) {
+        double E = e[k * 2 + 0];
+        E += weight * e[k * 2 + 1];
+        E /= n_pix;
+        if (k == 0) { E_init = E; E_prev = E; }
+        else if (fabs(E_prev - E) < eps * E_init) { stop = k; break; }
+        else E_prev = E;
+    }
+    return stop;
+}
+
+// One block per channel: the reduction of tv_channel_sums, then the stopping rule (kept written out: the un-tiled decision
+// compiles exactly as before).
 __global__ void __launch_bounds__(TV_DEC_THREADS) tv_decide_kernel(const double* __restrict__ epart, int nblk, double weight,
                                                                    double eps, double n_pix, int last_iter,
                                                                    int* __restrict__ nstop, int* __restrict__ nstop_out) {
@@ -249,6 +327,36 @@ __global__ void __launch_bounds__(TV_DEC_THREADS) tv_decide_kernel(const double*
     }
 }
 
+// Local half of a strip's decision: the same reduction as tv_decide_kernel, written out as esum[4B][8] for the
+// cross-rank gather.  With one strip these are the un-tiled sums, bit for bit.
+__global__ void __launch_bounds__(TV_DEC_THREADS) tv_strip_sums_kernel(const double* __restrict__ epart, int nblk,
+                                                                       double* __restrict__ esum) {
+    __shared__ double sm[TV_DEC_THREADS][8];
+    const int ch = blockIdx.x, t = ch >> 2, phase = ch & 3;
+    tv_channel_sums(epart, nblk, t, phase, sm);
+    if (threadIdx.x < 8) esum[ch * 8 + threadIdx.x] = sm[0][threadIdx.x];
+}
+
+// Finish half: esum_all[world][4B][8] summed in rank order (every rank gets the same bits, hence the same decision),
+// then the stopping rule.  One thread per channel.
+__global__ void __launch_bounds__(TV_DEC_THREADS) tv_strip_decide_kernel(const double* __restrict__ esum_all, int world,
+                                                                         int nch, double weight, double eps, double n_pix,
+                                                                         int last_iter, int* __restrict__ nstop,
+                                                                         int* __restrict__ nstop_out) {
+    const int ch = blockIdx.x * TV_DEC_THREADS + threadIdx.x;
+    if (ch >= nch) return;
+    double e[8];
+#pragma unroll
+    for (int q = 0; q < 8; ++q) e[q] = esum_all[ch * 8 + q];
+    for (int r = 1; r < world; ++r) {
+#pragma unroll
+        for (int q = 0; q < 8; ++q) e[q] += esum_all[((size_t)r * nch + ch) * 8 + q];
+    }
+    const int stop = tv_stop_rule(e, weight, eps, n_pix, last_iter);
+    nstop[ch] = stop;
+    if (nstop_out) nstop_out[ch] = stop;
+}
+
 }  // namespace
 
 extern "C" size_t sci_tv_workspace_bytes(int H, int W, int B) {
@@ -273,7 +381,7 @@ extern "C" int sci_tv_chambolle2d(const float* x, const float* b, float c_b, flo
     double* epart = reinterpret_cast<double*>(workspace);
     int* nstop = reinterpret_cast<int*>(epart + tv_epart_count(B, nblk));
     const size_t smem = (size_t)4 * TV2_N * sizeof(float);
-    const cudaError_t e = sci_smem_limit((const void*)tv_chambolle2_kernel, (int)smem);
+    const cudaError_t e = sci_smem_limit((const void*)tv_chambolle2_kernel<false>, (int)smem);
     if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "tv: smem attribute", e);
     const int last_iter = n_iter_max - 1;              // index of the last iterate (4 for n_iter_max=5)
     const float tau = 0.25f;                            // 1/(2*ndim), ndim = 2
@@ -282,13 +390,107 @@ extern "C" int sci_tv_chambolle2d(const float* x, const float* b, float c_b, flo
         // n_iter_max = 1 returns the input unchanged
         return sci_fail(SCI_EUNSUPPORTED, "tv: n_iter_max = 1 is the identity; not routed through the kernel");
     }
-    tv_chambolle2_kernel<<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nullptr, 0);
+    tv_chambolle2_kernel<false><<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nullptr, 0,
+                                                             TvStrip{});
     SCI_CHECK_LAUNCH("tv main pass");
     const int nch = B * 4;
     tv_decide_kernel<<<nch, TV_DEC_THREADS, 0, st>>>(epart, nblk, (double)weight, (double)eps,
                                                      (double)(H / 2) * (double)(W / 2), last_iter, nstop, nstop_out);
     SCI_CHECK_LAUNCH("tv decide");
-    tv_chambolle2_kernel<<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nstop, 1);
+    tv_chambolle2_kernel<false><<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, H, W, tau, tw, last_iter, epart, nstop, 1,
+                                                             TvStrip{});
     SCI_CHECK_LAUNCH("tv fix-up pass");
+    return SCI_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Row strips of one frame (one strip per GPU).  A pixel's result depends only on rows within +-TV_HALO, for all
+// n_iter_max <= 5 inner iterations, so one exchange of TV_HALO rows of f per call suffices; the only global coupling is
+// the early stop, whose energies are reduced locally (sci_tv_strip_main), gathered across ranks by the caller and
+// summed in rank order (sci_tv_strip_finish).
+// ---------------------------------------------------------------------------------------------------
+extern "C" size_t sci_tv_strip_workspace_bytes(int rows, int W, int B) { return sci_tv_workspace_bytes(rows, W, B); }
+
+namespace {
+
+// Every check runs before any CUDA call.
+int tv_strip_check(const float* x, const float* b, const float* theta, const float* b_out, int rows, int W, int B, int row0,
+                   int H_total, const float* halo_top, const float* halo_bot, int n_iter_max, const void* ws, size_t ws_bytes) {
+    SCI_REQUIRE(x && theta && ws, "tv_strip: null pointer");
+    SCI_REQUIRE((b == nullptr) == (b_out == nullptr), "tv_strip: b and b_out go together");
+    SCI_REQUIRE(b == nullptr || b != b_out, "tv_strip: b_out must not alias b");
+    SCI_REQUIRE(W >= 2 && W % 2 == 0 && B > 0 && B <= 65535, "tv_strip: shape");
+    SCI_REQUIRE(rows >= TV_HALO && rows % 2 == 0 && row0 >= 0 && row0 % 2 == 0 && row0 + rows <= H_total,
+                "tv_strip: rows and row0 must be even, rows >= 8, and the strip must lie inside the image");
+    SCI_REQUIRE((row0 > 0) == (halo_top != nullptr) && (row0 + rows < H_total) == (halo_bot != nullptr),
+                "tv_strip: a halo buffer is given exactly when a neighbouring strip exists");
+    if (n_iter_max < 2 || n_iter_max > TV_MAX_UPD + 1)
+        return sci_fail(SCI_EUNSUPPORTED, "tv_strip: n_iter_max must be in 2..5 (the reference uses 5)");
+    if (ws_bytes < sci_tv_strip_workspace_bytes(rows, W, B)) return sci_fail(SCI_EWORKSPACE, "tv_strip: workspace too small");
+    return SCI_OK;
+}
+
+}  // namespace
+
+extern "C" int sci_tv_strip_main(const float* x, const float* b, float c_b, float* theta, float* b_out, float s_b, int clip,
+                                 int rows, int W, int B, int row0, int H_total, const float* halo_top, const float* halo_bot,
+                                 const unsigned* flag_top, const unsigned* flag_bot, unsigned seq, unsigned* err, float weight,
+                                 float eps, int n_iter_max, void* workspace, size_t workspace_bytes, double* esum_out,
+                                 void* stream) {
+    const int rc = tv_strip_check(x, b, theta, b_out, rows, W, B, row0, H_total, halo_top, halo_bot, n_iter_max, workspace,
+                                  workspace_bytes);
+    if (rc != SCI_OK) return rc;
+    SCI_REQUIRE(esum_out, "tv_strip: null esum_out");
+    SCI_REQUIRE((flag_top == nullptr || halo_top) && (flag_bot == nullptr || halo_bot) && (!(flag_top || flag_bot) || err),
+                "tv_strip: a flag word needs its halo buffer and the error word");
+    (void)eps;
+    cudaStream_t st = sci_stream(stream);
+    const dim3 grid(sci_ceil_div(W, TV_TW), sci_ceil_div(rows, TV_TH), B);
+    const int nblk = grid.x * grid.y;
+    double* epart = reinterpret_cast<double*>(workspace);
+    const size_t smem = (size_t)4 * TV2_N * sizeof(float);
+    const cudaError_t e = sci_smem_limit((const void*)tv_chambolle2_kernel<true>, (int)smem);
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "tv_strip: smem attribute", e);
+    const float tau = 0.25f;
+    const float tw = (float)(0.25 / (double)weight);
+    const TvStrip strip{row0, H_total, halo_top, halo_bot, flag_top, flag_bot, seq, err};
+    tv_chambolle2_kernel<true><<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, rows, W, tau, tw, n_iter_max - 1, epart,
+                                                    nullptr, 0, strip);
+    SCI_CHECK_LAUNCH("tv_strip main pass");
+    tv_strip_sums_kernel<<<B * 4, TV_DEC_THREADS, 0, st>>>(epart, nblk, esum_out);
+    SCI_CHECK_LAUNCH("tv_strip sums");
+    return SCI_OK;
+}
+
+extern "C" int sci_tv_strip_finish(const float* x, const float* b, float c_b, float* theta, float* b_out, float s_b, int clip,
+                                   int rows, int W, int B, int row0, int H_total, const float* halo_top, const float* halo_bot,
+                                   float weight, float eps, int n_iter_max, void* workspace, size_t workspace_bytes,
+                                   const double* esum_all, int world, int* nstop_out, void* stream) {
+    const int rc = tv_strip_check(x, b, theta, b_out, rows, W, B, row0, H_total, halo_top, halo_bot, n_iter_max, workspace,
+                                  workspace_bytes);
+    if (rc != SCI_OK) return rc;
+    SCI_REQUIRE(esum_all && world >= 1, "tv_strip: esum_all / world");
+    cudaStream_t st = sci_stream(stream);
+    const dim3 grid(sci_ceil_div(W, TV_TW), sci_ceil_div(rows, TV_TH), B);
+    const int nblk = grid.x * grid.y, nch = B * 4;
+    double* epart = reinterpret_cast<double*>(workspace);
+    int* nstop = reinterpret_cast<int*>(epart + tv_epart_count(B, nblk));
+    const size_t smem = (size_t)4 * TV2_N * sizeof(float);
+    const cudaError_t e = sci_smem_limit((const void*)tv_chambolle2_kernel<true>, (int)smem);
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "tv_strip: smem attribute", e);
+    const int last_iter = n_iter_max - 1;
+    const float tau = 0.25f;
+    const float tw = (float)(0.25 / (double)weight);
+    tv_strip_decide_kernel<<<sci_ceil_div(nch, TV_DEC_THREADS), TV_DEC_THREADS, 0, st>>>(
+        esum_all, world, nch, (double)weight, (double)eps, (double)(H_total / 2) * (double)(W / 2), last_iter, nstop, nstop_out);
+    SCI_CHECK_LAUNCH("tv_strip decide");
+    // The fix-up pass reads the halo buffers again, without waiting: the main pass (earlier in this stream) has seen the
+    // flags.  A peer-to-peer slot of parity p is rewritten only at exchange seq + 2, which the neighbour can issue only
+    // after it has received this rank's halo of exchange seq + 1; this rank sends that after this pass in stream order,
+    // so the slot is not overwritten while this pass reads it (sci_p2p.cu header).
+    const TvStrip strip{row0, H_total, halo_top, halo_bot, nullptr, nullptr, 0u, nullptr};
+    tv_chambolle2_kernel<true><<<grid, TV_THREADS, smem, st>>>(x, b, c_b, theta, b_out, s_b, clip, rows, W, tau, tw, last_iter, epart, nstop,
+                                                    1, strip);
+    SCI_CHECK_LAUNCH("tv_strip fix-up pass");
     return SCI_OK;
 }

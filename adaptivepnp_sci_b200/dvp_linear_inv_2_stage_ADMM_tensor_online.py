@@ -110,7 +110,7 @@ def admm_denoise_bayer_demosaic_pre(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
                                     x0_bayer=None,
                                     X_orig=None, model=None, show_iqa=True, demosaic_method='malvar2004', lr_=0.000001,
                                     inital_iter=1, interval_iter=5, logf=None, useGPU=True, device=0, update_=False,
-                                    update_per_iter=1):
+                                    update_per_iter=1, tile=None, return_device=False):
     """Stage 1: ADMM/GAP with the TV prior (warm start).
 
     y_bayer [H,W], Phi_bayer [H,W,B] float32 numpy.  Returns
@@ -120,9 +120,17 @@ def admm_denoise_bayer_demosaic_pre(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
     ONE dual variable), the 6-tuple ``(xbgr3_np, x_bayer_np, psnr_, ssim_, psnr_all, model)`` (:552).
     The reference's 'PPP' branch compares ``denoiser.lower()`` with an upper-case literal (:411) and can
     never be taken.
+    ``tile`` (extension, ``parallel.TileContext``, 'tv' only): row-strip tiling of one large frame over the ranks.  Every
+    rank passes ITS rows of y / Phi / x0 / X_orig; the TV prior exchanges 8 rows of its input with the neighbouring ranks
+    and all-gathers its early-stop energies once per iteration, and the returned arrays are the full frame.
+    ``return_device`` (extension, 'tv' only) returns x as a CUDA tensor in the ``x0_bayer`` layout [H,W,B] (tiled: this
+    rank's rows) instead of the tuple - a warm start that stage 2 takes without a gather or a host round trip.
     """
     name = denoiser if denoiser == 'tv' else str(denoiser).lower()
     if name in ('ffdnet_color', 'fastdvd_color'):
+        if tile is not None or return_device:
+            raise NotImplementedError("tiled stage 1 and return_device cover the TV prior; the deep stage-1 branches "
+                                      "('%s') run on a whole frame" % name)
         return _stage1_deep(y_bayer, Phi_bayer, _lambda, gamma, name, denoiser, iter_max, noise_estimate, sigma, x0_bayer,
                             X_orig, model, show_iqa, demosaic_method, lr_, inital_iter, interval_iter, logf, update_,
                             update_per_iter)
@@ -130,9 +138,17 @@ def admm_denoise_bayer_demosaic_pre(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
         raise ValueError('Unsupported denoiser {}!'.format(denoiser))
     sigma, iter_max = _as_list(sigma, iter_max)
     pb = _Problem(y_bayer, Phi_bayer, x0_bayer, X_orig)
-    ws = ops.TvWorkspace(pb.H, pb.W, pb.B, pb.y.device)
+    if tile is not None:
+        if pb.H != tile.rows or pb.W != tile.W:
+            raise ValueError("tiled mode: pass this rank's rows (%d x %d), got %d x %d" % (tile.rows, tile.W, pb.H, pb.W))
+        tile.enable_p2p(pb.B, ops.TV_HALO)                               # the TV halo goes peer to peer over NVLink
+        ws = ops.TvStripWorkspace(pb.H, pb.W, pb.B, pb.y.device)
+        tv = tile.tv_chambolle
+    else:
+        ws = ops.TvWorkspace(pb.H, pb.W, pb.B, pb.y.device)
+        tv = ops.tv_chambolle
     n_total = int(sum(iter_max))
-    want_iqa = bool(show_iqa and X_orig is not None)
+    want_iqa = bool(show_iqa and X_orig is not None and not return_device)
     sse = torch.zeros(max(n_total, 1), dtype=torch.float64, device=pb.y.device) if want_iqa else None
     b_next = torch.empty_like(pb.b)
     theta, b, x = pb.theta, pb.b, pb.x
@@ -144,10 +160,14 @@ def admm_denoise_bayer_demosaic_pre(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
             ops.project_stage1(theta, b, pb.phi, pb.y, pb.phisum, x, _lambda, gamma,
                                orig=pb.orig if want_iqa else None, sse=sse[k:k + 1] if want_iqa else None)
             # theta = clip(TV(x - b)); b = b - (x - theta)                               (:403-407, :501-503)
-            ops.tv_chambolle(x, b, -1.0, theta, b_next, -1.0, True, ws, weight=0.1, n_iter_max=5)
+            tv(x, b, -1.0, theta, b_next, -1.0, True, ws, weight=0.1, n_iter_max=5)
             b, b_next = b_next, b
             sched.append(nsig)
             k += 1
+    if return_device:
+        return ops.planar_to_pixlast(x, 1, pb.B).view(pb.H, pb.W, pb.B)
+    if tile is not None:                                                # stage 1 returns x, not theta (:538-541)
+        return _tiled_outputs(tile, pb, None, x, sse, X_orig, denoiser, sched, noise_estimate, logf, None, None)
     psnr_all = []
     if want_iqa:
         psnr_all = list(iqa.psnr_from_sse(sse.cpu().numpy()[:n_total], pb.npix * pb.B))
@@ -228,7 +248,9 @@ def _tiled_demosaic_denoise(tile, adapter, halo, x, b, inv_rou, w, tau, x_rgb, u
 
 def _tiled_outputs(tile, pb, xhat, theta, sse, X_orig, denoiser, sched, noise_estimate, logf, model_denoise, model_demosaic):
     """Gather the strips into full-frame results on every rank (``tile.gather_root_only``: on rank 0 only, the others return
-    None for the two image arrays and an empty SSIM list); PSNR from all-reduced squared errors."""
+    None for the image arrays and an empty SSIM list); PSNR from all-reduced squared errors.  ``theta`` is the Bayer cube
+    returned (stage 1 passes x).  Without ``xhat`` (the TV prior) the result is the reference's 4-tuple
+    ``(x_bayer_np, psnr_, ssim_, psnr_all)``."""
     B = pb.B
     Ht, W = tile.H_total, tile.W
     psnr_all = []
@@ -243,12 +265,14 @@ def _tiled_outputs(tile, pb, xhat, theta, sse, X_orig, denoiser, sched, noise_es
         import time
         torch.cuda.synchronize(); t0 = time.time()
     theta_full = tile.gather_rows(theta, root)                              # [B, Ht, W]
-    xhat_full = tile.gather_rows(xhat, root)                                # [B, 3, Ht, W]
+    xhat_full = tile.gather_rows(xhat, root) if xhat is not None else None  # [B, 3, Ht, W]
     if timing:
         torch.cuda.synchronize(); t1 = time.time()
     have = theta_full is not None
     x_bayer_np = cuda2np(ops.planar_to_pixlast(theta_full.contiguous(), 1, B).view(Ht, W, B)) if have else None
-    xbgr3_np = cuda2np(ops.planar_to_pixlast(xhat_full.contiguous(), 3, B).view(Ht, W, 3, B)) if have else None
+    xbgr3_np = None
+    if have and xhat is not None:
+        xbgr3_np = cuda2np(ops.planar_to_pixlast(xhat_full.contiguous(), 3, B).view(Ht, W, 3, B))
     if timing:
         torch.cuda.synchronize(); t2 = time.time()
         print("tiled outputs: gather %.1f ms, remap + device-to-host %.1f ms" % (1e3 * (t1 - t0), 1e3 * (t2 - t1)), file=sys.stderr)
@@ -262,6 +286,8 @@ def _tiled_outputs(tile, pb, xhat, theta, sse, X_orig, denoiser, sched, noise_es
         if orig_g is not None:
             orig_full = cuda2np(ops.planar_to_pixlast(orig_g.contiguous(), 1, B).view(Ht, W, B))
             ssim_ = [iqa.ssim(orig_full[:, :, t], x_bayer_np[:, :, t], data_range=1.) for t in range(B)]
+    if xhat is None:
+        return x_bayer_np, psnr_, ssim_, psnr_all
     return xbgr3_np, x_bayer_np, psnr_, ssim_, psnr_all, model_denoise, model_demosaic
 
 
@@ -284,8 +310,9 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
     numpy arrays (no D2H copy, no host sync) — used by bench.py for the HBM-resident measurement.
     ``tile`` (extension, ``parallel.TileContext``): spatial row-strip tiling of one large frame over the ranks (BASELINE
     config 5).  Every rank passes ITS rows of y / Phi / x0 / X_orig; the mosaic (2 rows) and the denoiser input (80 rows
-    for FastDVDnet, 28 for FFDNet) are halo-exchanged with the neighbouring ranks once per iteration, PSNR sums and the
-    fine-tune gradients are all-reduced, and the returned arrays are the full frame (gathered on every rank).
+    for FastDVDnet, 28 for FFDNet; 8 rows of the TV input and an all-gather of its early-stop energies for 'tv') are
+    halo-exchanged with the neighbouring ranks once per iteration, PSNR sums and the fine-tune gradients are all-reduced,
+    and the returned arrays are the full frame (gathered on every rank).
     """
     name = denoiser if denoiser == 'tv' else str(denoiser).lower()
     if name not in ('tv', 'ffdnet_color', 'fastdvd_color'):
@@ -295,14 +322,14 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
     dev = pb.y.device
     H, W, B = pb.H, pb.W, pb.B
     if tile is not None:
-        if name == 'tv':
-            raise NotImplementedError("tiled mode covers the deep denoisers (the TV prior would need a halo exchange per "
-                                      "inner iteration; stage 1 shards over measurement groups instead)")
         if H != tile.rows or W != tile.W:
             raise ValueError("tiled mode: pass this rank's rows (%d x %d), got %d x %d" % (tile.rows, tile.W, H, W))
-        if grad_sync is None:
-            grad_sync = tile.all_reduce_sum          # loss is normalised by the whole frame -> gradients ADD over strips
-        tile.enable_p2p(3 * B, 28 if name == 'ffdnet_color' else 80)      # boundary rows go peer to peer over NVLink
+        if name == 'tv':
+            tile.enable_p2p(B, ops.TV_HALO)                                # 8 rows of the TV input, peer to peer
+        else:
+            if grad_sync is None:
+                grad_sync = tile.all_reduce_sum      # loss is normalised by the whole frame -> gradients ADD over strips
+            tile.enable_p2p(3 * B, 28 if name == 'ffdnet_color' else 80)  # boundary rows go peer to peer over NVLink
     alpha = 0.01 if name == 'tv' else 1                                  # :101-104
     rou = 0.55 if name == 'fastdvd_color' else 1                         # :106-109
     tau = 100                                                            # :110
@@ -315,7 +342,8 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
     theta, b, x = pb.theta, pb.b, pb.x
     xhat = None
     if name == 'tv':
-        ws = ops.TvWorkspace(H, W, B, dev)
+        ws = ops.TvWorkspace(H, W, B, dev) if tile is None else ops.TvStripWorkspace(H, W, B, dev)
+        tv = ops.tv_chambolle if tile is None else tile.tv_chambolle
         b_next = torch.empty_like(b)
     else:
         from . import ddnet_adapter, fastdvdnet_adapter, ffdnet_adapter
@@ -341,7 +369,7 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
             ops.project_stage2(theta, b, pb.phi, pb.y, pb.phisum, x, alpha, rou)
             if name == 'tv':
                 # theta = clip(TV(x + b/rho)); b = b + (x - theta)                                   (:153-160, :265-267)
-                ops.tv_chambolle(x, b, inv_rou, theta, b_next, 1.0, True, ws, weight=0.1, n_iter_max=5)
+                tv(x, b, inv_rou, theta, b_next, 1.0, True, ws, weight=0.1, n_iter_max=5)
                 b, b_next = b_next, b
                 if want_iqa:
                     ops.psnr_accum(theta.view(1, -1), pb.orig.view(1, -1), sse[k:k + 1])

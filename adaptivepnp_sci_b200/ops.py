@@ -82,6 +82,65 @@ def tv_chambolle(x, b, c_b, theta_out, b_out, s_b, clip, ws, weight=0.1, eps=2.0
     return theta_out
 
 
+TV_HALO = 8          # rows of f = x + c_b*b a TV row strip needs from each neighbour
+
+
+class TvStripWorkspace:
+    """Scratch for sci_tv_strip_main / _finish (per-block energy partials + stop indices) and this strip's energy sums
+    ``esum`` [4B, 8] float64, the tensor the ranks gather between the two halves."""
+
+    def __init__(self, rows, W, B, device):
+        self.nbytes = int(_lib.lib.sci_tv_strip_workspace_bytes(rows, W, B))
+        self.buf = torch.empty(self.nbytes, dtype=torch.uint8, device=device)
+        self.esum = torch.empty((4 * B, 8), dtype=torch.float64, device=device)
+        self.shape = (rows, W, B)
+
+
+def _vp(p):
+    """Raw device address (int) or None -> ctypes pointer."""
+    return ctypes.c_void_p(p) if p else None
+
+
+def tv_strip_main(x, b, c_b, theta_out, b_out, s_b, clip, ws, row0, H_total, halo_top=None, halo_bot=None, weight=0.1,
+                  eps=2.0e-4, n_iter_max=5, flag_top=None, flag_bot=None, seq=0, err=None):
+    """Main pass of the TV prior on the row strip x [B, rows, W] (global rows row0 ..) + its energy sums (-> ``ws.esum``).
+    halo_top / halo_bot: [B, 8, W] tensors of f, or raw device addresses (peer-to-peer slots, with their flag words)."""
+    require_cuda_f32(x, b, theta_out, b_out)
+    B, rows, W = x.shape
+    assert ws.shape == (rows, W, B)
+    ht = ptr(halo_top) if torch.is_tensor(halo_top) else _vp(halo_top)
+    hb = ptr(halo_bot) if torch.is_tensor(halo_bot) else _vp(halo_bot)
+    call("sci_tv_strip_main", ptr(x), ptr(b), float(c_b), ptr(theta_out), ptr(b_out), float(s_b), int(bool(clip)),
+         rows, W, B, int(row0), int(H_total), ht, hb, _vp(flag_top), _vp(flag_bot), int(seq), _vp(err), float(weight),
+         float(eps), int(n_iter_max), ptr(ws.buf), ctypes.c_size_t(ws.nbytes), ptr(ws.esum), stream())
+    return ws.esum
+
+
+def tv_strip_finish(x, b, c_b, theta_out, b_out, s_b, clip, ws, row0, H_total, esum_all, halo_top=None, halo_bot=None,
+                    weight=0.1, eps=2.0e-4, n_iter_max=5, nstop_out=None):
+    """Stop decision from esum_all [world, 4B, 8] (summed in strip order) + the fix-up pass of the channels that stop early."""
+    require_cuda_f32(x, b, theta_out, b_out)
+    B, rows, W = x.shape
+    assert ws.shape == (rows, W, B)
+    assert esum_all.is_cuda and esum_all.dtype == torch.float64 and esum_all.is_contiguous() and esum_all.shape[-2:] == (4 * B, 8)
+    ht = ptr(halo_top) if torch.is_tensor(halo_top) else _vp(halo_top)
+    hb = ptr(halo_bot) if torch.is_tensor(halo_bot) else _vp(halo_bot)
+    world = esum_all.numel() // (4 * B * 8)
+    call("sci_tv_strip_finish", ptr(x), ptr(b), float(c_b), ptr(theta_out), ptr(b_out), float(s_b), int(bool(clip)),
+         rows, W, B, int(row0), int(H_total), ht, hb, float(weight), float(eps), int(n_iter_max), ptr(ws.buf),
+         ctypes.c_size_t(ws.nbytes), ptr(esum_all), world, ptr(nstop_out), stream())
+    return theta_out
+
+
+def halo_send_tv(x, b, c_b, up_dst, down_dst, up_flag, down_flag, seq, done, halo=TV_HALO):
+    """f = x + c_b*b of the first / last ``halo`` rows of x [B, rows, W] -> the neighbours' slots (raw peer addresses or
+    None), then release ``seq`` into their flag words (``done``: the kernel's completion counter, raw address)."""
+    require_cuda_f32(x, b)
+    B, rows, W = x.shape
+    call("sci_halo_send_tv", ptr(x), ptr(b), float(c_b), B, rows, W, int(halo), _vp(up_dst), _vp(down_dst), _vp(up_flag),
+         _vp(down_flag), int(seq), _vp(done), stream())
+
+
 def malvar2004(x, b, c_b, w, inv_tau, x_rgb_out, u_out):
     """K6.  mosaic = x + c_b*b (b may be None) -> x_rgb [B,3,H,W]; u = x_rgb - inv_tau*w (if w given)."""
     require_cuda_f32(x, b, w, x_rgb_out, u_out)

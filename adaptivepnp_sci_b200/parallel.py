@@ -129,6 +129,24 @@ class P2PRegion:
              vp(self.scratch.data_ptr() + 4), stream())
         return ext
 
+    def send_tv(self, x, b, c_b, top, bot):
+        """The TV prior's halo: f = x + c_b*b of this strip's first / last 8 rows goes straight into the neighbours' slots
+        (``sci_halo_send_tv``).  Returns what ``sci_tv_strip_main`` needs to read this rank's own slots in place: (halo_top,
+        halo_bot, flag_top, flag_bot, seq, err) as raw addresses (None where there is no neighbour).  The slots of this
+        exchange are read again by the fix-up pass (``sci_tv_strip_finish``); the next exchange is issued after it in stream
+        order, which keeps the parity argument of the class docstring."""
+        from . import ops
+        B, rows, W = x.shape
+        if B * ops.TV_HALO * W * 4 > self.slot:
+            raise ValueError("TV halo of %d bytes exceeds the P2P slot (%d)" % (B * ops.TV_HALO * W * 4, self.slot))
+        self.seq += 1
+        par, r = self.seq & 1, self.ctx.rank
+        up, down = self.peer.get(r - 1) if top else None, self.peer.get(r + 1) if bot else None
+        ops.halo_send_tv(x, b, c_b, self.slot_ptr(up, par, 1) if up else None, self.slot_ptr(down, par, 0) if down else None,
+                         up + 4 if up else None, down if down else None, self.seq, self.scratch.data_ptr())
+        return (self.slot_ptr(self.base, par, 0) if top else None, self.slot_ptr(self.base, par, 1) if bot else None,
+                self.base if top else None, self.base + 4 if bot else None, self.seq, self.scratch.data_ptr() + 4)
+
     def check(self):
         """Host-side check of the bounded wait (call at a synchronisation point)."""
         e = int(self.scratch[1])
@@ -164,11 +182,15 @@ class TileContext:
       FFDNet-colour: -24..+25 -> 28), exchanged once per ADMM iteration; the strip is then denoised with its halo and
       cropped ("overlap-tile"), so zero padding is only ever applied at true image borders.
 
+    * TV prior (``tv_chambolle``): 8 rows of f = x + c_b*b, exchanged once per call (the kernel runs all inner iterations
+      on chip, and a pixel depends only on rows within +-8).
+
     ``exchange`` moves the halo rows peer to peer: after ``enable_p2p`` the boundary rows are stored straight into the
     neighbour's memory over NVLink by ``sci_halo_send`` / ``sci_halo_assemble`` (``P2PRegion``); without it (CPU tests,
-    ``SCI_TILE_P2P=0``) with point-to-point sends of torch.distributed.  No collective is on the per-iteration path; the only reductions are the scalar
-    PSNR sums, the fine-tune loss/gradient all-reduce (SUM: the loss is normalised by the pixel count of the whole frame)
-    and the final gather of the result strips."""
+    ``SCI_TILE_P2P=0``) with point-to-point sends of torch.distributed.  The only collective on the per-iteration path is
+    the TV prior's all-gather of its early-stop energies (``world`` x 4B x 8 doubles per call, in-stream on NCCL); the
+    other reductions are the scalar PSNR sums, the fine-tune loss/gradient all-reduce (SUM: the loss is normalised by the
+    pixel count of the whole frame) and the final gather of the result strips."""
 
     def __init__(self, ctx, H_total, W):
         if H_total % (4 * ctx.world) != 0:
@@ -211,7 +233,6 @@ class TileContext:
 
     def exchange(self, own, halo):
         """own [B,C,rows,W] (contiguous, this rank's rows) -> (ext [B,C,top+rows+bot,W], top)."""
-        import torch.distributed as dist
         top, bot = self.halo_sizes(halo)
         B, C, rows, W = own.shape
         self.halo_bytes_moved += (top + bot) * B * C * W * own.element_size()
@@ -221,28 +242,70 @@ class TileContext:
         ext[:, :, top:top + rows].copy_(own)
         if self.world == 1:
             return ext, 0
+        rcv_top, rcv_bot = self._sendrecv_rows(own, top, bot)
+        if rcv_top is not None:
+            ext[:, :, :top].copy_(rcv_top)
+        if rcv_bot is not None:
+            ext[:, :, top + rows:].copy_(rcv_bot)
+        return ext, top
+
+    def _sendrecv_rows(self, own, top, bot):
+        """Point-to-point sends of torch.distributed: my first ``top`` rows up and last ``bot`` rows down; returns the rows
+        received from the upper / lower neighbour (None where there is none)."""
+        import torch.distributed as dist
+        rows = own.shape[-2]
         host = self.ctx.backend != "nccl"          # gloo moves CUDA halos through host memory (tests / CPU runs)
-        ops, bufs = [], []
+        ops, bufs = [], {}
         if top:      # upper neighbour: send my first rows, receive its last rows
-            snd = own[:, :, :top].contiguous()
+            snd = own[..., :top, :].contiguous()
             snd = snd.cpu() if host else snd
             rcv = torch.empty_like(snd)
             ops += [dist.P2POp(dist.isend, snd, self.rank - 1), dist.P2POp(dist.irecv, rcv, self.rank - 1)]
-            bufs.append(("top", rcv, snd))
+            bufs["top"] = (rcv, snd)
         if bot:
-            snd = own[:, :, rows - bot:].contiguous()
+            snd = own[..., rows - bot:, :].contiguous()
             snd = snd.cpu() if host else snd
             rcv = torch.empty_like(snd)
             ops += [dist.P2POp(dist.isend, snd, self.rank + 1), dist.P2POp(dist.irecv, rcv, self.rank + 1)]
-            bufs.append(("bot", rcv, snd))
+            bufs["bot"] = (rcv, snd)
         for w in dist.batch_isend_irecv(ops):
             w.wait()
-        for where, rcv, _ in bufs:
-            if where == "top":
-                ext[:, :, :top].copy_(rcv)
+        got = {k: v[0].to(own.device) for k, v in bufs.items()}
+        return got.get("top"), got.get("bot")
+
+    def tv_chambolle(self, x, b, c_b, theta, b_out, s_b, clip, ws, weight=0.1, eps=2.0e-4, n_iter_max=5, nstop_out=None):
+        """``ops.tv_chambolle`` on this rank's strip x [B, rows, W] (``ws``: ``ops.TvStripWorkspace``).  Halo of 8 rows of
+        f = x + c_b*b from each neighbour (peer to peer after ``enable_p2p``, else torch.distributed), main pass, all-gather
+        of the early-stop energies, decision + fix-up pass.  Every rank sums the gathered energies in rank order, so all
+        make the same stop decisions; own pixels are those of the un-tiled kernel bit for bit given the same decisions."""
+        from . import ops
+        B, rows, W = x.shape
+        top, bot = self.halo_sizes(ops.TV_HALO)
+        kw = dict(weight=weight, eps=eps, n_iter_max=n_iter_max)
+        halo_top = halo_bot = None
+        wait = {}
+        if self.world > 1:
+            self.halo_bytes_moved += (top + bot) * B * W * 4
+            if self.p2p is not None and x.is_cuda:
+                halo_top, halo_bot, ft, fb, seq, err = self.p2p.send_tv(x, b, c_b, top, bot)
+                wait = dict(flag_top=ft, flag_bot=fb, seq=seq, err=err)
             else:
-                ext[:, :, top + rows:].copy_(rcv)
-        return ext, top
+                f = x if b is None else ops.axpy(x, c_b, b)
+                halo_top, halo_bot = self._sendrecv_rows(f, top, bot)
+        esum = ops.tv_strip_main(x, b, c_b, theta, b_out, s_b, clip, ws, self.r0, self.H_total, halo_top, halo_bot,
+                                 **kw, **wait)
+        esum_all = esum.view(1, *esum.shape)
+        if self.world > 1:
+            import torch.distributed as dist
+            if self.ctx.backend == "nccl":
+                esum_all = torch.empty((self.world,) + tuple(esum.shape), dtype=esum.dtype, device=esum.device)
+                dist.all_gather_into_tensor(esum_all, esum)
+            else:                                   # gloo: through host memory, like gather_rows
+                parts = [torch.empty(esum.shape, dtype=esum.dtype) for _ in range(self.world)]
+                dist.all_gather(parts, esum.cpu())
+                esum_all = torch.stack(parts).to(esum.device)
+        return ops.tv_strip_finish(x, b, c_b, theta, b_out, s_b, clip, ws, self.r0, self.H_total, esum_all, halo_top,
+                                   halo_bot, nstop_out=nstop_out, **kw)
 
     def all_reduce_sum(self, t):
         if self.world > 1:

@@ -108,6 +108,33 @@ int sci_tv_chambolle2d(const float* x, const float* b, float c_b, float* theta, 
                        float s_b, int clip, int H, int W, int B, float weight, float eps,
                        int n_iter_max, void* workspace, size_t workspace_bytes, int* nstop_out,
                        void* stream);
+/* K4 on a row strip of one frame (one strip per GPU).  The strip holds rows [row0, row0 + rows) of an
+ * H_total-row image (row0, rows even, rows >= 8); x, b, theta, b_out are [B][rows][W].  A pixel's
+ * result depends only on rows within +-8, so the caller provides, once per call, 8 rows of
+ * f = x + c_b*b from each neighbour: halo_top / halo_bot [B][8][W], NULL exactly when the strip
+ * touches that image border (see sci_halo_send_tv).  Every own pixel is then computed from the same
+ * inputs in the same order as by sci_tv_chambolle2d.  The early stop is global, so the decision is
+ * split in two:
+ *   sci_tv_strip_main:   main pass + this strip's energy sums, esum_out double[4B][8];
+ *   (caller: gather the esums of all strips in strip order, esum_all double[world][4B][8])
+ *   sci_tv_strip_finish: sums esum_all in strip order, applies the stopping rule, writes nstop_out
+ *                        (optional) and rewrites the channels that stopped early.
+ * With one strip the result, nstop included, equals sci_tv_chambolle2d bit for bit.  With several,
+ * the energies are summed in a different order, so a stop decision can differ from the un-tiled one
+ * only when |E_prev - E_k| - eps*E_init is within fp64 rounding of zero.
+ * flag_top / flag_bot (optional): local flag words of the peer-to-peer exchange; tiles that read a halo
+ * first wait (bounded, ~10 s, then *err != 0) until the flag has reached seq.  n_iter_max in 2..5.
+ * The workspace (sci_tv_strip_workspace_bytes) must be the same for main and finish. */
+size_t sci_tv_strip_workspace_bytes(int rows, int W, int B);
+int sci_tv_strip_main(const float* x, const float* b, float c_b, float* theta, float* b_out, float s_b, int clip,
+                      int rows, int W, int B, int row0, int H_total, const float* halo_top, const float* halo_bot,
+                      const unsigned* flag_top, const unsigned* flag_bot, unsigned seq, unsigned* err, float weight,
+                      float eps, int n_iter_max, void* workspace, size_t workspace_bytes, double* esum_out,
+                      void* stream);
+int sci_tv_strip_finish(const float* x, const float* b, float c_b, float* theta, float* b_out, float s_b, int clip,
+                        int rows, int W, int B, int row0, int H_total, const float* halo_top, const float* halo_bot,
+                        float weight, float eps, int n_iter_max, void* workspace, size_t workspace_bytes,
+                        const double* esum_all, int world, int* nstop_out, void* stream);
 
 /* ---- K6: Malvar-2004 demosaic + (-w/tau) ----------------------------------
  * packages/colour_demosaicing/bayer/demosaicing/malvar2004.py:169-246 applied to
@@ -435,7 +462,10 @@ int sci_adam_step(float* param, const float* grad, float* exp_avg, float* exp_av
  * NULL = no neighbour on that side), then release-stores `seq` into up_flag / down_flag (peer flag words).
  * sci_halo_assemble (same stream): waits until *flag_top / *flag_bot (LOCAL flag words written by the neighbours) have
  * reached `seq`, then writes ext [planes][top + rows + bot][W] = [recv_top | own | recv_bot].  *err becomes non-zero if a
- * neighbour did not deliver within ~10 s (the wait is bounded: a lost peer must not hang the GPU). */
+ * neighbour did not deliver within ~10 s (the wait is bounded: a lost peer must not hang the GPU).
+ * sci_halo_send_tv: the TV prior's halo (sci_tv_strip_main).  Like sci_halo_send, but stores f = x + c_b*b of the
+ * first / last `halo` rows of x, b [planes][rows][W] (b may be NULL: f = x; W even), rounded exactly as the TV kernel
+ * forms it; the receiver reads its slots in place. */
 int sci_p2p_alloc(size_t bytes, void** ptr);
 int sci_p2p_free(void* ptr);
 int sci_p2p_get_handle(void* ptr, void* handle64);
@@ -443,6 +473,9 @@ int sci_p2p_open_handle(const void* handle64, void** ptr);
 int sci_p2p_close_handle(void* ptr);
 int sci_halo_send(const float* own, int planes, int rows, int W, int halo, float* up_dst, float* down_dst,
                   unsigned* up_flag, unsigned* down_flag, unsigned seq, unsigned* done_counter, void* stream);
+int sci_halo_send_tv(const float* x, const float* b, float c_b, int planes, int rows, int W, int halo, float* up_dst,
+                     float* down_dst, unsigned* up_flag, unsigned* down_flag, unsigned seq, unsigned* done_counter,
+                     void* stream);
 int sci_halo_assemble(const float* own, int planes, int rows, int W, int top, int bot, const float* recv_top,
                       const float* recv_bot, const unsigned* flag_top, const unsigned* flag_bot, unsigned seq,
                       float* ext, unsigned* err, void* stream);
