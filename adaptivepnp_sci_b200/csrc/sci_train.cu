@@ -330,25 +330,14 @@ __global__ void fastdvd_pack_grad_kernel(const float* __restrict__ din, float* _
 }
 
 __global__ void fastdvd_output_kernel(const float* __restrict__ frames, const float* __restrict__ y, float* __restrict__ out,
-                                      int B, int H, int W, int Cpad, int to_grad) {
+                                      int B, int H, int W, int Cpad) {
     const long plane = (long)H * W;
-    if (!to_grad) {
-        const long total = (long)B * 3 * plane;
-        const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
-        if (idx >= total) return;
-        const long p = idx % plane;
-        const int c = (int)((idx / plane) % 3), f = (int)(idx / (3 * plane));
-        out[idx] = frames[idx] - __ldg(y + ((long)f * plane + p) * Cpad + c);    // models.py:196
-    } else {
-        // dy[f][p][c] = -dout[f][c][p] for c < 3, 0 for the padded columns   (frames = dout here)
-        const long total = (long)B * plane * Cpad;
-        const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
-        if (idx >= total) return;
-        const int k = (int)(idx % Cpad);
-        const long p = (idx / Cpad) % plane;
-        const int f = (int)(idx / (Cpad * plane));
-        out[idx] = (k < 3) ? -frames[((long)f * 3 + k) * plane + p] : 0.f;
-    }
+    const long total = (long)B * 3 * plane;
+    const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= total) return;
+    const long p = idx % plane;
+    const int c = (int)((idx / plane) % 3), f = (int)(idx / (3 * plane));
+    out[idx] = frames[idx] - __ldg(y + ((long)f * plane + p) * Cpad + c);    // models.py:196
 }
 
 // dy[f][p][c] = -dout[f][c][p] for c < 3, 0 for the padded columns.  One thread reads the three plane values of its pixel
@@ -780,8 +769,9 @@ extern "C" int sci_fastdvd_pack_input(const float* frames, float sigma, float* o
     SCI_REQUIRE(frames && out && B > 0 && H > 0 && W > 0 && Cpad >= (round_tf32 ? 32 : 12), "fastdvd_pack_input");
     SCI_REQUIRE(Cpad <= 48 && B <= 65535, "fastdvd_pack_input: Cpad <= 48");
     const size_t smem = (size_t)FPACK_PIX * (Cpad + 1) * sizeof(float);
-    if (smem > 48 * 1024)
-        cudaFuncSetAttribute(fastdvd_pack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    // the largest Cpad admitted above, so that the once-per-device limit covers every later call
+    const cudaError_t e = sci_smem_limit((const void*)fastdvd_pack_kernel, FPACK_PIX * (48 + 1) * (int)sizeof(float));
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "fastdvd_pack_input: shared-memory limit", e);
     fastdvd_pack_kernel<<<dim3(grid1d((long)H * W, FPACK_PIX), B), FPACK_PIX, smem, sci_stream(stream)>>>(frames, sigma, out, B,
                                                                                                       H, W, Cpad, round_tf32);
     SCI_CHECK_LAUNCH("fastdvd_pack_input");
@@ -800,7 +790,7 @@ extern "C" int sci_fastdvd_pack_input_grad(const float* din, float* dframes, int
 extern "C" int sci_fastdvd_output(const float* frames, const float* y, float* out, int B, int H, int W, int Cpad,
                                   void* stream) {
     SCI_REQUIRE(frames && y && out && B > 0 && H > 0 && W > 0 && Cpad >= 3, "fastdvd_output");
-    fastdvd_output_kernel<<<grid1d((long)B * 3 * H * W), 256, 0, sci_stream(stream)>>>(frames, y, out, B, H, W, Cpad, 0);
+    fastdvd_output_kernel<<<grid1d((long)B * 3 * H * W), 256, 0, sci_stream(stream)>>>(frames, y, out, B, H, W, Cpad);
     SCI_CHECK_LAUNCH("fastdvd_output");
     return SCI_OK;
 }
@@ -808,6 +798,9 @@ extern "C" int sci_fastdvd_output(const float* frames, const float* y, float* ou
 extern "C" int sci_fastdvd_output_grad(const float* dout, float* dy, int B, int H, int W, int Cpad, void* stream) {
     SCI_REQUIRE(dout && dy && B > 0 && H > 0 && W > 0 && Cpad >= 3, "fastdvd_output_grad");
     SCI_REQUIRE(Cpad <= 64, "fastdvd_output_grad: Cpad");
+    // 256 * (Cpad + 1) floats pass the 48 KB default from Cpad 48 on; raise the limit to what Cpad 64 needs
+    const cudaError_t e = sci_smem_limit((const void*)fastdvd_output_grad_kernel, FPACK_PIX * (64 + 1) * (int)sizeof(float));
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "fastdvd_output_grad: shared-memory limit", e);
     const long plane = (long)H * W;
     fastdvd_output_grad_kernel<<<dim3(grid1d(plane, FPACK_PIX), B), FPACK_PIX, (size_t)FPACK_PIX * (Cpad + 1) * sizeof(float),
                                  sci_stream(stream)>>>(dout, dy, H, W, Cpad);
