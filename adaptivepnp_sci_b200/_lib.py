@@ -96,6 +96,10 @@ PROTOTYPES = {
     "sci_ddnet_stage2_input": [_p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _i, _p],
     "sci_ddnet_upsample4": [_p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _p],
     "sci_ddnet_output": [_p, _p, _p, _i, _p, _p, _i, _i, _i, _p],
+    "sci_ddnet_pack_input1_frames": [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
+    "sci_ddnet_pack_input4_frames": [_p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
+    "sci_ddnet_stage2_input_frames": [_p, _p, _p, _i, _p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
+    "sci_ddnet_upsample4_strip": [_p, _p, _p, _i, _p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p],
     "sci_ddnet_loss_fwd_bwd": [_p, _p, _p, _p, _i, _i, _i, _p],
     "sci_ddnet_output_bwd": [_p, _p, _p, _p, _i, _p, _p, _p, _p, _p, _i, _i, _i, _p],
     "sci_ddnet_stage2_input_bwd": [_p, _p, _p, _p, _p, _i, _i, _i, _p],

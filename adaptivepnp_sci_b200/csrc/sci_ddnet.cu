@@ -10,6 +10,11 @@
 //
 // Batch order of the stacked triples: n = j*B + f  (j = 0,1,2 the triple, f the centre frame); triple j, slot k reads
 // frame (f - 2 + j + k) mod B and the scalar a[3j+k]  (network_demosaicking.py:442-448).
+//
+// The forward kernels evaluate a range of centre frames [f0, f0+Bc) of the B-frame sequence (frame chunks that bound the
+// memory of a pass): batch n = j*Bc + (f-f0), while the frame reads stay (f-2+j+k) mod B over the whole sequence.  The
+// up-sampler also takes the global row of its local row 0 and the global frame height, so that it runs on a row strip of a
+// larger frame (parallel.TileContext) with the source rows of the whole frame.  f0 = 0, Bc = B, row 0 = 0 is the whole.
 #include "sci_common.cuh"
 
 namespace {
@@ -43,11 +48,12 @@ __device__ __forceinline__ void flush_rows(const float* srow, float* dst, int np
     for (int i = threadIdx.x; i < npx * DD_CP; i += DD_PIX) dst[i] = srow[(i / DD_CP) * DD_CS + (i % DD_CP)];
 }
 
-// path 1 input: out[j*B+f][p][k] = mosaic[(f-2+j+k) mod B][p] * a[3j+k],  k = 0..2
+// path 1 input: out[j*Bc+f-f0][p][k] = mosaic[(f-2+j+k) mod B][p] * a[3j+k],  k = 0..2
 __global__ void __launch_bounds__(DD_PIX) dd_pack1_kernel(const float* __restrict__ mosaic, const float* __restrict__ a,
-                                                           float* __restrict__ out, int B, long plane, int split) {
+                                                           float* __restrict__ out, int B, int f0, int Bc, long plane,
+                                                           int split) {
     __shared__ float srow[DD_PIX * DD_CS];
-    const int n = blockIdx.y, j = n / B, f = n % B;
+    const int n = blockIdx.y, j = n / Bc, f = f0 + n % Bc;
     const long p0 = (long)blockIdx.x * DD_PIX, p = p0 + threadIdx.x;
     float* row = srow + threadIdx.x * DD_CS;
     for (int k = 0; k < DD_CP; ++k) row[k] = 0.f;
@@ -58,11 +64,12 @@ __global__ void __launch_bounds__(DD_PIX) dd_pack1_kernel(const float* __restric
     flush_rows(srow, out + ((long)n * plane + p0) * DD_CP, (int)min((long)DD_PIX, plane - p0));
 }
 
-// path 2 input (half resolution): out[j*B+f][y][x][4k+ib] = mosaic[fr][2y+ib/2][2x+ib%2] * a2[(3j+k)*4+ib]
+// path 2 input (half resolution): out[j*Bc+f-f0][y][x][4k+ib] = mosaic[fr][2y+ib/2][2x+ib%2] * a2[(3j+k)*4+ib]
 __global__ void __launch_bounds__(DD_PIX) dd_pack4_kernel(const float* __restrict__ mosaic, const float* __restrict__ a2,
-                                                           float* __restrict__ out, int B, int H, int W, int split) {
+                                                           float* __restrict__ out, int B, int f0, int Bc, int H, int W,
+                                                           int split) {
     __shared__ float srow[DD_PIX * DD_CS];
-    const int n = blockIdx.y, j = n / B, f = n % B;
+    const int n = blockIdx.y, j = n / Bc, f = f0 + n % Bc;
     const int h2 = H >> 1, w2 = W >> 1;
     const long plane = (long)H * W, hplane = (long)h2 * w2;
     const long p0 = (long)blockIdx.x * DD_PIX, p = p0 + threadIdx.x;
@@ -85,14 +92,15 @@ __global__ void __launch_bounds__(DD_PIX) dd_pack4_kernel(const float* __restric
     flush_rows(srow, out + ((long)n * hplane + p0) * DD_CP, (int)min((long)DD_PIX, hplane - p0));
 }
 
-// temp2 input of one path.  For centre frame f:  v[j][c] = (mosaic ? mosaic[(f-1+j) mod B][p]*a[3j+1] : 0) + xo[j*B+f][p][c]
-// (residual `in1 + x`, network_demosaicking.py:242, the 1-channel in1 broadcasting over 3 channels);
-// t2in[f][p][3j+c] = v[j][c];  res[f][c][p] = v[1][c]  (the `in1` of the temp2 call, kept in full fp32).
+// temp2 input of one path.  For centre frame f = f0+i:  v[j][c] = (mosaic ? mosaic[(f-1+j) mod B][p]*a[3j+1] : 0)
+// + xo[j*Bc+i][p][c] (residual `in1 + x`, network_demosaicking.py:242, the 1-channel in1 broadcasting over 3 channels);
+// t2in[i][p][3j+c] = v[j][c];  res[i][c][p] = v[1][c]  (the `in1` of the temp2 call, kept in full fp32).
 __global__ void __launch_bounds__(DD_PIX) dd_mid_kernel(const float* __restrict__ mosaic, const float* __restrict__ a,
                                                          const float* __restrict__ xo, int Cp, float* __restrict__ t2in,
-                                                         float* __restrict__ res, int B, long plane, int split) {
+                                                         float* __restrict__ res, int B, int f0, int Bc, long plane,
+                                                         int split) {
     __shared__ float srow[DD_PIX * DD_CS];
-    const int f = blockIdx.y;
+    const int i = blockIdx.y, f = f0 + i;
     const long p0 = (long)blockIdx.x * DD_PIX, p = p0 + threadIdx.x;
     float* row = srow + threadIdx.x * DD_CS;
     for (int k = 0; k < DD_CP; ++k) row[k] = 0.f;
@@ -100,26 +108,30 @@ __global__ void __launch_bounds__(DD_PIX) dd_mid_kernel(const float* __restrict_
 #pragma unroll
         for (int j = 0; j < 3; ++j) {
             const float in1 = mosaic ? mosaic[(long)wrap(f - 1 + j, B) * plane + p] * a[3 * j + 1] : 0.f;
-            const float* y = xo + ((long)(j * B + f) * plane + p) * Cp;
+            const float* y = xo + ((long)(j * Bc + i) * plane + p) * Cp;
 #pragma unroll
             for (int c = 0; c < 3; ++c) {
                 const float v = mosaic ? in1 + y[c] : y[c];
                 put(row, 3 * j + c, v, split);
-                if (j == 1) res[((long)f * 3 + c) * plane + p] = v;
+                if (j == 1) res[((long)i * 3 + c) * plane + p] = v;
             }
         }
     }
-    flush_rows(srow, t2in + ((long)f * plane + p0) * DD_CP, (int)min((long)DD_PIX, plane - p0));
+    flush_rows(srow, t2in + ((long)i * plane + p0) * DD_CP, (int)min((long)DD_PIX, plane - p0));
 }
 
 // path 2 after the U-shaped body: y4[n][ib] = in1 + xo4 at half resolution (in1 = centre slot of the packed input),
 // then nn.UpsamplingBilinear2d(scale_factor=2) (align_corners=True), written as the 4-channel input of the fusion convs.
+// The H rows held start at global row row0 (even) of a frame of Ht rows: the source coordinate is formed from the global
+// row; source rows outside the held ones (only for output rows within one row of the strip's edges, whose values the
+// caller discards with its halo) are clamped to the held rows.
 __global__ void __launch_bounds__(DD_PIX) dd_up4_kernel(const float* __restrict__ mosaic, const float* __restrict__ a2,
                                                          const float* __restrict__ xo4, int Cp, float* __restrict__ out,
-                                                         int B, int H, int W, float sy, float sx, int split) {
+                                                         int B, int f0, int Bc, int H, int W, int row0, int Ht, float sy,
+                                                         float sx, int split) {
     __shared__ float srow[DD_PIX * DD_CS];
-    const int n = blockIdx.y, j = n / B, f = n % B;
-    const int h2 = H >> 1, w2 = W >> 1;
+    const int n = blockIdx.y, j = n / Bc, f = f0 + n % Bc;
+    const int h2 = H >> 1, w2 = W >> 1, ht2 = Ht >> 1, hr0 = row0 >> 1;
     const long plane = (long)H * W, hplane = (long)h2 * w2;
     const long p0 = (long)blockIdx.x * DD_PIX, p = p0 + threadIdx.x;
     float* row = srow + threadIdx.x * DD_CS;
@@ -127,11 +139,12 @@ __global__ void __launch_bounds__(DD_PIX) dd_up4_kernel(const float* __restrict_
     if (p < plane) {
         const int Y = (int)(p / W), X = (int)(p % W);
         // ATen area_pixel_compute_source_index + guard_index_and_lambda (align_corners=True)
-        const float ry = sy * (float)Y, rx = sx * (float)X;
-        const int y0 = min((int)ry, h2 - 1), x0 = min((int)rx, w2 - 1);
-        const int y1 = min(y0 + 1, h2 - 1), x1 = min(x0 + 1, w2 - 1);
-        const float ly1 = fminf(fmaxf(ry - (float)y0, 0.f), 1.f), lx1 = fminf(fmaxf(rx - (float)x0, 0.f), 1.f);
+        const float ry = sy * (float)(row0 + Y), rx = sx * (float)X;
+        const int gy0 = min((int)ry, ht2 - 1), x0 = min((int)rx, w2 - 1);
+        const int gy1 = min(gy0 + 1, ht2 - 1), x1 = min(x0 + 1, w2 - 1);
+        const float ly1 = fminf(fmaxf(ry - (float)gy0, 0.f), 1.f), lx1 = fminf(fmaxf(rx - (float)x0, 0.f), 1.f);
         const float ly0 = 1.f - ly1, lx0 = 1.f - lx1;
+        const int y0 = min(max(gy0 - hr0, 0), h2 - 1), y1 = min(max(gy1 - hr0, 0), h2 - 1);
         const float* src = mosaic + (long)wrap(f - 1 + j, B) * plane;
         const float* s = a2 + (3 * j + 1) * 4;
         const float* xb = xo4 + (long)n * hplane * Cp;
@@ -358,46 +371,76 @@ inline int grid1d(long n, int block = 256) { return (int)((n + block - 1) / bloc
 
 }  // namespace
 
+#define DD_FRAMES_OK (B > 0 && f0 >= 0 && Bc > 0 && f0 + Bc <= B)
+
+extern "C" int sci_ddnet_pack_input1_frames(const float* mosaic, const float* a, float* out, int B, int f0, int Bc, int H,
+                                            int W, int Cpad, int split_tf32, void* stream) {
+    SCI_REQUIRE(mosaic && a && out && DD_FRAMES_OK && H > 0 && W > 0 && Cpad == DD_CP, "ddnet_pack_input1");
+    const long plane = (long)H * W;
+    dd_pack1_kernel<<<dim3(grid1d(plane, DD_PIX), 3 * Bc), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a, out, B, f0, Bc, plane,
+                                                                                            split_tf32);
+    SCI_CHECK_LAUNCH("ddnet_pack_input1");
+    return SCI_OK;
+}
+
 extern "C" int sci_ddnet_pack_input1(const float* mosaic, const float* a, float* out, int B, int H, int W, int Cpad,
                                      int split_tf32, void* stream) {
-    SCI_REQUIRE(mosaic && a && out && B > 0 && H > 0 && W > 0 && Cpad == DD_CP, "ddnet_pack_input1");
-    const long plane = (long)H * W;
-    dd_pack1_kernel<<<dim3(grid1d(plane, DD_PIX), 3 * B), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a, out, B, plane, split_tf32);
-    SCI_CHECK_LAUNCH("ddnet_pack_input1");
+    return sci_ddnet_pack_input1_frames(mosaic, a, out, B, 0, B, H, W, Cpad, split_tf32, stream);
+}
+
+extern "C" int sci_ddnet_pack_input4_frames(const float* mosaic, const float* a2, float* out, int B, int f0, int Bc, int H,
+                                            int W, int Cpad, int split_tf32, void* stream) {
+    SCI_REQUIRE(mosaic && a2 && out && DD_FRAMES_OK && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0 && Cpad == DD_CP,
+                "ddnet_pack_input4");
+    const long hplane = (long)(H / 2) * (W / 2);
+    dd_pack4_kernel<<<dim3(grid1d(hplane, DD_PIX), 3 * Bc), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a2, out, B, f0, Bc, H, W,
+                                                                                             split_tf32);
+    SCI_CHECK_LAUNCH("ddnet_pack_input4");
     return SCI_OK;
 }
 
 extern "C" int sci_ddnet_pack_input4(const float* mosaic, const float* a2, float* out, int B, int H, int W, int Cpad,
                                      int split_tf32, void* stream) {
-    SCI_REQUIRE(mosaic && a2 && out && B > 0 && H > 0 && W > 0 && H % 2 == 0 && W % 2 == 0 && Cpad == DD_CP,
-                "ddnet_pack_input4");
-    const long hplane = (long)(H / 2) * (W / 2);
-    dd_pack4_kernel<<<dim3(grid1d(hplane, DD_PIX), 3 * B), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a2, out, B, H, W, split_tf32);
-    SCI_CHECK_LAUNCH("ddnet_pack_input4");
+    return sci_ddnet_pack_input4_frames(mosaic, a2, out, B, 0, B, H, W, Cpad, split_tf32, stream);
+}
+
+extern "C" int sci_ddnet_stage2_input_frames(const float* mosaic, const float* a, const float* xo, int xo_cpad, float* t2in,
+                                             float* res, int B, int f0, int Bc, int H, int W, int Cpad, int split_tf32,
+                                             void* stream) {
+    SCI_REQUIRE(xo && t2in && res && DD_FRAMES_OK && H > 0 && W > 0 && Cpad == DD_CP && xo_cpad >= 3, "ddnet_stage2_input");
+    SCI_REQUIRE((mosaic == nullptr) == (a == nullptr), "ddnet_stage2_input: mosaic and a go together");
+    const long plane = (long)H * W;
+    dd_mid_kernel<<<dim3(grid1d(plane, DD_PIX), Bc), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a, xo, xo_cpad, t2in, res, B, f0,
+                                                                                      Bc, plane, split_tf32);
+    SCI_CHECK_LAUNCH("ddnet_stage2_input");
     return SCI_OK;
 }
 
 extern "C" int sci_ddnet_stage2_input(const float* mosaic, const float* a, const float* xo, int xo_cpad, float* t2in,
                                       float* res, int B, int H, int W, int Cpad, int split_tf32, void* stream) {
-    SCI_REQUIRE(xo && t2in && res && B > 0 && H > 0 && W > 0 && Cpad == DD_CP && xo_cpad >= 3, "ddnet_stage2_input");
-    SCI_REQUIRE((mosaic == nullptr) == (a == nullptr), "ddnet_stage2_input: mosaic and a go together");
+    return sci_ddnet_stage2_input_frames(mosaic, a, xo, xo_cpad, t2in, res, B, 0, B, H, W, Cpad, split_tf32, stream);
+}
+
+extern "C" int sci_ddnet_upsample4_strip(const float* mosaic, const float* a2, const float* xo4, int xo_cpad, float* out,
+                                         int B, int f0, int Bc, int H, int W, int row0, int H_total, int Cpad, int split_tf32,
+                                         void* stream) {
+    SCI_REQUIRE(mosaic && a2 && xo4 && out && DD_FRAMES_OK && H >= 2 && W >= 4 && H % 2 == 0 && W % 2 == 0 &&
+                Cpad == DD_CP && xo_cpad >= 4, "ddnet_upsample4");
+    SCI_REQUIRE(row0 >= 0 && row0 % 2 == 0 && H_total >= 4 && H_total % 2 == 0 && row0 + H <= H_total,
+                "ddnet_upsample4: rows [row0, row0+H) must be an even-aligned part of the H_total-row frame");
     const long plane = (long)H * W;
-    dd_mid_kernel<<<dim3(grid1d(plane, DD_PIX), B), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a, xo, xo_cpad, t2in, res, B, plane,
-                                                                                     split_tf32);
-    SCI_CHECK_LAUNCH("ddnet_stage2_input");
+    // the scale factors of the WHOLE frame, with the float operations of ATen's area_pixel_compute_scale
+    const float sy = (float)(H_total / 2 - 1) / (float)(H_total - 1), sx = (float)(W / 2 - 1) / (float)(W - 1);
+    dd_up4_kernel<<<dim3(grid1d(plane, DD_PIX), 3 * Bc), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a2, xo4, xo_cpad, out, B, f0,
+                                                                                          Bc, H, W, row0, H_total, sy, sx,
+                                                                                          split_tf32);
+    SCI_CHECK_LAUNCH("ddnet_upsample4");
     return SCI_OK;
 }
 
 extern "C" int sci_ddnet_upsample4(const float* mosaic, const float* a2, const float* xo4, int xo_cpad, float* out, int B,
                                    int H, int W, int Cpad, int split_tf32, void* stream) {
-    SCI_REQUIRE(mosaic && a2 && xo4 && out && B > 0 && H >= 4 && W >= 4 && H % 2 == 0 && W % 2 == 0 && Cpad == DD_CP &&
-                xo_cpad >= 4, "ddnet_upsample4");
-    const long plane = (long)H * W;
-    const float sy = (float)(H / 2 - 1) / (float)(H - 1), sx = (float)(W / 2 - 1) / (float)(W - 1);
-    dd_up4_kernel<<<dim3(grid1d(plane, DD_PIX), 3 * B), DD_PIX, 0, sci_stream(stream)>>>(mosaic, a2, xo4, xo_cpad, out, B, H, W,
-                                                                                         sy, sx, split_tf32);
-    SCI_CHECK_LAUNCH("ddnet_upsample4");
-    return SCI_OK;
+    return sci_ddnet_upsample4_strip(mosaic, a2, xo4, xo_cpad, out, B, 0, B, H, W, 0, H, Cpad, split_tf32, stream);
 }
 
 extern "C" int sci_ddnet_output(const float* res1, const float* res2, const float* xo2, int xo_cpad, const float* a3,

@@ -227,16 +227,27 @@ class _TileView:
         self.g0 = tile.r0 - top                      # global row of the first row of the extended strip
 
 
-def _tiled_demosaic_denoise(tile, adapter, halo, x, b, inv_rou, w, tau, x_rgb, u, pb, nsig, model, lr_, do_update,
-                            update_per_iter, grad_sync):
-    """One demosaic + denoise step of a row strip (SURVEY 8(e)): 2-row mosaic halo for Malvar, `halo` rows of the denoiser
-    input, overlap-tile denoising, crop.  x_rgb and u (own rows) are filled in place; returns xhat (own rows)."""
+def _tiled_demosaic(tile, x, b, inv_rou, w, tau, x_rgb, u, model_demosaic, mosaic):
+    """The demosaic step of a row strip (SURVEY 8(e)): DDnet on strips (``DDnetEngine.forward_tiled``: 88 rows of the
+    merged mosaic, 40 rows of its temp2 input) or Malvar (2 rows of the merged mosaic), then u = x_rgb - w/tau.  u (own
+    rows) is filled in place; returns x_rgb (own rows: ``x_rgb`` itself for Malvar, the engine's buffer for DDnet)."""
     B, rows, W = x.shape
-    m_ext, top2 = tile.exchange(ops.axpy(x, inv_rou, b).view(B, 1, rows, W), 2)        # merged mosaic x + b/rho
-    rgb_ext = torch.empty((B, 3, m_ext.shape[2], W), dtype=torch.float32, device=x.device)
-    ops.malvar2004(m_ext.view(B, m_ext.shape[2], W), None, 0.0, None, 0.0, rgb_ext, None)
-    x_rgb.copy_(rgb_ext[:, :, top2:top2 + rows])
+    if model_demosaic is not None:
+        from . import ddnet_adapter
+        x_rgb = ddnet_adapter._unwrap(model_demosaic).engine().forward_tiled(ops.axpy(x, inv_rou, b, out=mosaic), tile)
+    else:
+        m_ext, top2 = tile.exchange(ops.axpy(x, inv_rou, b).view(B, 1, rows, W), 2)    # merged mosaic x + b/rho
+        rgb_ext = torch.empty((B, 3, m_ext.shape[2], W), dtype=torch.float32, device=x.device)
+        ops.malvar2004(m_ext.view(B, m_ext.shape[2], W), None, 0.0, None, 0.0, rgb_ext, None)
+        x_rgb.copy_(rgb_ext[:, :, top2:top2 + rows])
     ops.axpy(x_rgb, -float(np.float32(1 / tau)), w, out=u)                              # u = x_rgb - w/tau (:198)
+    return x_rgb
+
+
+def _tiled_denoise(tile, adapter, halo, u, pb, nsig, model, lr_, do_update, update_per_iter, grad_sync):
+    """The denoise step of a row strip: `halo` rows of the denoiser input u (own rows), overlap-tile denoising, crop;
+    FastDVDnet inference instead exchanges 40 rows per DenBlock.  Returns xhat (own rows)."""
+    rows = u.shape[2]
     if adapter.__name__.endswith("fastdvdnet_adapter") and not do_update:
         # inference: one 40-row exchange per DenBlock instead of an 80-row overlap for the whole cascade
         return adapter._unwrap(model).engine().forward_tiled(u, nsig, tile)
@@ -309,15 +320,20 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
     ``return_device`` (extension) returns the planar device tensors ``(xhat[B,3,H,W], theta[B,H,W])`` instead of
     numpy arrays (no D2H copy, no host sync) — used by bench.py for the HBM-resident measurement.
     ``tile`` (extension, ``parallel.TileContext``): spatial row-strip tiling of one large frame over the ranks (BASELINE
-    config 5).  Every rank passes ITS rows of y / Phi / x0 / X_orig; the mosaic (2 rows) and the denoiser input (80 rows
-    for FastDVDnet, 28 for FFDNet; 8 rows of the TV input and an all-gather of its early-stop energies for 'tv') are
-    halo-exchanged with the neighbouring ranks once per iteration, PSNR sums and the fine-tune gradients are all-reduced,
-    and the returned arrays are the full frame (gathered on every rank).
+    config 5).  Every rank passes ITS rows of y / Phi / x0 / X_orig; the mosaic (2 rows for Malvar; for DDnet 88 rows, and
+    40 rows of its temp2 input per frame chunk) and the denoiser input (80 rows for FastDVDnet, 28 for FFDNet; 8 rows of the
+    TV input and an all-gather of its early-stop energies for 'tv') are halo-exchanged with the neighbouring ranks once per
+    iteration, PSNR sums and the fine-tune gradients are all-reduced, and the returned arrays are the full frame (gathered
+    on every rank).  The closed-form demosaic is pixel-wise and needs no halo.  DDnet needs strips and a width that are
+    multiples of 8, and strips of at least 88 rows over several ranks (ValueError otherwise).
     """
     name = denoiser if denoiser == 'tv' else str(denoiser).lower()
     if name not in ('tv', 'ffdnet_color', 'fastdvd_color'):
         raise ValueError('Unsupported denoiser {}!'.format(denoiser))
     sigma, iter_max = _as_list(sigma, iter_max)
+    if tile is not None and name != 'tv' and model_demosaic is not None:
+        from .engine import DDnetEngine
+        DDnetEngine.check_tile(tile)                                   # strips DDnet cannot run on: refused before GPU work
     pb = _Problem(y_bayer, Phi_bayer, x0_bayer, X_orig)
     dev = pb.y.device
     H, W, B = pb.H, pb.W, pb.B
@@ -329,7 +345,11 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
         else:
             if grad_sync is None:
                 grad_sync = tile.all_reduce_sum      # loss is normalised by the whole frame -> gradients ADD over strips
-            tile.enable_p2p(3 * B, 28 if name == 'ffdnet_color' else 80)  # boundary rows go peer to peer over NVLink
+            exchanges = [(3 * B, 28 if name == 'ffdnet_color' else 80)]    # (planes, rows) of the largest exchanges
+            if model_demosaic is not None:
+                bc = DDnetEngine.tiled_chunk_frames(B, tile)
+                exchanges += [(B, DDnetEngine.STAGE_A_HALO), (2 * bc * 32, DDnetEngine.STAGE_B_HALO)]
+            tile.enable_p2p(*max(exchanges, key=lambda e: e[0] * e[1]))   # boundary rows go peer to peer over NVLink
     alpha = 0.01 if name == 'tv' else 1                                  # :101-104
     rou = 0.55 if name == 'fastdvd_color' else 1                         # :106-109
     tau = 100                                                            # :110
@@ -382,26 +402,22 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
                 adapter = ffdnet_adapter if name == 'ffdnet_color' else fastdvdnet_adapter
                 if close_form_demosaic and k > 0:
                     # x_rgb = (rho*x3 + b3 + tau*xhat + w) / (rho*mask + tau) [clip for FFDNet] ; u = x_rgb - w/tau   (:175-182)
-                    if tile is not None:
-                        raise NotImplementedError("tiled mode does not cover the closed-form demosaic branch")
+                    # (pixel-wise: on a strip its own rows, the Bayer phase kept by rows % 4 == 0)
                     ops.closed_form_demosaic(x, b, xhat, w, rou, tau, name == 'ffdnet_color', x_rgb, u)
-                    xhat = adapter.denoise_planar(u, pb, nsig, model_denoise, lr_, do_update, update_per_iter,
-                                                  grad_sync=grad_sync)
+                elif tile is not None:
+                    x_rgb = _tiled_demosaic(tile, x, b, inv_rou, w, tau, x_rgb, u, model_demosaic, mosaic)
                 elif model_demosaic is not None:
                     # deep demosaicking: x_rgb = DDnet(merge(x + b/rho)) ; u = x_rgb - w/tau          (:192-198, :241-246)
-                    if tile is not None:
-                        raise NotImplementedError("tiled mode uses the Malvar demosaic (DDnet would need its own halo)")
                     x_rgb = ddnet_adapter.demosaic_planar(ops.axpy(x, inv_rou, b, out=mosaic), model_demosaic)
                     ops.axpy(x_rgb, -float(np.float32(1 / tau)), w, out=u)
-                    xhat = adapter.denoise_planar(u, pb, nsig, model_denoise, lr_, do_update, update_per_iter,
-                                                  grad_sync=grad_sync)
-                elif tile is None:
+                else:
                     ops.malvar2004(x, b, inv_rou, w, 1 / tau, x_rgb, u)
+                if tile is None:
                     xhat = adapter.denoise_planar(u, pb, nsig, model_denoise, lr_, do_update, update_per_iter,
                                                   grad_sync=grad_sync)
                 else:
-                    xhat = _tiled_demosaic_denoise(tile, adapter, 28 if name == 'ffdnet_color' else 80, x, b, inv_rou, w, tau,
-                                                   x_rgb, u, pb, nsig, model_denoise, lr_, do_update, update_per_iter, grad_sync)
+                    xhat = _tiled_denoise(tile, adapter, 28 if name == 'ffdnet_color' else 80, u, pb, nsig, model_denoise,
+                                          lr_, do_update, update_per_iter, grad_sync)
                 # theta = clip(RGGB samples of xhat) ; b += x - theta ; w += x_rgb - xhat [+ PSNR]    (:206-209, :265-280)
                 ops.dual_update_rgb(xhat, x_rgb, w, x, b, theta, first_iter=(k == 0),
                                     orig=pb.orig if want_iqa else None, sse=sse[k:k + 1] if want_iqa else None)

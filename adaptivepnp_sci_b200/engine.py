@@ -837,11 +837,12 @@ class DDnetEngine(_EngineBase):
                     for i, (c, r, st, ps) in enumerate(module.temp11.fusion_specs())]
         super().__init__(module, self.t1 + self.t11 + self.fus + self.t2)
 
-    def _body(self, L, a_in, N, H, W, keep=None):
+    def _body(self, L, a_in, N, H, W, keep=None, cap=None):
         """The 16-conv U-shaped body shared by all DenBlock variants (:232-241): returns the last conv's output.
-        ``keep`` (a tag): every activation gets its own buffer and the dict of them is returned too (training)."""
+        ``keep`` (a tag): every activation gets its own buffer and the dict of them is returned too (training).
+        ``cap`` >= N: buffers are allocated for ``cap`` images and used for the first N (the ragged last frame chunk)."""
         dev = a_in.device
-        g = self.ws.get
+        g = lambda name, shape, dev: self.ws.get(name, (cap or shape[0],) + shape[1:], dev)[:shape[0]]
         h2, w2, h4, w4 = H // 2, W // 2, H // 4, W // 4
         S = {"a_in": a_in}
 
@@ -914,58 +915,143 @@ class DDnetEngine(_EngineBase):
         d_a0 = bw(L[1], d_x0, S["x0"], S["a0"], N, H, W, nm("f_w"))
         return bw(L[0], d_a0, S["a0"], S["a_in"], N, H, W, nm("f_in"), want_dx=want_dx)
 
+    # Row strips (forward_tiled).  Receptive field of one output row, measured on the float64 oracle (tests/test_ddnet_halo.py):
+    # path 1 (temp1) -40..+37 rows, path 2 (pack, temp11 at half resolution, bilinear x2, fusion) -84..+78, temp2 -40..+37.
+    STAGE_A_HALO = 88    # rows of the mosaic for both paths up to the temp2 input; a multiple of 8 (path 2 goes down by 8)
+    STAGE_B_HALO = 40    # rows of the temp2 input (the U-shaped body, FastDVDnetEngine.BLOCK_HALO)
+    # frame chunks: images x pixels of one path-1 body pass (3 images per centre frame).  The activations of a pass grow with
+    # it (fp32 NHWC, 32..128 padded channels per level, three bodies); the budget keeps every size the tests and the
+    # single-GPU benchmarks run in one pass and a 2048-wide strip of a 24-frame sequence in a few passes
+    PASS_PIXELS = 1 << 24
+
+    @classmethod
+    def chunk_frames(cls, B, H, W):
+        """Centre frames per pass for a B-frame sequence of H x W mosaics: at most PASS_PIXELS / (3 H W), the chunks made as
+        even as that allows.  Every image's convolutions are the same whatever the chunk, so chunking changes no bit."""
+        most = max(1, cls.PASS_PIXELS // (3 * H * W))
+        n = -(-B // most)
+        return -(-B // n)
+
+    @classmethod
+    def tiled_chunk_frames(cls, B, tile):
+        """Chunk of forward_tiled: from the frame's global sizes (the longest halo-extended strip), so that every rank runs
+        the same number of halo exchanges (P2PRegion counts them in lock-step)."""
+        return cls.chunk_frames(B, min(tile.rows + 2 * cls.STAGE_A_HALO, tile.H_total), tile.W)
+
+    @classmethod
+    def check_tile(cls, tile):
+        """Refuse strips forward_tiled cannot reproduce the whole frame on (before any GPU work)."""
+        if tile.rows % 8 or tile.W % 8:
+            raise ValueError("DDnet on row strips needs strips and width that are multiples of 8 (the half-resolution path "
+                             "goes down by 8; strip starts must keep its stride phases), got %d rows x %d" % (tile.rows, tile.W))
+        if tile.world > 1 and tile.rows < cls.STAGE_A_HALO:
+            raise ValueError("DDnet on row strips: strips of %d rows are shorter than its %d-row halo (use fewer ranks for a "
+                             "%d-row frame)" % (tile.rows, cls.STAGE_A_HALO, tile.H_total))
+
     def forward(self, mosaic, train=False):
-        """mosaic [B,H,W] planar (whole circular sequence) -> demosaicked [B,3,H,W].  train=True keeps the activations."""
+        """mosaic [B,H,W] planar (whole circular sequence) -> demosaicked [B,3,H,W].  train=True keeps the activations.
+        Inference runs the centre frames in chunks of ``chunk_frames`` (training in one pass: backward() needs it all)."""
         B, H, W = mosaic.shape
         if H % 8 or W % 8:
             raise NotImplementedError("native DDnet engine needs H, W multiples of 8 (half-resolution path with two "
                                       "stride-2 levels; the reference reflect-pads to 4, DDnet_test.py:180-187, and "
                                       "would itself fail on sizes that are not multiples of 8)")
         self.prepare(training=train)
+        out = self.ws.get("dd_tr_out" if train else "dd_out", (B, 3, H, W), mosaic.device)
+        Bc = B if train else self.chunk_frames(B, H, W)
         self.pdl_chain = (not train) and self.profile is None and self.impl == IMPL_TC      # see FastDVDnetEngine.forward
         try:
-            return self._forward(mosaic, train)
+            for f0 in range(0, B, Bc):
+                bc = min(Bc, B - f0)
+                t2in, res1, res2 = self._stage_a(mosaic, f0, bc, Bc, 0, H, train)
+                self._stage_b(t2in, res1, res2, bc, Bc, H, W, out[f0:f0 + bc], train)
         finally:
             self.pdl_chain = False
+        if train:
+            self._saved.update(mosaic=mosaic, B=B, H=H, W=W)
+        return out
 
-    def _forward(self, mosaic, train):
+    def forward_tiled(self, mosaic_own, tile):
+        """Inference on a row strip of a larger frame (``parallel.TileContext``): mosaic_own [B,rows,W], this rank's rows of
+        the whole sequence -> demosaicked own rows [B,3,rows,W] (engine-owned buffer, valid until the next call).
+
+        The mosaic is exchanged once with STAGE_A_HALO rows; per frame chunk both paths run on that extended strip up to the
+        temp2 input, whose own rows are exchanged with STAGE_B_HALO rows (the packed NHWC rows as they are, viewed as
+        [2Bc,1,rows,32W]); temp2 runs on that and the output mix on the own rows (res1 / res2 are used pixel-wise, they need
+        no halo).  Extended strips start on global rows that are multiples of 8, so every stride phase is that of the whole
+        frame, zero padding applies only at true image borders and the own rows are those of ``forward``."""
+        B, rows, W = mosaic_own.shape
+        self.prepare(training=False)
+        m_ext, top = tile.exchange(mosaic_own.view(B, 1, rows, W), self.STAGE_A_HALO)
+        m_ext = m_ext.view(B, m_ext.shape[2], W)
+        out = self.ws.get("ddt_out", (B, 3, rows, W), mosaic_own.device)
+        Bc = self.tiled_chunk_frames(B, tile)
+        self.pdl_chain = self.profile is None and self.impl == IMPL_TC
+        try:
+            for f0 in range(0, B, Bc):
+                bc = min(Bc, B - f0)
+                t2in, res1, res2 = self._stage_a(m_ext, f0, bc, Bc, tile.r0 - top, tile.H_total, False)
+                own = t2in[:, top:top + rows].contiguous().view(2 * bc, 1, rows, W * 32)
+                t2_ext, top2 = tile.exchange(own, self.STAGE_B_HALO)
+                self._stage_b(t2_ext.view(2 * bc, -1, W, 32), res1[:, :, top:top + rows].contiguous(),
+                              res2[:, :, top:top + rows].contiguous(), bc, Bc, rows, W, out[f0:f0 + bc], False, top2)
+        finally:
+            self.pdl_chain = False
+        return out
+
+    def _stage_a(self, mosaic, f0, bc, cap, row0, H_total, train):
+        """Both paths up to the temp2 input for the centre frames [f0, f0+bc) of mosaic [B,H,W], whose row 0 is row ``row0``
+        of an ``H_total``-row frame.  Returns t2in [2bc,H,W,32] (path 1, then path 2), res1, res2 [bc,3,H,W]; buffers hold
+        ``cap`` frames."""
         B, H, W = mosaic.shape
         dev = mosaic.device
         m = self.module
-        a, a2, a3 = m.weight_tensor_in.data, m.weight_tensor_in2.data, m.weight_tensor_out.data
+        a, a2 = m.weight_tensor_in.data, m.weight_tensor_in2.data
         sp = int(self.tf32)
-        g = self.ws.get
         t = "tr_" if train else ""
-        t2in = g("dd_%st2in" % t, (2 * B, H, W, 32), dev)
-        res1, res2 = g("dd_%sres1" % t, (B, 3, H, W), dev), g("dd_%sres2" % t, (B, 3, H, W), dev)
+        g = lambda name, k, shape: self.ws.get("dd_%s%s" % (t, name), (k * cap,) + shape, dev)[:k * bc]
+        keep = (lambda tag: tag) if train else (lambda tag: None)
+        t2in = g("t2in", 2, (H, W, 32))
+        res1, res2 = g("res1", 1, (3, H, W)), g("res2", 1, (3, H, W))
         # path 1: full-resolution single-channel triples
-        in1 = g("dd_%sin1" % t, (3 * B, H, W, 32), dev)
-        call("sci_ddnet_pack_input1", ptr(mosaic), ptr(a), ptr(in1), B, H, W, 32, sp, stream())
-        r1 = self._body(self.t1, in1, 3 * B, H, W, keep="t1" if train else None)
+        in1 = g("in1", 3, (H, W, 32))
+        call("sci_ddnet_pack_input1_frames", ptr(mosaic), ptr(a), ptr(in1), B, f0, bc, H, W, 32, sp, stream())
+        r1 = self._body(self.t1, in1, 3 * bc, H, W, keep=keep("t1"), cap=3 * cap)
         xo1, S1 = r1 if train else (r1, None)
-        call("sci_ddnet_stage2_input", ptr(mosaic), ptr(a), ptr(xo1), xo1.shape[-1], ptr(t2in), ptr(res1), B, H, W, 32, sp,
-             stream())
+        call("sci_ddnet_stage2_input_frames", ptr(mosaic), ptr(a), ptr(xo1), xo1.shape[-1], ptr(t2in), ptr(res1), B, f0, bc,
+             H, W, 32, sp, stream())
         # path 2: half-resolution RGGB planes, residual, bilinear x2, fusion convs
-        in4 = g("dd_%sin4" % t, (3 * B, H // 2, W // 2, 32), dev)
-        call("sci_ddnet_pack_input4", ptr(mosaic), ptr(a2), ptr(in4), B, H, W, 32, sp, stream())
-        r4 = self._body(self.t11, in4, 3 * B, H // 2, W // 2, keep="t11" if train else None)
+        in4 = g("in4", 3, (H // 2, W // 2, 32))
+        call("sci_ddnet_pack_input4_frames", ptr(mosaic), ptr(a2), ptr(in4), B, f0, bc, H, W, 32, sp, stream())
+        r4 = self._body(self.t11, in4, 3 * bc, H // 2, W // 2, keep=keep("t11"), cap=3 * cap)
         xo4, S4 = r4 if train else (r4, None)
-        up = g("dd_%sup" % t, (3 * B, H, W, 32), dev)
-        call("sci_ddnet_upsample4", ptr(mosaic), ptr(a2), ptr(xo4), xo4.shape[-1], ptr(up), B, H, W, 32, sp, stream())
-        f0 = g("dd_%sf0" % t, (3 * B, H, W, self.fus[0].out_ch), dev)
-        self.conv(self.fus[0], up, 3 * B, H, W, f0)
-        xf = g("dd_%sxf" % t, (3 * B, H, W, self.fus[1].out_ch), dev)
-        self.conv(self.fus[1], f0, 3 * B, H, W, xf, round_out=False)
-        call("sci_ddnet_stage2_input", None, None, ptr(xf), xf.shape[-1], ptr(t2in[B:]), ptr(res2), B, H, W, 32, sp, stream())
-        # temp2 on both paths (one batch of 2B), then the learnable output mix
-        r2 = self._body(self.t2, t2in, 2 * B, H, W, keep="t2" if train else None)
-        xo2, S2 = r2 if train else (r2, None)
-        out = g("dd_%sout" % t, (B, 3, H, W), dev)
-        call("sci_ddnet_output", ptr(res1), ptr(res2), ptr(xo2), xo2.shape[-1], ptr(a3), ptr(out), B, H, W, stream())
-        self.n_launch += 6
+        up = g("up", 3, (H, W, 32))
+        call("sci_ddnet_upsample4_strip", ptr(mosaic), ptr(a2), ptr(xo4), xo4.shape[-1], ptr(up), B, f0, bc, H, W, row0,
+             H_total, 32, sp, stream())
+        f0_ = g("f0", 3, (H, W, self.fus[0].out_ch))
+        self.conv(self.fus[0], up, 3 * bc, H, W, f0_)
+        xf = g("xf", 3, (H, W, self.fus[1].out_ch))
+        self.conv(self.fus[1], f0_, 3 * bc, H, W, xf, round_out=False)
+        call("sci_ddnet_stage2_input_frames", None, None, ptr(xf), xf.shape[-1], ptr(t2in[bc:]), ptr(res2), bc, 0, bc, H, W,
+             32, sp, stream())
+        self.n_launch += 5
         if train:
-            self._saved = dict(mosaic=mosaic, B=B, H=H, W=W, S1=S1, S4=S4, S2=S2, up=up, f0=f0, xf=xf, res1=res1, res2=res2, xo2=xo2)
-        return out
+            self._saved = dict(S1=S1, S4=S4, up=up, f0=f0_, xf=xf, res1=res1, res2=res2)
+        return t2in, res1, res2
+
+    def _stage_b(self, t2in, res1, res2, bc, cap, rows, W, out, train, top=0):
+        """temp2 on both paths (one batch of 2bc) and the learnable output mix of the ``rows`` rows from ``top`` on.
+        t2in [2bc,top+rows+bot,W,32], res1 / res2 [bc,3,rows,W] -> out [bc,3,rows,W]."""
+        Ht = t2in.shape[1]
+        r2 = self._body(self.t2, t2in, 2 * bc, Ht, W, keep="t2" if train else None, cap=2 * cap)
+        xo2, S2 = r2 if train else (r2, None)
+        if Ht != rows:
+            xo2 = xo2[:, top:top + rows].contiguous()
+        a3 = self.module.weight_tensor_out.data
+        call("sci_ddnet_output", ptr(res1), ptr(res2), ptr(xo2), xo2.shape[-1], ptr(a3), ptr(out), bc, rows, W, stream())
+        self.n_launch += 1
+        if train:
+            self._saved.update(S2=S2, xo2=xo2)
 
     def backward(self, dout):
         """Gradients of ALL trained parameters (convs of temp1 / temp11 / fusion / temp2 and the three mixing tensors) into

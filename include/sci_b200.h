@@ -405,6 +405,21 @@ int sci_ddnet_upsample4(const float* mosaic, const float* a2, const float* xo4, 
                         int W, int Cpad, int split_tf32, void* stream);
 int sci_ddnet_output(const float* res1, const float* res2, const float* xo2, int xo_cpad, const float* a3, float* out,
                      int B, int H, int W, void* stream);
+/* Frame chunks and row strips of the same kernels.  *_frames evaluate the centre frames [f0, f0+Bc) of the B-frame
+ * sequence (0 <= f0, Bc > 0, f0+Bc <= B): batch n = j*Bc + (f-f0) in out / xo / t2in / res (Bc frames), frame reads stay
+ * (f-2+j+k) mod B over the whole mosaic [B][H][W].  upsample4_strip also takes the global row row0 (even) of the first of
+ * the H rows held and the height H_total of the whole frame (row0 + H <= H_total): the bilinear source coordinate is that
+ * of the whole frame, source rows outside the held ones are clamped to them (output rows within one row of a strip edge
+ * whose neighbour rows are not held are therefore not those of the whole frame; a caller with a halo discards them).
+ * The whole-frame entry points above are these with f0 = 0, Bc = B, row0 = 0, H_total = H. */
+int sci_ddnet_pack_input1_frames(const float* mosaic, const float* a, float* out, int B, int f0, int Bc, int H, int W,
+                                 int Cpad, int split_tf32, void* stream);
+int sci_ddnet_pack_input4_frames(const float* mosaic, const float* a2, float* out, int B, int f0, int Bc, int H, int W,
+                                 int Cpad, int split_tf32, void* stream);
+int sci_ddnet_stage2_input_frames(const float* mosaic, const float* a, const float* xo, int xo_cpad, float* t2in,
+                                  float* res, int B, int f0, int Bc, int H, int W, int Cpad, int split_tf32, void* stream);
+int sci_ddnet_upsample4_strip(const float* mosaic, const float* a2, const float* xo4, int xo_cpad, float* out, int B,
+                              int f0, int Bc, int H, int W, int row0, int H_total, int Cpad, int split_tf32, void* stream);
 /* Backward of the DDnet boundary (self-supervised demosaicker update, DDnet_test.py:231-276).
  *   loss_fwd_bwd     : loss += mean over [B][3][H][W] of (v - site(out))^2, site() keeps the RGGB site of each channel
  *                      (DDnet_test.py:208-216, :268); dout (may be NULL) = d loss / d out
