@@ -73,6 +73,7 @@ PROTOTYPES = {
     "sci_halo_send_tv": [_p, _p, _f, _i, _i, _i, _i, _p, _p, _p, _p, ctypes.c_uint, _p, _p],
     "sci_halo_assemble": [_p, _i, _i, _i, _i, _i, _p, _p, _p, _p, ctypes.c_uint, _p, _p, _p],
     "sci_fastdvd_pack_input_half": [_p, _f, _p, _i, _i, _i, _i, _p],
+    "sci_fastdvd_pack_input_half_planes": [_p, _f, _p, _i, _i, _i, _i, _i, _p],
     "sci_conv_unpack_wgrad": [_p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
     "sci_bn_fold": [_p, _p, _p, _p, _f, _p, _p, _i, _i, _p],
     "sci_act_bwd": [_p, _p, _p, _l, _i, _i, _p, _p, _p],
@@ -89,6 +90,10 @@ PROTOTYPES = {
     "sci_fastdvd_output": [_p, _p, _p, _i, _i, _i, _i, _p],
     "sci_fastdvd_output_grad": [_p, _p, _i, _i, _i, _i, _p],
     "sci_fastdvd_pack_input_grad": [_p, _p, _i, _i, _i, _i, _i, _p],
+    "sci_fastdvd_pack_input_planes": [_p, _f, _p, _i, _i, _i, _i, _i, _i, _p],
+    "sci_fastdvd_output_planes": [_p, _p, _p, _i, _i, _i, _i, _i, _p],
+    "sci_fastdvd_output_grad_planes": [_p, _p, _i, _i, _i, _i, _i, _p],
+    "sci_fastdvd_pack_input_grad_planes": [_p, _p, _i, _i, _i, _i, _i, _i, _p],
     "sci_fastdvd_noisy_input": [_p, _p, _p, _l, _p],
     "sci_rgb_sum": [_p, _p, _i, _i, _i, _p],
     "sci_ddnet_pack_input1": [_p, _p, _p, _i, _i, _i, _i, _i, _p],

@@ -435,7 +435,7 @@ struct Fwd2Params {
     const float* scale; const float* shift; const float* residual; float* y;
     int N, H, W, Cin, Cout, relu, ps, round_tf32;
     int tiles_w, num_tiles, k_chunks, stages, acc_stride, tmem_cols, resident, out_bufs;
-    const float* planar_in1; float* planar_out;   // fused network output: out[n][c][h][w] = in1[n][c][h][w] - conv[c], c < 3
+    const float* planar_in1; float* planar_out;   // fused network output: out[n][c][h][w] = in1[n][c][h][w] - conv[c], c < 3 (MODE 3: 1)
     int pdl;          // launched with programmatic stream serialization: see griddepcontrol below
     int col0, Ctot;   // this launch computes GEMM columns [col0, col0 + Cout) of a layer with Ctot columns (Cout = 256 layers run as two halves)
     int stack;        // filter rows stacked along N (see the MMA issuer); needs resident weights, R >= 2, 3*Cout <= 256
@@ -469,7 +469,7 @@ struct Fwd2Params {
 //     second group shares the quarters and takes every second (row, chunk) unit): two warps per scheduler hide each
 //     other's latencies;
 //   * MODE selects the epilogue at compile time (0 = TMA store, 1 = TMA store + skip-add, 2 = fused planar network
-//     output, 4 = data gradient with the fused activation backward) instead of run-time flags per element; scale / shift come from shared memory as float4;
+//     output of 3 planes, 3 = the same with 1 plane (gray), 4 = data gradient with the fused activation backward) instead of run-time flags per element; scale / shift come from shared memory as float4;
 //   * the planar mode fetches the in1 values of ALL its rows before it waits for the accumulator (the per-row prefetch
 //     left the HBM latency of those loads exposed: 46 % of the epilogue's samples in the 32->3 layer).
 //   * HALF: fp16 storage and operands (kind::f16, fp32 accumulation): the same 11-bit significand as TF32 - the products
@@ -769,6 +769,8 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         const int nch = p.Cout >> 5;                       // 32-column chunks per output row
         const float lower = p.relu ? 0.f : -INFINITY;
         const long pl_plane = (long)p.H * p.W;
+        constexpr bool PLANAR = MODE == 2 || MODE == 3;
+        constexpr int NPL = MODE == 3 ? 1 : 3;                // planes per frame of the planar output
         constexpr int PIN_ROWS = (8 + EPI_WG - 1) / EPI_WG;   // planar mode: rows of a super-tile (R <= 8) per warpgroup
         const uint32_t tile_b = (uint32_t)p.rb_out * 32u;      // staging tile of a warp: 32 pixel rows of the stored output
         const uint32_t sbuf0 = stage_out_base + (uint32_t)((g * 4 + q) * p.out_bufs) * tile_b;
@@ -802,22 +804,22 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     for (int j = 0; j < 8; ++j) rr[j] = __ldg(rp + j);
                 }
             }
-            if (MODE == 2) {
+            if (PLANAR) {
 #pragma unroll
                 for (int i = 0; i < PIN_ROWS; ++i) {
                     const int t = g + i * EPI_WG;
 #pragma unroll
                     for (int c = 0; c < 3; ++c) pin[i][c] = 0.f;
                     if (valid && t < rows) {
-                        const long o = (long)n * 3 * pl_plane + (long)(y0 + t) * p.W + wo;
+                        const long o = (long)n * NPL * pl_plane + (long)(y0 + t) * p.W + wo;
 #pragma unroll
-                        for (int c = 0; c < 3; ++c) pin[i][c] = __ldg(p.planar_in1 + o + c * pl_plane);
+                        for (int c = 0; c < NPL; ++c) pin[i][c] = __ldg(p.planar_in1 + o + c * pl_plane);
                     }
                 }
             }
             mbar_wait(&tfull_bar[acc], acc_phase);
             tc_fence_after();
-            if (HALF && MODE != 2) {
+            if (HALF && !PLANAR) {
                 // ---- fp16 output: unit = `ucols` accumulator columns -> one 64-channel (128-byte) pixel row
                 const int nun = (p.Cout + p.ucols - 1) / p.ucols;
                 const int hunits = rows * nun;
@@ -942,8 +944,8 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     v[j + 3] = fmaxf(fmaf(v[j + 3], sc.w, sh.w), lower);
                 }
             };
-            if (MODE == 2) {
-                // last conv of a FastDVDnet DenBlock: the 3 real channels leave as planar frames, residual form
+            if (PLANAR) {
+                // last conv of a FastDVDnet DenBlock: the NPL real channels leave as planar frames, residual form
                 // in1 - net (models.py:196) applied here; lanes are consecutive pixels -> coalesced plane accesses
 #pragma unroll
                 for (int i = 0; i < PIN_ROWS; ++i) {
@@ -952,9 +954,9 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                         float v[32];
                         unit(t, 0, v);
                         if (valid) {
-                            const long o = (long)n * 3 * pl_plane + (long)(y0 + t) * p.W + wo;
+                            const long o = (long)n * NPL * pl_plane + (long)(y0 + t) * p.W + wo;
 #pragma unroll
-                            for (int c = 0; c < 3; ++c) p.planar_out[o + c * pl_plane] = pin[i][c] - v[c];
+                            for (int c = 0; c < NPL; ++c) p.planar_out[o + c * pl_plane] = pin[i][c] - v[c];
                         }
                     }
                 }
@@ -1342,7 +1344,7 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
         p.ucols = 32;
         p.ks_last = 4;
     }
-    int mode = p.planar_out ? 2 : (d->residual ? 1 : 0);
+    int mode = p.planar_out ? (d->planar_planes == 1 ? 3 : 2) : (d->residual ? 1 : 0);
     p.mask_y = d->mask_y; p.col_s1 = d->col_s1; p.col_s2 = d->col_s2; p.mask_relu = d->mask_relu;
     if (d->mask_y) {
         if (half || p.planar_out || (d->pixel_shuffle ? d->Cout / 4 : d->Cout) > 128 || (d->col_s2 && !d->col_s1))
@@ -1434,14 +1436,16 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     const size_t smem = (size_t)(p.resident ? w_bytes : 0) + (size_t)p.stages * stage_bytes + out_stage + 1024;
     if (smem > 220 * 1024) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: shared memory budget exceeded");
     typedef void (*Fwd2Kernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const Fwd2Params);
-    // indexed by MODE (there is no MODE 3; MODE 4 exists for fp32 only)
+    // indexed by MODE (MODE 4 exists for fp32 only)
     static const Fwd2Kernel kernels[2][2][5] = {
-        {{conv_fwd2_tc_kernel<1, 0, false>, conv_fwd2_tc_kernel<1, 1, false>, conv_fwd2_tc_kernel<1, 2, false>, nullptr,
-          conv_fwd2_tc_kernel<1, 4, false>},
-         {conv_fwd2_tc_kernel<2, 0, false>, conv_fwd2_tc_kernel<2, 1, false>, conv_fwd2_tc_kernel<2, 2, false>, nullptr,
-          conv_fwd2_tc_kernel<2, 4, false>}},
-        {{conv_fwd2_tc_kernel<1, 0, true>, conv_fwd2_tc_kernel<1, 1, true>, conv_fwd2_tc_kernel<1, 2, true>, nullptr, nullptr},
-         {conv_fwd2_tc_kernel<2, 0, true>, conv_fwd2_tc_kernel<2, 1, true>, conv_fwd2_tc_kernel<2, 2, true>, nullptr, nullptr}}};
+        {{conv_fwd2_tc_kernel<1, 0, false>, conv_fwd2_tc_kernel<1, 1, false>, conv_fwd2_tc_kernel<1, 2, false>,
+          conv_fwd2_tc_kernel<1, 3, false>, conv_fwd2_tc_kernel<1, 4, false>},
+         {conv_fwd2_tc_kernel<2, 0, false>, conv_fwd2_tc_kernel<2, 1, false>, conv_fwd2_tc_kernel<2, 2, false>,
+          conv_fwd2_tc_kernel<2, 3, false>, conv_fwd2_tc_kernel<2, 4, false>}},
+        {{conv_fwd2_tc_kernel<1, 0, true>, conv_fwd2_tc_kernel<1, 1, true>, conv_fwd2_tc_kernel<1, 2, true>,
+          conv_fwd2_tc_kernel<1, 3, true>, nullptr},
+         {conv_fwd2_tc_kernel<2, 0, true>, conv_fwd2_tc_kernel<2, 1, true>, conv_fwd2_tc_kernel<2, 2, true>,
+          conv_fwd2_tc_kernel<2, 3, true>, nullptr}}};
     const Fwd2Kernel kern = kernels[half ? 1 : 0][epi_wg - 1][mode];
     if (!kern) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: epilogue not built");
     const int grid = min(p.num_tiles, SCI_NUM_SMS);
@@ -1839,6 +1843,7 @@ int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream) {
 int check_conv_desc(const sci_conv_desc* d) {
     SCI_REQUIRE(d && d->x && d->w && (d->y || d->planar_out), "conv: null pointer");
     SCI_REQUIRE(!d->planar_out || (d->stride == 1 && !d->w_split && !d->emit_lo), "conv: planar output options");
+    SCI_REQUIRE(d->planar_planes == 0 || d->planar_planes == 1 || d->planar_planes == 3, "conv: planar_planes 0, 1 or 3");
     SCI_REQUIRE(d->N > 0 && d->H > 0 && d->W > 0 && d->Cin > 0 && d->Cout > 0, "conv: shape");
     SCI_REQUIRE(d->Cin % 8 == 0 && d->Cout % 4 == 0, "conv: Cin % 8, Cout % 4");
     SCI_REQUIRE(!d->half_io || ((d->Cin % 64 == 0 || d->Cin == 32) && d->Cout % 32 == 0 && !d->emit_lo), "conv fp16: Cin % 64 (or 32), Cout % 32, no emit_lo");

@@ -276,7 +276,10 @@ __global__ void ffdnet_unpack_grad_kernel(const float* __restrict__ dxhat, float
 // ---- FastDVDnet boundary --------------------------------------------------------------------------
 // One thread builds the 32-channel row of one pixel (9 coalesced plane reads), the block transposes it through
 // shared memory so that the NHWC write is fully coalesced.
+// NC = planes per frame of the planar frames: 3 (colour) or 1 (gray, written as the first plane of the colour layout:
+// the other two channels of each slot are +0, exactly what packing the zero-embedded cube gives).
 constexpr int FPACK_PIX = 256;
+template <int NC>
 __global__ void __launch_bounds__(FPACK_PIX) fastdvd_pack_kernel(const float* __restrict__ frames, float sigma,
                                                                    float* __restrict__ out, int B, int H, int W, int Cpad,
                                                                    int round_tf32) {
@@ -294,7 +297,7 @@ __global__ void __launch_bounds__(FPACK_PIX) fastdvd_pack_kernel(const float* __
             const int src = (f + slot - 1 + B) % B;                              // circular window (fastdvdnet.py:115)
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                const float v = (c == 3) ? sigma : frames[((long)src * 3 + c) * plane + p];
+                const float v = (c == 3) ? sigma : (c < NC ? frames[((long)src * NC + c) * plane + p] : 0.f);
                 if (round_tf32) {        // channel k: tf32(v); channel k+16: remainder (weights duplicated)
                     const float hi = rna_tf32(v);
                     row[slot * 4 + c] = hi;
@@ -311,15 +314,16 @@ __global__ void __launch_bounds__(FPACK_PIX) fastdvd_pack_kernel(const float* __
     for (int i = threadIdx.x; i < npx * Cpad; i += FPACK_PIX) dst[i] = srow[(i / Cpad) * CS + (i % Cpad)];
 }
 
+template <int NC>
 __global__ void fastdvd_pack_grad_kernel(const float* __restrict__ din, float* __restrict__ dframes, int B, int H, int W,
                                          int Cpad, int accumulate) {
-    // dframes[j][c][p] (+)= sum_{slot} din[(j - slot + 1) mod B][p][slot*4 + c]
+    // dframes[j][c][p] (+)= sum_{slot} din[(j - slot + 1) mod B][p][slot*4 + c], c < NC
     const long plane = (long)H * W;
-    const long total = (long)B * 3 * plane;
+    const long total = (long)B * NC * plane;
     const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= total) return;
     const long p = idx % plane;
-    const int c = (int)((idx / plane) % 3), j = (int)(idx / (3 * plane));
+    const int c = (int)((idx / plane) % NC), j = (int)(idx / (NC * plane));
     float v = accumulate ? dframes[idx] : 0.f;
 #pragma unroll
     for (int slot = 0; slot < 3; ++slot) {
@@ -329,19 +333,21 @@ __global__ void fastdvd_pack_grad_kernel(const float* __restrict__ din, float* _
     dframes[idx] = v;
 }
 
+template <int NC>
 __global__ void fastdvd_output_kernel(const float* __restrict__ frames, const float* __restrict__ y, float* __restrict__ out,
                                       int B, int H, int W, int Cpad) {
     const long plane = (long)H * W;
-    const long total = (long)B * 3 * plane;
+    const long total = (long)B * NC * plane;
     const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= total) return;
     const long p = idx % plane;
-    const int c = (int)((idx / plane) % 3), f = (int)(idx / (3 * plane));
+    const int c = (int)((idx / plane) % NC), f = (int)(idx / (NC * plane));
     out[idx] = frames[idx] - __ldg(y + ((long)f * plane + p) * Cpad + c);    // models.py:196
 }
 
-// dy[f][p][c] = -dout[f][c][p] for c < 3, 0 for the padded columns.  One thread reads the three plane values of its pixel
+// dy[f][p][c] = -dout[f][c][p] for c < NC, 0 for the padded columns.  One thread reads the NC plane values of its pixel
 // (coalesced), the block writes the [256 px][Cpad] rows through shared memory (fully coalesced NHWC write).
+template <int NC>
 __global__ void __launch_bounds__(FPACK_PIX) fastdvd_output_grad_kernel(const float* __restrict__ dout, float* __restrict__ dy,
                                                                           int H, int W, int Cpad) {
     extern __shared__ float srow[];                   // [FPACK_PIX][Cpad + 1]
@@ -353,7 +359,10 @@ __global__ void __launch_bounds__(FPACK_PIX) fastdvd_output_grad_kernel(const fl
     for (int k = 0; k < Cpad; ++k) row[k] = 0.f;
     if (p < plane) {
 #pragma unroll
-        for (int c = 0; c < 3; ++c) row[c] = -dout[((long)f * 3 + c) * plane + p];
+        for (int c = 0; c < NC; ++c) row[c] = -dout[((long)f * NC + c) * plane + p];
+        // gray frames: what the colour kernel writes for the zero planes of the embedded cube, -(+0), so that the backward
+        // pass of a gray sequence is bit for bit that of its embedding
+        if (NC == 1) row[1] = row[2] = -0.f;
     }
     __syncthreads();
     const int npx = (int)min((long)FPACK_PIX, plane - p0);
@@ -447,8 +456,9 @@ __device__ __forceinline__ uint4 pack8(const __half* v) {
     auto pk = [](__half a, __half b) -> uint32_t { return (uint32_t)__half_as_ushort(a) | ((uint32_t)__half_as_ushort(b) << 16); };
     return make_uint4(pk(v[0], v[1]), pk(v[2], v[3]), pk(v[4], v[5]), pk(v[6], v[7]));
 }
-// NCH = 16-byte chunks per pixel row: 8 (64 channels, the upper 36 zero) or 4 (32 channels = 64-byte rows)
-template <int NCH>
+// NCH = 16-byte chunks per pixel row: 8 (64 channels, the upper 36 zero) or 4 (32 channels = 64-byte rows); NC = planes per
+// frame as in fastdvd_pack_kernel
+template <int NCH, int NC>
 __global__ void __launch_bounds__(256) fastdvd_pack_half_kernel(const float* __restrict__ frames, float sigma,
                                                                 __half* __restrict__ out, int B, int H, int W) {
     __shared__ uint4 tile[8][32 * NCH];               // per warp: 32 pixels x NCH chunks of 16 bytes, XOR-swizzled
@@ -466,7 +476,7 @@ __global__ void __launch_bounds__(256) fastdvd_pack_half_kernel(const float* __r
             const int src = (f + slot - 1 + B) % B;                          // circular window (fastdvdnet.py:115)
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                const float v = (c == 3) ? sigma : __ldg(frames + ((long)src * 3 + c) * plane + p);
+                const float v = (c == 3) ? sigma : (c < NC ? __ldg(frames + ((long)src * NC + c) * plane + p) : 0.f);
                 const __half h = __float2half_rn(v);
                 hi[slot * 4 + c] = h;
                 lo[slot * 4 + c] = __float2half_rn(v - __half2float(h));
@@ -645,13 +655,25 @@ extern "C" int sci_conv_pack_weights_half(const float* w, void* packed, int Co, 
     return SCI_OK;
 }
 
-extern "C" int sci_fastdvd_pack_input_half(const float* frames, float sigma, void* out, int B, int H, int W, int C, void* stream) {
-    SCI_REQUIRE(frames && out && B > 0 && H > 0 && W > 0 && B <= 65535 && (C == 32 || C == 64), "fastdvd_pack_input_half");
+extern "C" int sci_fastdvd_pack_input_half_planes(const float* frames, float sigma, void* out, int B, int NC, int H, int W, int C,
+                                                  void* stream) {
+    SCI_REQUIRE(frames && out && B > 0 && H > 0 && W > 0 && B <= 65535 && (C == 32 || C == 64) && (NC == 1 || NC == 3),
+                "fastdvd_pack_input_half");
     const dim3 grid(grid1d((long)H * W, 256), B);
-    if (C == 64) fastdvd_pack_half_kernel<8><<<grid, 256, 0, sci_stream(stream)>>>(frames, sigma, reinterpret_cast<__half*>(out), B, H, W);
-    else         fastdvd_pack_half_kernel<4><<<grid, 256, 0, sci_stream(stream)>>>(frames, sigma, reinterpret_cast<__half*>(out), B, H, W);
+    __half* o = reinterpret_cast<__half*>(out);
+    if (NC == 3) {
+        if (C == 64) fastdvd_pack_half_kernel<8, 3><<<grid, 256, 0, sci_stream(stream)>>>(frames, sigma, o, B, H, W);
+        else         fastdvd_pack_half_kernel<4, 3><<<grid, 256, 0, sci_stream(stream)>>>(frames, sigma, o, B, H, W);
+    } else {
+        if (C == 64) fastdvd_pack_half_kernel<8, 1><<<grid, 256, 0, sci_stream(stream)>>>(frames, sigma, o, B, H, W);
+        else         fastdvd_pack_half_kernel<4, 1><<<grid, 256, 0, sci_stream(stream)>>>(frames, sigma, o, B, H, W);
+    }
     SCI_CHECK_LAUNCH("fastdvd_pack_input_half");
     return SCI_OK;
+}
+
+extern "C" int sci_fastdvd_pack_input_half(const float* frames, float sigma, void* out, int B, int H, int W, int C, void* stream) {
+    return sci_fastdvd_pack_input_half_planes(frames, sigma, out, B, 3, H, W, C, stream);
 }
 
 extern "C" int sci_conv_pack_weights_s2t(const float* w, float* packed, int Co, int Ci, int Co_pad, int Ci_pad,
@@ -764,48 +786,76 @@ extern "C" int sci_ffdnet_unpack_output_grad(const float* dxhat, float* dy, int 
     return SCI_OK;
 }
 
-extern "C" int sci_fastdvd_pack_input(const float* frames, float sigma, float* out, int B, int H, int W, int Cpad,
-                                      int round_tf32, void* stream) {
-    SCI_REQUIRE(frames && out && B > 0 && H > 0 && W > 0 && Cpad >= (round_tf32 ? 32 : 12), "fastdvd_pack_input");
+extern "C" int sci_fastdvd_pack_input_planes(const float* frames, float sigma, float* out, int B, int NC, int H, int W, int Cpad,
+                                             int round_tf32, void* stream) {
+    SCI_REQUIRE(frames && out && B > 0 && H > 0 && W > 0 && Cpad >= (round_tf32 ? 32 : 12) && (NC == 1 || NC == 3),
+                "fastdvd_pack_input");
     SCI_REQUIRE(Cpad <= 48 && B <= 65535, "fastdvd_pack_input: Cpad <= 48");
     const size_t smem = (size_t)FPACK_PIX * (Cpad + 1) * sizeof(float);
     // the largest Cpad admitted above, so that the once-per-device limit covers every later call
-    const cudaError_t e = sci_smem_limit((const void*)fastdvd_pack_kernel, FPACK_PIX * (48 + 1) * (int)sizeof(float));
+    const void* kern = NC == 3 ? (const void*)fastdvd_pack_kernel<3> : (const void*)fastdvd_pack_kernel<1>;
+    const cudaError_t e = sci_smem_limit(kern, FPACK_PIX * (48 + 1) * (int)sizeof(float));
     if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "fastdvd_pack_input: shared-memory limit", e);
-    fastdvd_pack_kernel<<<dim3(grid1d((long)H * W, FPACK_PIX), B), FPACK_PIX, smem, sci_stream(stream)>>>(frames, sigma, out, B,
-                                                                                                      H, W, Cpad, round_tf32);
+    const dim3 grid(grid1d((long)H * W, FPACK_PIX), B);
+    if (NC == 3) fastdvd_pack_kernel<3><<<grid, FPACK_PIX, smem, sci_stream(stream)>>>(frames, sigma, out, B, H, W, Cpad, round_tf32);
+    else         fastdvd_pack_kernel<1><<<grid, FPACK_PIX, smem, sci_stream(stream)>>>(frames, sigma, out, B, H, W, Cpad, round_tf32);
     SCI_CHECK_LAUNCH("fastdvd_pack_input");
+    return SCI_OK;
+}
+
+extern "C" int sci_fastdvd_pack_input(const float* frames, float sigma, float* out, int B, int H, int W, int Cpad,
+                                      int round_tf32, void* stream) {
+    return sci_fastdvd_pack_input_planes(frames, sigma, out, B, 3, H, W, Cpad, round_tf32, stream);
+}
+
+extern "C" int sci_fastdvd_pack_input_grad_planes(const float* din, float* dframes, int B, int NC, int H, int W, int Cpad,
+                                                  int accumulate, void* stream) {
+    SCI_REQUIRE(din && dframes && B > 0 && H > 0 && W > 0 && Cpad >= 12 && (NC == 1 || NC == 3), "fastdvd_pack_input_grad");
+    const int grid = grid1d((long)B * NC * H * W);
+    if (NC == 3) fastdvd_pack_grad_kernel<3><<<grid, 256, 0, sci_stream(stream)>>>(din, dframes, B, H, W, Cpad, accumulate);
+    else         fastdvd_pack_grad_kernel<1><<<grid, 256, 0, sci_stream(stream)>>>(din, dframes, B, H, W, Cpad, accumulate);
+    SCI_CHECK_LAUNCH("fastdvd_pack_input_grad");
     return SCI_OK;
 }
 
 extern "C" int sci_fastdvd_pack_input_grad(const float* din, float* dframes, int B, int H, int W, int Cpad, int accumulate,
                                            void* stream) {
-    SCI_REQUIRE(din && dframes && B > 0 && H > 0 && W > 0 && Cpad >= 12, "fastdvd_pack_input_grad");
-    fastdvd_pack_grad_kernel<<<grid1d((long)B * 3 * H * W), 256, 0, sci_stream(stream)>>>(din, dframes, B, H, W, Cpad,
-                                                                                        accumulate);
-    SCI_CHECK_LAUNCH("fastdvd_pack_input_grad");
+    return sci_fastdvd_pack_input_grad_planes(din, dframes, B, 3, H, W, Cpad, accumulate, stream);
+}
+
+extern "C" int sci_fastdvd_output_planes(const float* frames, const float* y, float* out, int B, int NC, int H, int W, int Cpad,
+                                         void* stream) {
+    SCI_REQUIRE(frames && y && out && B > 0 && H > 0 && W > 0 && (NC == 1 || NC == 3) && Cpad >= NC, "fastdvd_output");
+    const int grid = grid1d((long)B * NC * H * W);
+    if (NC == 3) fastdvd_output_kernel<3><<<grid, 256, 0, sci_stream(stream)>>>(frames, y, out, B, H, W, Cpad);
+    else         fastdvd_output_kernel<1><<<grid, 256, 0, sci_stream(stream)>>>(frames, y, out, B, H, W, Cpad);
+    SCI_CHECK_LAUNCH("fastdvd_output");
     return SCI_OK;
 }
 
 extern "C" int sci_fastdvd_output(const float* frames, const float* y, float* out, int B, int H, int W, int Cpad,
                                   void* stream) {
-    SCI_REQUIRE(frames && y && out && B > 0 && H > 0 && W > 0 && Cpad >= 3, "fastdvd_output");
-    fastdvd_output_kernel<<<grid1d((long)B * 3 * H * W), 256, 0, sci_stream(stream)>>>(frames, y, out, B, H, W, Cpad);
-    SCI_CHECK_LAUNCH("fastdvd_output");
+    return sci_fastdvd_output_planes(frames, y, out, B, 3, H, W, Cpad, stream);
+}
+
+extern "C" int sci_fastdvd_output_grad_planes(const float* dout, float* dy, int B, int NC, int H, int W, int Cpad, void* stream) {
+    SCI_REQUIRE(dout && dy && B > 0 && H > 0 && W > 0 && (NC == 1 || NC == 3) && Cpad >= NC, "fastdvd_output_grad");
+    SCI_REQUIRE(Cpad <= 64, "fastdvd_output_grad: Cpad");
+    // 256 * (Cpad + 1) floats pass the 48 KB default from Cpad 48 on; raise the limit to what Cpad 64 needs
+    const void* kern = NC == 3 ? (const void*)fastdvd_output_grad_kernel<3> : (const void*)fastdvd_output_grad_kernel<1>;
+    const cudaError_t e = sci_smem_limit(kern, FPACK_PIX * (64 + 1) * (int)sizeof(float));
+    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "fastdvd_output_grad: shared-memory limit", e);
+    const long plane = (long)H * W;
+    const dim3 grid(grid1d(plane, FPACK_PIX), B);
+    const size_t smem = (size_t)FPACK_PIX * (Cpad + 1) * sizeof(float);
+    if (NC == 3) fastdvd_output_grad_kernel<3><<<grid, FPACK_PIX, smem, sci_stream(stream)>>>(dout, dy, H, W, Cpad);
+    else         fastdvd_output_grad_kernel<1><<<grid, FPACK_PIX, smem, sci_stream(stream)>>>(dout, dy, H, W, Cpad);
+    SCI_CHECK_LAUNCH("fastdvd_output_grad");
     return SCI_OK;
 }
 
 extern "C" int sci_fastdvd_output_grad(const float* dout, float* dy, int B, int H, int W, int Cpad, void* stream) {
-    SCI_REQUIRE(dout && dy && B > 0 && H > 0 && W > 0 && Cpad >= 3, "fastdvd_output_grad");
-    SCI_REQUIRE(Cpad <= 64, "fastdvd_output_grad: Cpad");
-    // 256 * (Cpad + 1) floats pass the 48 KB default from Cpad 48 on; raise the limit to what Cpad 64 needs
-    const cudaError_t e = sci_smem_limit((const void*)fastdvd_output_grad_kernel, FPACK_PIX * (64 + 1) * (int)sizeof(float));
-    if (e != cudaSuccess) return sci_fail(SCI_ELAUNCH, "fastdvd_output_grad: shared-memory limit", e);
-    const long plane = (long)H * W;
-    fastdvd_output_grad_kernel<<<dim3(grid1d(plane, FPACK_PIX), B), FPACK_PIX, (size_t)FPACK_PIX * (Cpad + 1) * sizeof(float),
-                                 sci_stream(stream)>>>(dout, dy, H, W, Cpad);
-    SCI_CHECK_LAUNCH("fastdvd_output_grad");
-    return SCI_OK;
+    return sci_fastdvd_output_grad_planes(dout, dy, B, 3, H, W, Cpad, stream);
 }
 
 extern "C" int sci_fastdvd_noisy_input(const float* v, const double* noise, float* vplus, long n, void* stream) {

@@ -446,23 +446,37 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
 
 def twoStageAdmm_denoise_gray(y, Phi, denoiser='ffdnet_gray', iter_max=50, sigma=None, x0=None, X_orig=None,
                               model_denoise=None, show_iqa=True, lr_=0.000001, inital_iter=1, interval_iter=5, logf=None,
-                              update_=False, update_per_iter=1, noise_estimate=False, grad_sync=None):
-    """BASELINE config 2: two-stage ADMM + online FFDNet-gray on a GRAYSCALE cube.
+                              update_=False, update_per_iter=1, noise_estimate=False, grad_sync=None, update_times=-1):
+    """Two-stage ADMM with an online-adapted deep denoiser on a GRAYSCALE cube: 'ffdnet_gray' (BASELINE config 2) or
+    'fastdvd_gray' (the grayscale video SCI case of adaptive PnP with FastDVDnet, ``fastdvdnet_models.FastDVDnet`` with
+    ``num_color_channels=1``).
 
-    The reference has no function for this configuration (``twoStageAdmm_denoise_bayer`` only knows 'tv', 'ffdnet_color'
-    and 'fastdvd_color', dvp...online.py:147,164,214,262; the gray network is only constructed by the script's ``else``
+    The reference has no function for either (``twoStageAdmm_denoise_bayer`` only knows 'tv', 'ffdnet_color' and
+    'fastdvd_color', dvp...online.py:147,164,214,262; the gray network is only constructed by the script's ``else``
     branch, two_stage_ADMM_Online_FFD_Warm.py:37-40).  Following SURVEY §8(c) this is the SAME loop with the Bayer split /
-    demosaic replaced by the identity (alpha = 1, rho = 1, tau = 100, k = 0 aliasing included); parity is checked against the
-    derived oracle ``oracle.admm.twoStageAdmm_denoise_gray`` and reported as "parity vs derived oracle".
+    demosaic replaced by the identity and every constant the colour branch uses for the same denoiser: tau = 100, k = 0
+    aliasing included, alpha = 1 and rho = 1 for 'ffdnet_gray', rho = 0.55 for 'fastdvd_gray' (dvp:101-109), whose
+    fine-tune is ``fastdvdnet_denoiser_full_tensor_v2`` with one plane (noise (B,1,H,W) from the global numpy RNG, loss
+    MSE(sum_t xhat_t Phi_t, y)) and is limited by ``update_times`` (dvp:247; 'ffdnet_gray' ignores it).  Parity is checked
+    against the derived oracles (``oracle.admm.twoStageAdmm_denoise_gray`` for 'ffdnet_gray',
+    ``oracle.gray_fastdvd.twoStageAdmm_denoise_gray`` for 'fastdvd_gray') and reported as "parity vs derived oracle".
+    'fastdvd_gray' needs H and W multiples of 4 (ValueError before any GPU work).
 
     y [H,W], Phi [H,W,B], x0 [H,W,B] (warm start) -> (xhat_np[H,W,B], theta_np[H,W,B], psnr_, ssim_, psnr_all, model)."""
-    if denoiser != 'ffdnet_gray':
+    name = str(denoiser).lower()
+    if name not in ('ffdnet_gray', 'fastdvd_gray'):
         raise ValueError('Unsupported denoiser {}!'.format(denoiser))
-    from . import ffdnet_adapter
+    if name == 'fastdvd_gray' and (y.shape[0] % 4 or y.shape[1] % 4):
+        raise ValueError("'fastdvd_gray' needs H and W multiples of 4 (the native FastDVDnet engine), got %d x %d"
+                         % (y.shape[0], y.shape[1]))
+    from . import fastdvdnet_adapter, ffdnet_adapter
+    adapter = ffdnet_adapter if name == 'ffdnet_gray' else fastdvdnet_adapter
     sigma, iter_max = _as_list(sigma, iter_max)
     pb = _Problem(y, Phi, x0, X_orig)
     dev = pb.y.device
     H, W, B = pb.H, pb.W, pb.B
+    rou = 0.55 if name == 'fastdvd_gray' else 1                                       # dvp:106-109
+    inv_rou = float(np.float32(1 / rou))
     tau = 100
     n_total = int(sum(iter_max))
     want_iqa = bool(show_iqa and X_orig is not None)
@@ -471,15 +485,19 @@ def twoStageAdmm_denoise_gray(y, Phi, denoiser='ffdnet_gray', iter_max=50, sigma
     w = torch.zeros((B, 1, H, W), dtype=torch.float32, device=dev)
     x_pre = torch.empty((B, H, W), dtype=torch.float32, device=dev)
     u = torch.empty((B, 1, H, W), dtype=torch.float32, device=dev)
-    sched, k, xhat = [], 0, None
+    if name == 'fastdvd_gray' and update_:
+        fastdvdnet_adapter.noise_stream.prefetch((B, 1, H, W))                        # see twoStageAdmm_denoise_bayer
+    sched, k, xhat, update_i = [], 0, None, 0
     for idx, nsig in enumerate(sigma):
         for _ in range(iter_max[idx]):
-            ops.project_stage2(theta, b, pb.phi, pb.y, pb.phisum, x, 1, 1)                # alpha = rho = 1
-            ops.axpy(x, 1.0, b, out=x_pre)                                                # x + b/rho
+            ops.project_stage2(theta, b, pb.phi, pb.y, pb.phisum, x, 1, rou)              # alpha = 1
+            ops.axpy(x, inv_rou, b, out=x_pre)                                            # x + b/rho
             ops.axpy(x_pre.view(B, 1, H, W), -float(np.float32(1 / tau)), w, out=u)       # - w/tau
             do_update = bool(update_ and k > inital_iter and k % interval_iter == 0)
-            xhat = ffdnet_adapter.denoise_planar(u, pb, nsig, model_denoise, lr_, do_update, update_per_iter,
-                                                 grad_sync=grad_sync)
+            if name == 'fastdvd_gray':
+                do_update = do_update and (update_i < update_times or update_times < 0)   # dvp:247
+                update_i += int(do_update)
+            xhat = adapter.denoise_planar(u, pb, nsig, model_denoise, lr_, do_update, update_per_iter, grad_sync=grad_sync)
             _lib_call("sci_dual_update_gray", xhat, x_pre, w, x, b, theta, k == 0, pb.orig if want_iqa else None,
                       sse[k:k + 1] if want_iqa else None)
             sched.append(nsig)

@@ -37,7 +37,7 @@ class ConvDesc(ctypes.Structure):
                 ("planar_in1", _f32p), ("planar_out", _f32p), ("pdl", ctypes.c_int),
                 ("half_io", ctypes.c_int), ("Cin_store", ctypes.c_int), ("Cout_store", ctypes.c_int),
                 ("mask_y", _f32p), ("col_s1", _f32p), ("col_s2", _f32p), ("mask_relu", ctypes.c_int), ("lo_channel0", ctypes.c_int),
-                ("K_used", ctypes.c_int)]
+                ("K_used", ctypes.c_int), ("planar_planes", ctypes.c_int)]
 
 
 class WgradDesc(ctypes.Structure):
@@ -353,13 +353,16 @@ class _EngineBase:
 
     # ---- kernel wrappers ------------------------------------------------------------------------------
     def conv(self, L, x, N, H, W, y, residual=None, round_out=True, emit_lo=False, planar=None):
-        """planar = (in1, out) planar [N,3,H,W] tensors: tensor-core path only, fused `out = in1 - conv` (y unused)."""
+        """planar = (in1, out) planar [N,P,H,W] tensors (P = 3, or 1 for gray frames): tensor-core path only, fused
+        `out = in1 - conv` (y unused)."""
         d = ConvDesc(_dp(x), _dp(L.wpk), _dp(L.scale), _dp(L.shift), _dp(residual), _dp(y), N, H, W, L.Ci_pad, L.Co_pad,
                      L.stride, int(L.relu), int(L.ps), int(self.tf32 and round_out), int(self.tf32 and L.wsplit),
                      int(emit_lo), _dp(planar[0]) if planar else None, _dp(planar[1]) if planar else None,
                      int(self.pdl_chain))
         if L.dup_in and self.tf32 and L.wsplit:
             d.lo_channel0 = L.ci_half                # "3xTF32": the remainder half of the input starts here (split accumulators)
+        if planar:
+            d.planar_planes = planar[0].shape[1]
         if self.profile is not None:
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             ev0.record()
@@ -378,6 +381,8 @@ class _EngineBase:
                      Lh.stride, int(Lh.relu), int(Lh.ps), 0, int(Lh.split), 0, _dp(planar[0]) if planar else None,
                      _dp(planar[1]) if planar else None, int(self.pdl_chain), 1, Lh.cin_store, Lh.cout_store)
         d.K_used = Lh.k_used                         # zero-padded channels of the last 64-channel chunk are not multiplied
+        if planar:
+            d.planar_planes = planar[0].shape[1]
         if self.profile is not None:
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             ev0.record()
@@ -598,14 +603,14 @@ class FastDVDnetEngine(_EngineBase):
 
     def _block_forward_h(self, Lh, frames, sigma, out):
         """One DenBlock on the fp16 kernels (inference): planar fp32 frames in, planar fp32 ``frames - net`` out."""
-        B, _, H, W = frames.shape
+        B, C, H, W = frames.shape
         dev = frames.device
         f16 = torch.float16
         g = lambda n, shape: self.ws.get("h_" + n, shape, dev, dtype=f16)
         h2, w2, h4, w4 = H // 2, W // 2, H // 4, W // 4
         c32 = Lh[0].cin_store                # 32 (64-byte pixel rows) or 64: channels per pixel of the 32-channel tensors
         a_in = g("in", (B, H, W, c32))
-        call("sci_fastdvd_pack_input_half", ptr(frames), float(sigma), ptr(a_in), B, H, W, c32, stream())
+        call("sci_fastdvd_pack_input_half_planes", ptr(frames), float(sigma), ptr(a_in), B, C, H, W, c32, stream())
         a0 = g("a0", (B, H, W, 96));        self.conv_h(Lh[0], a_in, B, H, W, a0)
         x0 = g("x0", (B, H, W, c32));       self.conv_h(Lh[1], a0, B, H, W, x0)
         d0a = g("d0a", (B, h2, w2, 64));    self.conv_h(Lh[2], x0, B, H, W, d0a)
@@ -627,14 +632,15 @@ class FastDVDnetEngine(_EngineBase):
 
     # ---- one DenBlock ---------------------------------------------------------------------------------
     def _block_forward(self, tag, blk, frames, sigma, out, train):
-        B, _, H, W = frames.shape
+        B, C, H, W = frames.shape
         dev = frames.device
         L = blk.L
         g = self.ws.get
         keep = (lambda n: "%s_%s" % (tag, n)) if train else (lambda n: "inf_" + n)
         h2, w2, h4, w4 = H // 2, W // 2, H // 4, W // 4
         a_in = g(keep("in"), (B, H, W, L[0].Ci_pad), dev)
-        call("sci_fastdvd_pack_input", ptr(frames), float(sigma), ptr(a_in), B, H, W, L[0].Ci_pad, int(self.tf32), stream())
+        call("sci_fastdvd_pack_input_planes", ptr(frames), float(sigma), ptr(a_in), B, C, H, W, L[0].Ci_pad, int(self.tf32),
+             stream())
         a0 = g(keep("a0"), (B, H, W, L[0].Co_pad), dev);   self.conv(L[0], a_in, B, H, W, a0)
         x0 = g(keep("x0"), (B, H, W, L[1].Co_pad), dev);   self.conv(L[1], a0, B, H, W, x0)
         d0a = g(keep("d0a"), (B, h2, w2, 64), dev);        self.conv(L[2], x0, B, H, W, d0a)
@@ -660,22 +666,26 @@ class FastDVDnetEngine(_EngineBase):
             self.conv(L[15], o0, B, H, W, None, round_out=False, planar=(frames, out))
         else:
             xo = g(keep("xo"), (B, H, W, L[15].Co_pad), dev);  self.conv(L[15], o0, B, H, W, xo, round_out=False)
-            call("sci_fastdvd_output", ptr(frames), ptr(xo), ptr(out), B, H, W, L[15].Co_pad, stream())
+            call("sci_fastdvd_output_planes", ptr(frames), ptr(xo), ptr(out), B, C, H, W, L[15].Co_pad, stream())
         if train:
             return dict(a_in=a_in, a0=a0, x0=x0, d0a=d0a, d0b=d0b, x1=x1, d1a=d1a, d1b=d1b, x2=x2, u2a=u2a, u2b=u2b,
                         s1=s1, u1a=u1a, u1b=u1b, s0=s0, o0=o0, xo=xo)
         return None
 
     def forward(self, frames, sigma, train=False):
-        """frames [B,3,H,W] planar -> denoised [B,3,H,W] (whole circular sequence)."""
-        B, _, H, W = frames.shape
+        """frames [B,C,H,W] planar -> denoised [B,C,H,W] (whole circular sequence).  C = 3, or C = 1: gray frames on the
+        colour-shaped embedding of the gray model (fastdvdnet_models.FastDVDnet), which the boundary kernels pack as the
+        first plane of a colour cube whose other planes are zero, and of whose output only the first plane is computed."""
+        B, C, H, W = frames.shape
+        if C not in (1, 3):
+            raise _lib.SciError("native FastDVDnet engine: frames with 3 (colour) or 1 (gray) planes, got %d" % C)
         if H % 4 or W % 4:
             raise NotImplementedError("native FastDVDnet engine needs H, W multiples of 4 (the reference reflect-pads, "
                                       "fastdvdnet.py:119-127; the hot-path sizes never need it)")
         self.prepare(training=train)
         dev = frames.device
-        t1_out = self.ws.get("t1_out_train" if train else "t1_out", (B, 3, H, W), dev)
-        out = self.ws.get("out_train" if train else "out", (B, 3, H, W), dev)
+        t1_out = self.ws.get("t1_out_train" if train else "t1_out", (B, C, H, W), dev)
+        out = self.ws.get("out_train" if train else "out", (B, C, H, W), dev)
         # inference: the packed weights are final before the first conv starts, so consecutive layers may overlap their
         # prologue with the previous layer's tail (programmatic dependent launch); not while profiling per layer
         self.pdl_chain = (not train) and self.profile is None and self.impl == IMPL_TC
@@ -727,7 +737,7 @@ class FastDVDnetEngine(_EngineBase):
 
     # ---- backward of one DenBlock -----------------------------------------------------------------------
     def _block_backward(self, blk, S, dout, B, H, W, need_input_grad):
-        """dout [B,3,H,W] = d loss / d block output.  Returns d loss / d (packed input) [B,H,W,32] or None."""
+        """dout [B,C,H,W] = d loss / d block output.  Returns d loss / d (packed input) [B,H,W,32] or None."""
         L = blk.L
         dev = dout.device
         g = self.ws.get
@@ -766,7 +776,7 @@ class FastDVDnetEngine(_EngineBase):
 
         # out = in1 - xo  ->  d xo = -dout (padded columns 0)
         d_xo = g("g_xo", (B, H, W, L[15].Co_pad), dev)
-        call("sci_fastdvd_output_grad", ptr(dout), ptr(d_xo), B, H, W, L[15].Co_pad, stream())
+        call("sci_fastdvd_output_grad_planes", ptr(dout), ptr(d_xo), B, dout.shape[1], H, W, L[15].Co_pad, stream())
         d_o0 = layer_bwd(15, d_xo, S["xo"], S["o0"], B, H, W, nf, "g_f32a", (B, H, W, 32), prev=14)
         d_s0 = layer_bwd(14, d_o0, S["o0"], S["s0"], B, H, W, nf, "g_f32b", (B, H, W, 32))
         # s0 = x0 + PS(conv13(u1b)): gradient of the GEMM output is the pixel-unshuffle of d_s0
@@ -792,15 +802,16 @@ class FastDVDnetEngine(_EngineBase):
                          want_dx=need_input_grad)
 
     def backward(self, dout):
-        """Parameter gradients of both DenBlocks given d loss / d output [B,3,H,W]."""
+        """Parameter gradients of both DenBlocks given d loss / d output [B,C,H,W]."""
         s1, s2, B, H, W = self._saved
         dev = dout.device
         self.begin_backward()
         d_in2 = self._block_backward(self.t2, s2, dout, B, H, W, need_input_grad=True)
         # temp1 output j feeds slot (j - f + 1) of temp2 block f = j-1, j, j+1, and is `in1` of block j
-        d_t1 = self.ws.get("g_t1", (B, 3, H, W), dev)
+        C = dout.shape[1]
+        d_t1 = self.ws.get("g_t1", (B, C, H, W), dev)
         d_t1.copy_(dout)
-        call("sci_fastdvd_pack_input_grad", ptr(d_in2), ptr(d_t1), B, H, W, self.t2.L[0].Ci_pad, 1, stream())
+        call("sci_fastdvd_pack_input_grad_planes", ptr(d_in2), ptr(d_t1), B, C, H, W, self.t2.L[0].Ci_pad, 1, stream())
         self._block_backward(self.t1, s1, d_t1, B, H, W, need_input_grad=False)
         self.finish_param_grads()
 

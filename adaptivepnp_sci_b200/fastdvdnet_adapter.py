@@ -240,12 +240,17 @@ noise_stream = NoiseStream()
 
 
 def finetune_and_denoise(v, phi, y, sigma, model, lr, update_per_iter, grad_sync=None, noise=None, tile=None):
-    """v [B,3,H,W], phi [B,H,W], y [H,W] planar; returns the denoised CLEAN sequence [B,3,H,W].
+    """v [B,C,H,W], phi [B,H,W], y [H,W] planar; returns the denoised CLEAN sequence [B,C,H,W].  C = 3 with the colour
+    model (Bayer measurement), C = 1 with the gray one (the measurement sums the frames themselves; the noise is drawn with
+    shape (B,1,H,W); the twin that is trained is written back into the gray parameters after the last Adam step).
     ``tile`` (parallel.TileView): v is a halo-extended row strip of a larger frame, phi / y cover the own rows; the
     noise is drawn for the WHOLE frame (same global-RNG stream on every rank) and the strip's rows are cut out."""
     from .ffdnet_adapter import _tile_loss
-    eng = _unwrap(model).engine()
-    B, _, H, W = v.shape
+    net = _unwrap(model)
+    if v.shape[1] != net.num_color_channels:
+        raise SciError("sequence has %d planes, the model %d" % (v.shape[1], net.num_color_channels))
+    eng = net.engine()
+    B, C, H, W = v.shape
     dev = v.device
     if isinstance(update_per_iter, int):
         n_update_iter, lr_all = [update_per_iter], [lr]                                  # :344-349
@@ -254,9 +259,9 @@ def finetune_and_denoise(v, phi, y, sigma, model, lr, update_per_iter, grad_sync
     full = None
     if noise is None:
         if tile is None:
-            noise = noise_stream.get((B, 3, H, W))
+            noise = noise_stream.get((B, C, H, W))
         else:
-            full = noise_stream.get((B, 3, tile.H_total, W))
+            full = noise_stream.get((B, C, tile.H_total, W))
             noise = full[:, :, tile.g0:tile.g0 + H]
     noise_h = np.ascontiguousarray(noise, dtype=np.float64)
     if full is not None and noise_h.ctypes.data != full.ctypes.data:
@@ -272,7 +277,7 @@ def finetune_and_denoise(v, phi, y, sigma, model, lr, update_per_iter, grad_sync
         else:
             still.append((e, a))
     _inflight[:] = still + [(ev, noise_h)]
-    vplus = eng.ws.get("vplus", (B, 3, H, W), dev)
+    vplus = eng.ws.get("vplus", (B, C, H, W), dev)
     call("sci_fastdvd_noisy_input", ptr(v), ptr(noise_d), ptr(vplus), v.numel(), stream())    # :359
     eng.prepare(training=True)
     n_steps = int(sum(n_update_iter))
@@ -289,6 +294,8 @@ def finetune_and_denoise(v, phi, y, sigma, model, lr, update_per_iter, grad_sync
             eng.bucket.adam_step(lr_i)                                                    # :446
             eng.after_step()
             k += 1
+    if net.num_color_channels == 1:
+        net._restrict_twin()
     out = eng.forward(v, sigma, train=False)                                              # :453-458
     _tile_loss(eng, out, phi, y, "dout", loss[n_steps:], tile, False)
     last_losses[:] = [loss]
@@ -306,22 +313,16 @@ def denoise_planar(u, pb, sigma, model, lr, do_update, update_per_iter, grad_syn
 
 def fastdvdnet_seqdenoise(seq, noise_std, windsize, model, train=None):
     """fastdvdnet.py:82-146 — seq [N,C,H,W] -> [N,C,H,W], circular 5-frame window (C = 3, or 1 with the gray model, whose
-    frames travel as the first plane of a colour cube: fastdvdnet_models.FastDVDnet)."""
+    frames the engine packs as the first plane of a colour cube: fastdvdnet_models.FastDVDnet)."""
     if windsize != NUM_IN_FR_EXT:
         raise NotImplementedError("window size 5 only")
     net = _unwrap(model)
-    gray = net.num_color_channels == 1
     if seq.shape[1] != net.num_color_channels:
         raise SciError("sequence has %d channels, the model %d" % (seq.shape[1], net.num_color_channels))
     seq = seq.contiguous().float()
-    if gray:
-        seq3 = seq.new_zeros((seq.shape[0], 3, seq.shape[2], seq.shape[3]))
-        seq3[:, 0:1] = seq
-        seq = seq3
     padded, H, W = ops.pad_to_multiple(seq, 4)                                          # reflect pad to x4 (:119-127)
     out = net.engine().forward(padded, float(noise_std.flatten()[0]), train=False)
-    out = ops.crop_to(out, H, W)                                                        # un-pad (:134-141)
-    out = out[:, 0:1].clone() if gray else out.clone()
+    out = ops.crop_to(out, H, W).clone()                                                # un-pad (:134-141)
     return (out, model) if train else out
 
 

@@ -86,7 +86,13 @@ class FastDVDnet(nn.Module):
     test_fastdvdnet.py:149-235) keeps the reference's parameter shapes (``inc`` 3 x (1+1) -> 90 in 3 groups, ``outc``
     32 -> 1) and runs on the colour engine through an exact embedding: a colour-shaped twin holds the same weights with
     zeros in the rows / columns of the two missing colour planes, the frames enter as its first plane, and its first
-    output plane is the result - the zero terms add nothing to any accumulator."""
+    output plane is the result - the zero terms add nothing to any accumulator.  The engine takes gray frames [B,1,H,W]
+    as they are (its boundary kernels pack them as that first plane and compute only the first output plane).
+
+    Fine-tuning the gray model trains the twin (gradients, ``grad_sync`` and Adam on the twin's flat bucket) and writes the
+    result back with ``_restrict_twin``.  The embedded zeros stay exactly +0 through training: their inputs are zero planes
+    and the loss never reads output planes 1 and 2, so their gradients are exactly zero, and an Adam step with g = 0 from
+    fresh moments m = v = 0 moves nothing."""
 
     def __init__(self, num_input_frames=5, num_color_channels=3):
         super().__init__()
@@ -100,6 +106,9 @@ class FastDVDnet(nn.Module):
         self._twin = None
         self._twin_version = None
 
+    def _state_version(self, own):
+        return tuple(int(t._version) for t in own.values()) + tuple(t.data_ptr() for t in own.values())
+
     def _colour_twin(self):
         own = dict(self.state_dict())
         dev = next(self.parameters()).device
@@ -108,7 +117,7 @@ class FastDVDnet(nn.Module):
             self._twin_version = None
         twin = self._twin[0]
         twin.train(self.training)
-        version = tuple(int(t._version) for t in own.values()) + tuple(t.data_ptr() for t in own.values())
+        version = self._state_version(own)
         if version != self._twin_version:
             with torch.no_grad():
                 for k, dst in twin.state_dict().items():
@@ -126,6 +135,25 @@ class FastDVDnet(nn.Module):
                         raise RuntimeError("gray FastDVDnet: unexpected parameter shape for " + k)
             self._twin_version = version
         return twin
+
+    def _restrict_twin(self):
+        """Inverse of the embedding of ``_colour_twin``: the twin's (fine-tuned) weights back into the gray parameters, so
+        that ``state_dict()`` holds them.  The twin's version is recorded after the write-back: it is not re-copied over
+        itself on the next use."""
+        own = dict(self.state_dict())
+        with torch.no_grad():
+            for k, src in self._twin[0].state_dict().items():
+                dst = own[k]
+                if src.shape == dst.shape:
+                    dst.copy_(src)
+                elif k.endswith("inc.convblock.0.weight"):            # [r, g, b, sigma] per frame group -> [y, sigma]
+                    dst[:, 0].copy_(src[:, 0])
+                    dst[:, 1].copy_(src[:, 3])
+                elif k.endswith("outc.convblock.3.weight"):           # first of 32 -> 3 becomes 32 -> 1
+                    dst.copy_(src[0:1])
+                else:
+                    raise RuntimeError("gray FastDVDnet: unexpected parameter shape for " + k)
+        self._twin_version = self._state_version(own)
 
     def engine(self):
         from .engine import FastDVDnetEngine

@@ -236,7 +236,7 @@ typedef struct sci_conv_desc {
                                accuracy of the "3xTF32" scheme at the fp16 tensor rate and half the bytes */
     int emit_lo;            /* TC only. 1: y has 2*Cout channels per pixel: [tf32(v) | tf32(v - tf32(v))]; the next
                                layer is packed with ci_dup = Cout so it multiplies both ("3xTF32": ~fp32 accuracy) */
-    const float* planar_in1; /* TC only, with planar_out: [N][3][H][W] frames                                   */
+    const float* planar_in1; /* TC only, with planar_out: [N][P][H][W] frames, P = planar_planes                */
     float* planar_out;      /* TC only. non-NULL: the layer is the last conv of a FastDVDnet DenBlock (Cout == 32, 3 real
                                channels): instead of y the kernel writes out[n][c][h][w] = planar_in1[n][c][h][w] - conv[c]
                                (packages/fastdvdnet/models.py:196) as planar frames; y may be NULL */
@@ -270,6 +270,9 @@ typedef struct sci_conv_desc {
     int K_used;             /* TC only. > 0: only the first K_used input channels (K columns of the packed weights) can be non-zero;
                                the MMAs over the all-zero tail of the last 128-byte channel chunk are skipped (results unchanged).
                                0 = Cin */
+    int planar_planes;      /* TC only, with planar_out: planes P per frame of planar_in1 / planar_out, 3 (colour) or 1 (the
+                               gray FastDVDnet: columns 1 and 2 of the layer, all-zero weights in the colour-shaped embedding,
+                               are not written).  0 = 3 */
 } sci_conv_desc;
 
 /* 1 if this build contains the tcgen05 tensor-core convolution kernels. */
@@ -311,6 +314,10 @@ int sci_conv_pack_weights_half(const float* w, void* packed, int Co, int Ci, int
  * out [B][H][W][C] binary16 (C = 32 or 64), channels 0..11 = fp16 of [f0 RGB, sigma, f1 RGB, sigma, f2 RGB, sigma], 16..27 =
  * the fp16 remainders, others zero. */
 int sci_fastdvd_pack_input_half(const float* frames, float sigma, void* out, int B, int H, int W, int C, void* stream);
+/* The same with frames of NC planes (3, or 1 for gray frames: channels slot*4+1 and slot*4+2 are then +0, bit for bit what
+ * packing the zero-embedded colour cube gives).  sci_fastdvd_pack_input_half is this with NC = 3. */
+int sci_fastdvd_pack_input_half_planes(const float* frames, float sigma, void* out, int B, int NC, int H, int W, int C,
+                                       void* stream);
 /* Data-gradient weights of a STRIDE-2 layer (groups = 1) as a sub-pixel convolution over dz at the low resolution:
  * packed [9][4*Ci_pad][Co_pad]; run sci_conv3x3_dgrad with x = dz [N][Ho][Wo][Co_pad], Cin = Co_pad, Cout = 4*Ci_pad,
  * stride 1, pixel_shuffle = 1 -> dx [N][2Ho][2Wo][Ci_pad].  Replaces "zero-dilate dz, then convolve at full resolution"
@@ -381,6 +388,17 @@ int sci_fastdvd_output(const float* frames, const float* y, float* out, int B, i
 int sci_fastdvd_output_grad(const float* dout, float* dy, int B, int H, int W, int Cpad, void* stream);
 int sci_fastdvd_pack_input_grad(const float* din, float* dframes, int B, int H, int W, int Cpad, int accumulate,
                                 void* stream);
+/* The four above for frames of NC planes: 3 (the entry points above are these with NC = 3) or 1 (gray FastDVDnet in the
+ * colour-shaped embedding: frames / out / dout / dframes [B][1][H][W]; the packer writes the frame into channel slot*4 and +0
+ * into slot*4+1..2, the output kernels read or write column / plane 0 only).  For NC = 1 every result is bit for bit the NC = 3
+ * result on the zero-embedded cube (plane 0 of it for the planar outputs). */
+int sci_fastdvd_pack_input_planes(const float* frames, float sigma, float* out, int B, int NC, int H, int W, int Cpad,
+                                  int round_tf32, void* stream);
+int sci_fastdvd_output_planes(const float* frames, const float* y, float* out, int B, int NC, int H, int W, int Cpad,
+                              void* stream);
+int sci_fastdvd_output_grad_planes(const float* dout, float* dy, int B, int NC, int H, int W, int Cpad, void* stream);
+int sci_fastdvd_pack_input_grad_planes(const float* din, float* dframes, int B, int NC, int H, int W, int Cpad, int accumulate,
+                                       void* stream);
 /* ---- DDnet deep-demosaic boundary (models/network_demosaicking.py:377-463; packages/DDnet/DDnet_test.py:166-204) ----
  * mosaic [B][H][W] planar (the sum over the three sparse colour planes DDnet takes, :411-416 — sci_rgb_sum).
  * The triples of the circular 5-window are stacked as batch n = j*B + f (j = triple 0..2, f = centre frame); triple j,
