@@ -77,6 +77,7 @@ PROTOTYPES = {
     "sci_conv_unpack_wgrad": [_p, _p, _i, _i, _i, _i, _i, _i, _i, _p],
     "sci_bn_fold": [_p, _p, _p, _p, _f, _p, _p, _i, _i, _p],
     "sci_act_bwd": [_p, _p, _p, _l, _i, _i, _p, _p, _p],
+    "sci_act_bwd_ordered": [_p, _p, _p, _l, _i, _i, _p, _p, _p, _sz, _p],
     "sci_bn_param_grad": [_p, _p, _p, _p, _p, _p, _i, _p],
     "sci_nhwc_pixel_unshuffle": [_p, _p, _i, _i, _i, _i, _p],
     "sci_nhwc_dilate2": [_p, _p, _i, _i, _i, _i, _p],
@@ -116,7 +117,9 @@ PROTOTYPES = {
     "sci_axpy": [_p, _f, _p, _p, _l, _p],
     "sci_adam_step": [_p, _p, _p, _p, _l, _d, _d, _d, _d, _i, _p],
 }
-_SPECIAL_RESTYPE = {"sci_last_error": ctypes.c_char_p, "sci_tv_workspace_bytes": _sz, "sci_tv_strip_workspace_bytes": _sz}
+_SPECIAL_RESTYPE = {"sci_last_error": ctypes.c_char_p, "sci_tv_workspace_bytes": _sz, "sci_tv_strip_workspace_bytes": _sz,
+                    "sci_conv3x3_fwd_workspace_bytes": _sz, "sci_conv3x3_wgrad_workspace_bytes": _sz,
+                    "sci_act_bwd_workspace_bytes": _sz}
 
 for _name, _args in PROTOTYPES.items():
     _fn = getattr(lib, _name)
@@ -128,6 +131,12 @@ lib.sci_tv_workspace_bytes.argtypes = [_i, _i, _i]
 lib.sci_tv_workspace_bytes.restype = _sz
 lib.sci_tv_strip_workspace_bytes.argtypes = [_i, _i, _i]
 lib.sci_tv_strip_workspace_bytes.restype = _sz
+lib.sci_conv3x3_fwd_workspace_bytes.argtypes = [_p, _i]
+lib.sci_conv3x3_fwd_workspace_bytes.restype = _sz
+lib.sci_conv3x3_wgrad_workspace_bytes.argtypes = [_p, _i]
+lib.sci_conv3x3_wgrad_workspace_bytes.restype = _sz
+lib.sci_act_bwd_workspace_bytes.argtypes = [_l, _i]
+lib.sci_act_bwd_workspace_bytes.restype = _sz
 
 
 class SciError(RuntimeError):
@@ -153,7 +162,7 @@ def check(rc, what):
 
 # kernel launches issued through the C ABI since import (bench.py reports the count inside its timed region)
 KERNELS_PER_CALL = {"sci_tv_chambolle2d": 3, "sci_tv_strip_main": 2, "sci_tv_strip_finish": 2, "sci_version": 0,
-                    "sci_conv_tc_available": 0, "sci_host_legacy_normal": 0}
+                    "sci_conv_tc_available": 0, "sci_host_legacy_normal": 0, "sci_act_bwd_ordered": 2}
 launch_count = 0
 
 

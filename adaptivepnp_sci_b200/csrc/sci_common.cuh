@@ -44,12 +44,25 @@ static inline cudaError_t sci_smem_limit(const void* kernel, int bytes) {
         if (k == kernel) break;
     }
     if (i < SLOTS && (devices[i].load(std::memory_order_acquire) & bit)) return cudaSuccess;
+    // static and dynamic shared memory share the per-block opt-in maximum: a kernel with more static shared memory gets a
+    // correspondingly lower dynamic limit (its launches stay within it)
+    cudaFuncAttributes fa;
+    int optin = 0;
+    if (cudaFuncGetAttributes(&fa, kernel) == cudaSuccess &&
+        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) == cudaSuccess && optin > 0)
+        bytes = bytes < optin - (int)fa.sharedSizeBytes ? bytes : optin - (int)fa.sharedSizeBytes;
     const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
     if (e == cudaSuccess && i < SLOTS) devices[i].fetch_or(bit, std::memory_order_release);
     return e;
 }
 
 static inline int sci_ceil_div(long a, long b) { return (int)((a + b - 1) / b); }
+
+// Second half of every fixed-order reduction (sci_train.cu): out0[i] = out0[i] + (((part[0][i] + part[1][i]) + ...) over the
+// `slots` slots of `width` floats at `part`, in slot order, for i < n; out1 likewise over part[b][n + i].  NULL outputs are
+// skipped.  The first half - one kernel whose block b STORES its partial sums into slot b - replaces atomic adds, so the
+// result no longer depends on the order in which blocks finish.
+int sci_ordered_slot_sum(const float* part, int slots, long width, long n, float* out0, float* out1, void* stream);
 
 // Streaming (read-once) 128-bit load: bypass L1 allocation, keep L2.
 __device__ __forceinline__ float4 ldg_stream4(const float* p) {

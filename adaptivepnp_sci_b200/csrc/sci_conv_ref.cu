@@ -98,7 +98,10 @@ __global__ void __launch_bounds__(256) conv3x3_ref_kernel(sci_conv_desc d) {
 }
 
 // Weight gradient: one block = one tap x (64 co x 64 ci) tile x one chunk of output pixels.
+// ORDERED: d.dw points at slot 0 of a [chunks][9][Cout][Cin] workspace; pixel chunk b stores its partial into slot b
+// (sci_ordered_slot_sum then adds the slots in order) instead of adding it into dw with atomics.
 constexpr int WG_PIX = 16;
+template <bool ORDERED>
 __global__ void __launch_bounds__(256) wgrad_ref_kernel(sci_wgrad_desc d, int pix_per_block) {
     __shared__ float sZ[WG_PIX][64];
     __shared__ float sX[WG_PIX][64];
@@ -150,7 +153,9 @@ __global__ void __launch_bounds__(256) wgrad_ref_kernel(sci_wgrad_desc d, int pi
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int ci = ci0 + tx * 4 + j;
-            if (ci < d.Cin) atomicAdd(&d.dw[((long)tap * d.Cout + co) * d.Cin + ci], s * acc[i][j]);
+            if (ci >= d.Cin) continue;
+            if (ORDERED) d.dw[((long)blockIdx.x * 9 + tap) * d.Cout * d.Cin + (long)co * d.Cin + ci] = s * acc[i][j];
+            else atomicAdd(&d.dw[((long)tap * d.Cout + co) * d.Cin + ci], s * acc[i][j]);
         }
     }
 }
@@ -166,15 +171,31 @@ int sci_conv3x3_ref_launch(const sci_conv_desc* d, void* stream) {
     return SCI_OK;
 }
 
-int sci_wgrad_ref_launch(const sci_wgrad_desc* d, void* stream) {
+// pixel chunks of the weight-gradient launch (its grid.x) and the pixels per chunk
+static int wgrad_ref_chunks(const sci_wgrad_desc* d, int* ppb_out) {
     const int Ho = (d->H - 1) / d->stride + 1, Wo = (d->W - 1) / d->stride + 1;
     const long npix = (long)d->N * Ho * Wo;
     int chunks = (int)min((long)SCI_NUM_SMS * 2, (npix + 255) / 256);
     const int ppb = (int)((npix + chunks - 1) / chunks);
     const int ppb_al = ((ppb + WG_PIX - 1) / WG_PIX) * WG_PIX;
-    chunks = (int)((npix + ppb_al - 1) / ppb_al);
+    if (ppb_out) *ppb_out = ppb_al;
+    return (int)((npix + ppb_al - 1) / ppb_al);
+}
+
+int sci_wgrad_ref_slots(const sci_wgrad_desc* d) { return wgrad_ref_chunks(d, nullptr); }
+
+int sci_wgrad_ref_launch(const sci_wgrad_desc* d, void* stream) {
+    int ppb_al = 0;
+    const int chunks = wgrad_ref_chunks(d, &ppb_al);
     const dim3 grid(chunks, 9, ((d->Cout + 63) / 64) * ((d->Cin + 63) / 64));
-    wgrad_ref_kernel<<<grid, 256, 0, sci_stream(stream)>>>(*d, ppb_al);
+    if (d->workspace) {
+        sci_wgrad_desc o = *d;
+        o.dw = static_cast<float*>(d->workspace);
+        wgrad_ref_kernel<true><<<grid, 256, 0, sci_stream(stream)>>>(o, ppb_al);
+        SCI_CHECK_LAUNCH("wgrad ref");
+        return sci_ordered_slot_sum(o.dw, chunks, 9L * d->Cout * d->Cin, 9L * d->Cout * d->Cin, d->dw, nullptr, stream);
+    }
+    wgrad_ref_kernel<false><<<grid, 256, 0, sci_stream(stream)>>>(*d, ppb_al);
     SCI_CHECK_LAUNCH("wgrad ref");
     return SCI_OK;
 }

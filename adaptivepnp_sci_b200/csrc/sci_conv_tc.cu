@@ -23,6 +23,7 @@
 
 int sci_conv3x3_ref_launch(const sci_conv_desc* d, void* stream);
 int sci_wgrad_ref_launch(const sci_wgrad_desc* d, void* stream);
+int sci_wgrad_ref_slots(const sci_wgrad_desc* d);
 
 namespace {
 
@@ -446,7 +447,9 @@ struct Fwd2Params {
     // the stored tensor (the missing half is written as zeros); Cstore = channels per pixel of the stored output tensor
     int ucols, Cstore;
     // MODE 4 (data gradient + activation backward of the layer that PRODUCED this tensor, fused): dz = (conv [+ residual]) *
-    // (mask_y > 0); col_s1[c] += sum dz, col_s2[c] += sum dz * mask_y  (bias / BatchNorm gradients), see the epilogue
+    // (mask_y > 0); col_s1[c] += sum dz, col_s2[c] += sum dz * mask_y  (bias / BatchNorm gradients), see the epilogue.
+    // MODE 5 = MODE 4 with fixed-order sums: col_s1 is then slot 0 of this launch's [grid][2][ncol] workspace slots (ncol =
+    // stored channels) and col_s2 only says whether the second sums are wanted
     const float* mask_y; float* col_s1; float* col_s2; int mask_relu;
     // split > 0 (HALF, FFDNet inference at ~fp32 accuracy): every activation and weight travels as fp16 value + fp16 remainder
     // scaled by 2^11; a 64-channel chunk is [32 values | their 32 remainders].  Per chunk the issuer multiplies value x value
@@ -469,7 +472,8 @@ struct Fwd2Params {
 //     second group shares the quarters and takes every second (row, chunk) unit): two warps per scheduler hide each
 //     other's latencies;
 //   * MODE selects the epilogue at compile time (0 = TMA store, 1 = TMA store + skip-add, 2 = fused planar network
-//     output of 3 planes, 3 = the same with 1 plane (gray), 4 = data gradient with the fused activation backward) instead of run-time flags per element; scale / shift come from shared memory as float4;
+//     output of 3 planes, 3 = the same with 1 plane (gray), 4 = data gradient with the fused activation backward, 5 = the
+//     same with fixed-order column sums) instead of run-time flags per element; scale / shift come from shared memory as float4;
 //   * the planar mode fetches the in1 values of ALL its rows before it waits for the accumulator (the per-row prefetch
 //     left the HBM latency of those loads exposed: 46 % of the epilogue's samples in the 32->3 layer).
 //   * HALF: fp16 storage and operands (kind::f16, fp32 accumulation): the same 11-bit significand as TF32 - the products
@@ -484,10 +488,14 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     __shared__ uint32_t tmem_slot;
     __shared__ __align__(16) float s_scale[128], s_shift[128];
     __shared__ float s_cs1[MODE == 4 ? 128 : 1], s_cs2[MODE == 4 ? 128 : 1];      // CTA partial column sums (MODE 4)
+    __shared__ float s_wcs[MODE == 5 ? 4 * EPI_WG : 1][2][128];                    // per epilogue warp (MODE 5)
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (MODE == 4) {
         for (int i = threadIdx.x; i < 128; i += 128 + 128 * EPI_WG) { s_cs1[i] = 0.f; s_cs2[i] = 0.f; }
+    }
+    if (MODE == 5) {
+        for (int i = threadIdx.x; i < 4 * EPI_WG * 2 * 128; i += 128 + 128 * EPI_WG) (&s_wcs[0][0][0])[i] = 0.f;
     }
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t b_bytes = (uint32_t)p.Cout * (uint32_t)p.rb_in;
@@ -965,7 +973,7 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     const int t = u / nch, c0 = (u - t * nch) << 5;
                     const int ho = y0 + t;
                     float v[32];
-                    if (MODE == 4) {
+                    if (MODE == 4 || MODE == 5) {
                         // ---- data gradient + activation backward, fused (replaces a separate pass over dy, y and dz) ----
                         // operands of this unit from global memory first (the other warpgroup hides their latency)
                         float4 yy[8], ra[8];
@@ -1045,8 +1053,16 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                             // column of the stored tensor this lane summed (PixelShuffle: the sub-pixel groups share the channels)
                             const int cg = p.col0 + c0;
                             const int cc = (p.ps ? cg % Cq : cg) + lane;
-                            atomicAdd(&s_cs1[cc], cs1);
-                            if (p.col_s2) atomicAdd(&s_cs2[cc], cs2);
+                            if (MODE == 5) {
+                                // this warp's own row of partials: every address has ONE writer (lane cc % 32 of this warp)
+                                // and a thread's reductions to one address apply in program order, i.e. in the fixed order
+                                // the units reach the warp - the fire-and-forget shared reduction of MODE 4, deterministic
+                                atomicAdd(&s_wcs[warp - 4][0][cc], cs1);
+                                if (p.col_s2) atomicAdd(&s_wcs[warp - 4][1][cc], cs2);
+                            } else {
+                                atomicAdd(&s_cs1[cc], cs1);
+                                if (p.col_s2) atomicAdd(&s_cs2[cc], cs2);
+                            }
                         }
                         __syncwarp();
                         continue;
@@ -1115,6 +1131,20 @@ conv_fwd2_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             if (e < min(ncol, 128)) {
                 atomicAdd(p.col_s1 + e, s_cs1[e]);
                 if (p.col_s2) atomicAdd(p.col_s2 + e, s_cs2[e]);
+            }
+        }
+        if (MODE == 5 && p.col_s1) {
+            // column e of the CTA's slot = the epilogue warps' partials added in warp order
+            asm volatile("bar.sync 1, %0;" ::"r"(128 * EPI_WG) : "memory");
+            const int e = threadIdx.x - 128;
+            const int ncol = p.ps ? Cq : p.Ctot;
+            if (e < min(ncol, 128)) {
+                float a1 = s_wcs[0][0][e], a2 = s_wcs[0][1][e];
+#pragma unroll
+                for (int w = 1; w < 4 * EPI_WG; ++w) { a1 += s_wcs[w][0][e]; a2 += s_wcs[w][1][e]; }
+                float* slot = p.col_s1 + (long)blockIdx.x * 2 * ncol;
+                slot[e] = a1;
+                if (p.col_s2) slot[ncol + e] = a2;
             }
         }
     }
@@ -1295,8 +1325,10 @@ bool fwd2_eligible(const sci_conv_desc* d) {
            env_int("SCI_CONV_V2", 1) != 0;
 }
 
-// columns [col0, col0 + ncols) of the layer
-int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncols) {
+// columns [col0, col0 + ncols) of the layer.  ord_slots != NULL: fused data gradient with fixed-order column sums (MODE 5)
+// into the [grid][2][stored channels] slots there.  grid_out: the launch's grid; plan_only: only that, no launch.
+int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncols, float* ord_slots = nullptr,
+                        int* grid_out = nullptr, bool plan_only = false) {
     const bool half = d->half_io != 0;
     const int esz = half ? 2 : 4;
     const int rb_in = operand_row_bytes(d);
@@ -1350,6 +1382,7 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
         if (half || p.planar_out || (d->pixel_shuffle ? d->Cout / 4 : d->Cout) > 128 || (d->col_s2 && !d->col_s1))
             return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: fused activation backward needs the fp32 TMA-store path and <= 128 stored channels");
         mode = 4;
+        if (ord_slots && d->col_s1) { mode = 5; p.col_s1 = ord_slots; }
     }
     const int w_bytes = 9 * p.k_chunks * b_bytes;
     // shared-memory plan: [resident weights] [pipeline stages] [store staging: 4 * epi_wg warps x out_bufs x 4 KB].
@@ -1410,6 +1443,9 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     p.num_tiles = p.tiles_w * p.tiles_h * p.N;
     p.tmem_cols = next_pow2_cols(2 * p.R * p.acc_stride);
     p.dbg = env_int("SCI_CONV_DBG", 0);
+    const int grid = min(p.num_tiles, SCI_NUM_SMS);
+    if (grid_out) *grid_out = grid;
+    if (plan_only) return SCI_OK;
     CUtensorMap tmA, tmB;
     // activation map with a {kch ch, 130 px, 1 row, 1 image} box.  fp16: the channel extent is the STORED one; a box that
     // sticks out of it (e.g. channels 64..127 of a 96-channel tensor) is zero-filled by TMA, matching the zero rows of the
@@ -1436,19 +1472,18 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
     const size_t smem = (size_t)(p.resident ? w_bytes : 0) + (size_t)p.stages * stage_bytes + out_stage + 1024;
     if (smem > 220 * 1024) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: shared memory budget exceeded");
     typedef void (*Fwd2Kernel)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const Fwd2Params);
-    // indexed by MODE (MODE 4 exists for fp32 only)
-    static const Fwd2Kernel kernels[2][2][5] = {
+    // indexed by MODE (MODEs 4 and 5 exist for fp32 only)
+    static const Fwd2Kernel kernels[2][2][6] = {
         {{conv_fwd2_tc_kernel<1, 0, false>, conv_fwd2_tc_kernel<1, 1, false>, conv_fwd2_tc_kernel<1, 2, false>,
-          conv_fwd2_tc_kernel<1, 3, false>, conv_fwd2_tc_kernel<1, 4, false>},
+          conv_fwd2_tc_kernel<1, 3, false>, conv_fwd2_tc_kernel<1, 4, false>, conv_fwd2_tc_kernel<1, 5, false>},
          {conv_fwd2_tc_kernel<2, 0, false>, conv_fwd2_tc_kernel<2, 1, false>, conv_fwd2_tc_kernel<2, 2, false>,
-          conv_fwd2_tc_kernel<2, 3, false>, conv_fwd2_tc_kernel<2, 4, false>}},
+          conv_fwd2_tc_kernel<2, 3, false>, conv_fwd2_tc_kernel<2, 4, false>, conv_fwd2_tc_kernel<2, 5, false>}},
         {{conv_fwd2_tc_kernel<1, 0, true>, conv_fwd2_tc_kernel<1, 1, true>, conv_fwd2_tc_kernel<1, 2, true>,
-          conv_fwd2_tc_kernel<1, 3, true>, nullptr},
+          conv_fwd2_tc_kernel<1, 3, true>, nullptr, nullptr},
          {conv_fwd2_tc_kernel<2, 0, true>, conv_fwd2_tc_kernel<2, 1, true>, conv_fwd2_tc_kernel<2, 2, true>,
-          conv_fwd2_tc_kernel<2, 3, true>, nullptr}}};
+          conv_fwd2_tc_kernel<2, 3, true>, nullptr, nullptr}}};
     const Fwd2Kernel kern = kernels[half ? 1 : 0][epi_wg - 1][mode];
     if (!kern) return sci_fail(SCI_EUNSUPPORTED, "conv tc v2: epilogue not built");
-    const int grid = min(p.num_tiles, SCI_NUM_SMS);
     const int threads = 128 + 128 * epi_wg;
     p.pdl = (d->pdl && env_int("SCI_CONV_PDL", 1)) ? 1 : 0;
     if (env_int("SCI_CONV_VERBOSE", 0))
@@ -1466,7 +1501,8 @@ int conv_fwd2_tc_launch(const sci_conv_desc* d, void* stream, int col0, int ncol
 //   {32 ch, 8 px, 8 rows, 1 image} of dz and of x at the tap-shifted (and, for stride-2 layers, element-strided)
 //   coordinates; out-of-image pixels are zero-filled.  One CTA group owns a filter row and one 128-wide M block, each
 //   CTA a strided subset of the 8x8 pixel tiles; it accumulates in TMEM and finishes with red.global.add into the
-//   packed gradient.  The launch list of a first version with M = Cout fixed (profiles/) showed the full-resolution
+//   packed gradient (ORDERED: with plain stores into its own region of slot blockIdx.x of a [gx][9][Cout][Cin] workspace
+//   at p.dw, which sci_ordered_slot_sum adds into dw in slot order).  The launch list of a first version with M = Cout fixed (profiles/) showed the full-resolution
 //   32-channel layers at 0.73-0.89 ms each: with M = 32 of 128 rows used, three quarters of every MMA were wasted and
 //   each tap reloaded the dz tile.  Hence
 //   * swap = 0: M side = dz (Cout), N side = x.  swap = 1: M side = x (Cin), N side = dz (Cout) - chosen when that
@@ -1485,6 +1521,7 @@ struct Wgrad2Params {
     int swap, fuse, p_chunks, q_chunks, n_mma, accs, m_tiles, tmem_cols, stages;
 };
 
+template <bool ORDERED>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 conv_wgrad2_tc_kernel(const __grid_constant__ CUtensorMap tmZ, const __grid_constant__ CUtensorMap tmX, const Wgrad2Params p) {
     extern __shared__ uint8_t smem_raw[];
@@ -1573,9 +1610,10 @@ conv_wgrad2_tc_kernel(const __grid_constant__ CUtensorMap tmZ, const __grid_cons
         }
         tc_commit_elect(&done_bar);
     } else if (warp >= 4) {
-        // ===== epilogue: TMEM -> registers -> red.global.add into the packed gradient =====
+        // ===== epilogue: TMEM -> registers -> red.global.add into the packed gradient (ORDERED: stores into the slot) =====
         const int q = warp & 3;
         const int m = q * 32 + lane;
+        float* const dw = ORDERED ? p.dw + (long)blockIdx.x * 9 * p.Cout * p.Cin : p.dw;
         mbar_wait(&done_bar, 0);
         tc_fence_after();
         for (int a = 0; a < p.accs; ++a) {
@@ -1589,11 +1627,15 @@ conv_wgrad2_tc_kernel(const __grid_constant__ CUtensorMap tmZ, const __grid_cons
                     const int s = p.fuse ? c0 / p.Cin : a, ci0 = p.fuse ? c0 % p.Cin : c0;
                     if (co < p.Cout) {
                         const float sc = p.oscale ? p.oscale[co] : 1.f;
-                        float* dst = p.dw + ((long)(frow * 3 + s) * p.Cout + co) * p.Cin + ci0;
+                        float* dst = dw + ((long)(frow * 3 + s) * p.Cout + co) * p.Cin + ci0;
 #pragma unroll
-                        for (int j = 0; j < 32; j += 4)
-                            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(v[j] * sc),
-                                         "f"(v[j + 1] * sc), "f"(v[j + 2] * sc), "f"(v[j + 3] * sc) : "memory");
+                        for (int j = 0; j < 32; j += 4) {
+                            if (ORDERED)
+                                *reinterpret_cast<float4*>(dst + j) = make_float4(v[j] * sc, v[j + 1] * sc, v[j + 2] * sc, v[j + 3] * sc);
+                            else
+                                asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(v[j] * sc),
+                                             "f"(v[j + 1] * sc), "f"(v[j + 2] * sc), "f"(v[j + 3] * sc) : "memory");
+                        }
                     }
                 } else {
                     // row = (tap s, input channel), columns = output channels: lanes are consecutive ci -> coalesced reds
@@ -1603,7 +1645,9 @@ conv_wgrad2_tc_kernel(const __grid_constant__ CUtensorMap tmZ, const __grid_cons
                         for (int j = 0; j < 32; ++j) {
                             const int co = c0 + j;
                             const float sc = p.oscale ? __ldg(p.oscale + co) : 1.f;
-                            atomicAdd(p.dw + ((long)(frow * 3 + s) * p.Cout + co) * p.Cin + ci, v[j] * sc);
+                            float* dst = dw + ((long)(frow * 3 + s) * p.Cout + co) * p.Cin + ci;
+                            if (ORDERED) *dst = v[j] * sc;
+                            else atomicAdd(dst, v[j] * sc);
                         }
                     }
                 }
@@ -1618,7 +1662,8 @@ conv_wgrad2_tc_kernel(const __grid_constant__ CUtensorMap tmZ, const __grid_cons
     }
 }
 
-int conv_wgrad2_tc_launch(const sci_wgrad_desc* d, void* stream) {
+// slots != NULL: only the plan - *slots = the launch's CTA columns gx (the workspace slots of the ordered form), no launch
+int conv_wgrad2_tc_launch(const sci_wgrad_desc* d, void* stream, int* slots = nullptr) {
     Wgrad2Params p;
     p.oscale = d->oscale; p.dw = d->dw;
     p.N = d->N; p.stride = d->stride; p.Cin = d->Cin; p.Cout = d->Cout;
@@ -1649,18 +1694,24 @@ int conv_wgrad2_tc_launch(const sci_wgrad_desc* d, void* stream) {
     const size_t stage_bytes = (size_t)4 * WG_CHUNK_BYTES + (size_t)p.q_chunks * WG_CHUNK_BYTES;
     p.stages = (int)min((size_t)4, (size_t)(214 * 1024) / stage_bytes);
     if (p.stages < 2) return sci_fail(SCI_EUNSUPPORTED, "wgrad tc v2: pipeline does not fit");
+    const int groups = 3 * p.m_tiles;
+    const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS / groups));
+    if (slots) { *slots = gx; return SCI_OK; }
     CUtensorMap tmZ, tmX;
     int rc = make_act_map(&tmZ, d->dz, d->N, p.Ho, p.Wo, d->Cout, 1, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (rc) return rc;
     rc = make_act_map(&tmX, d->x, d->N, d->H, d->W, d->Cin, d->stride, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (rc) return rc;
     const size_t smem = p.stages * stage_bytes + 1024;
-    const int groups = 3 * p.m_tiles;
-    const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS / groups));
     if (env_int("SCI_CONV_VERBOSE", 0))
         fprintf(stderr, "wgrad v2 plan: %dx%d Cin %d Cout %d stride %d | swap %d fuse %d m_tiles %d accs %d stages %d grid %d groups %d tiles %d\n",
                 d->H, d->W, d->Cin, d->Cout, d->stride, p.swap, p.fuse, p.m_tiles, p.accs, p.stages, gx, groups, p.num_tiles);
-    return launch(conv_wgrad2_tc_kernel, dim3(gx, groups), TC_THREADS, smem, stream, false, "conv tc wgrad v2", tmZ, tmX, p);
+    if (d->workspace) {
+        p.dw = static_cast<float*>(d->workspace);
+        rc = launch(conv_wgrad2_tc_kernel<true>, dim3(gx, groups), TC_THREADS, smem, stream, false, "conv tc wgrad v2", tmZ, tmX, p);
+        return rc ? rc : sci_ordered_slot_sum(p.dw, gx, 9L * p.Cout * p.Cin, 9L * p.Cout * p.Cin, d->dw, nullptr, stream);
+    }
+    return launch(conv_wgrad2_tc_kernel<false>, dim3(gx, groups), TC_THREADS, smem, stream, false, "conv tc wgrad v2", tmZ, tmX, p);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1685,6 +1736,7 @@ struct Wgrad3Params {
     int p_is_dz, p_chunks, q_chunks, q_slots, n_tot, tmem_cols, stages;
 };
 
+template <bool ORDERED>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 conv_wgrad3_tc_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_constant__ CUtensorMap tmQ, const Wgrad3Params p) {
     extern __shared__ uint8_t smem_raw[];
@@ -1765,8 +1817,10 @@ conv_wgrad3_tc_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_cons
         }
         tc_commit_elect(&done_bar);
     } else if (warp >= 4) {
-        // ===== epilogue: TMEM -> registers -> red.global.add into the packed gradient dw[tap][co][ci] =====
+        // ===== epilogue: TMEM -> registers -> red.global.add into the packed gradient dw[tap][co][ci] (ORDERED: plain stores
+        // into slot blockIdx.x of the [gx][9][Cout][Cin] workspace at p.dw; each CTA covers the whole slot) =====
         const int i = warp & 3;                        // stacked view index: TMEM lanes 32 i .. 32 i + 31
+        float* const dw = ORDERED ? p.dw + (long)blockIdx.x * 9 * p.Cout * p.Cin : p.dw;
         if (i < 3 && blockIdx.x < p.num_tiles) {
             mbar_wait(&done_bar, 0);
             tc_fence_after();
@@ -1781,17 +1835,23 @@ conv_wgrad3_tc_kernel(const __grid_constant__ CUtensorMap tmP, const __grid_cons
                     const int tap = r * 3 + s;
                     if (p.p_is_dz) {                   // row = output channel, 32 consecutive input channels
                         const float sc = p.oscale ? p.oscale[pch] : 1.f;
-                        float* dst = p.dw + ((long)tap * p.Cout + pch) * p.Cin + q0;
+                        float* dst = dw + ((long)tap * p.Cout + pch) * p.Cin + q0;
 #pragma unroll
-                        for (int j = 0; j < 32; j += 4)
-                            asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(v[j] * sc),
-                                         "f"(v[j + 1] * sc), "f"(v[j + 2] * sc), "f"(v[j + 3] * sc) : "memory");
+                        for (int j = 0; j < 32; j += 4) {
+                            if (ORDERED)
+                                *reinterpret_cast<float4*>(dst + j) = make_float4(v[j] * sc, v[j + 1] * sc, v[j + 2] * sc, v[j + 3] * sc);
+                            else
+                                asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + j), "f"(v[j] * sc),
+                                             "f"(v[j + 1] * sc), "f"(v[j + 2] * sc), "f"(v[j + 3] * sc) : "memory");
+                        }
                     } else {                           // row = input channel (lanes consecutive -> coalesced), 32 output channels
 #pragma unroll
                         for (int j = 0; j < 32; ++j) {
                             const int co = q0 + j;
                             const float sc = p.oscale ? __ldg(p.oscale + co) : 1.f;
-                            atomicAdd(p.dw + ((long)tap * p.Cout + co) * p.Cin + pch, v[j] * sc);
+                            float* dst = dw + ((long)tap * p.Cout + co) * p.Cin + pch;
+                            if (ORDERED) *dst = v[j] * sc;
+                            else atomicAdd(dst, v[j] * sc);
                         }
                     }
                 }
@@ -1811,7 +1871,8 @@ bool wgrad3_eligible(const sci_wgrad_desc* d) {
     return d->stride == 1 && (cp == 32 || cp == 64) && cq <= 96 && (cp / 32) * 3 * cq <= 512 && env_int("SCI_WGRAD_V3", 1) != 0;
 }
 
-int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream) {
+// slots: as conv_wgrad2_tc_launch
+int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream, int* slots = nullptr) {
     Wgrad3Params p;
     p.oscale = d->oscale; p.dw = d->dw;
     p.N = d->N; p.H = d->H; p.W = d->W; p.Cin = d->Cin; p.Cout = d->Cout;
@@ -1825,6 +1886,8 @@ int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream) {
     // the 4th (unused) stacked view of the last k-step reads up to 1 KB past the P box: keep a guard after the ring
     p.stages = (int)min((size_t)4, (size_t)(212 * 1024) / stage_bytes);
     if (p.stages < 2) return sci_fail(SCI_EUNSUPPORTED, "wgrad tc v3: pipeline does not fit");
+    const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS));
+    if (slots) { *slots = gx; return SCI_OK; }
     CUtensorMap tmP, tmQ;
     const float* P = p.p_is_dz ? d->dz : d->x;
     const float* Q = p.p_is_dz ? d->x : d->dz;
@@ -1833,11 +1896,15 @@ int conv_wgrad3_tc_launch(const sci_wgrad_desc* d, void* stream) {
     rc = make_act_map(&tmQ, Q, d->N, d->H, d->W, cq, 1, WG_TILE, WG_TILE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
     if (rc) return rc;
     const size_t smem = p.stages * stage_bytes + 2048 + 1024;
-    const int gx = max(1, min(p.num_tiles, SCI_NUM_SMS));
     if (env_int("SCI_CONV_VERBOSE", 0))
         fprintf(stderr, "wgrad v3 plan: %dx%d Cin %d Cout %d stride 1 | p_is_dz %d cp %d cq %d stages %d grid %d tiles %d\n", d->H, d->W,
                 d->Cin, d->Cout, p.p_is_dz, cp, cq, p.stages, gx, p.num_tiles);
-    return launch(conv_wgrad3_tc_kernel, dim3(gx), TC_THREADS, smem, stream, false, "conv tc wgrad v3", tmP, tmQ, p);
+    if (d->workspace) {
+        p.dw = static_cast<float*>(d->workspace);
+        rc = launch(conv_wgrad3_tc_kernel<true>, dim3(gx), TC_THREADS, smem, stream, false, "conv tc wgrad v3", tmP, tmQ, p);
+        return rc ? rc : sci_ordered_slot_sum(p.dw, gx, 9L * p.Cout * p.Cin, 9L * p.Cout * p.Cin, d->dw, nullptr, stream);
+    }
+    return launch(conv_wgrad3_tc_kernel<false>, dim3(gx), TC_THREADS, smem, stream, false, "conv tc wgrad v3", tmP, tmQ, p);
 }
 
 int check_conv_desc(const sci_conv_desc* d) {
@@ -1857,20 +1924,43 @@ int check_conv_desc(const sci_conv_desc* d) {
 
 extern "C" int sci_conv_tc_available(void) { return 1; }
 
+extern "C" size_t sci_conv3x3_fwd_workspace_bytes(const sci_conv_desc* d, int impl) {
+    if (!d || impl != SCI_CONV_TC || !d->mask_y || !d->col_s1 || check_conv_desc(d) || !fwd2_eligible(d)) return 0;
+    const int halves = d->Cout <= 128 ? 1 : 2;
+    int grid = 0;
+    if (conv_fwd2_tc_launch(d, nullptr, 0, halves == 1 ? d->Cout : 128, nullptr, &grid, true)) return 0;
+    const int ncol = d->pixel_shuffle ? d->Cout / 4 : d->Cout;
+    return (size_t)halves * grid * 2 * ncol * sizeof(float);
+}
+
 extern "C" int sci_conv3x3_fwd(const sci_conv_desc* d, int impl, void* stream) {
     int rc = check_conv_desc(d);
     if (rc) return rc;
+    size_t need = 0;
+    if (d->workspace || d->workspace_bytes) {
+        need = sci_conv3x3_fwd_workspace_bytes(d, impl);
+        SCI_REQUIRE(d->workspace && d->workspace_bytes >= need, "conv ordered column sums: workspace missing or too small");
+        SCI_REQUIRE(((uintptr_t)d->workspace & 15) == 0, "conv ordered column sums: workspace must be 16-byte aligned");
+    }
     if (impl == SCI_CONV_REF) {
         SCI_REQUIRE(!d->w_split && !d->emit_lo && !d->planar_out && !d->half_io, "conv ref: w_split / emit_lo / planar_out / half_io are tensor-core options");
         return sci_conv3x3_ref_launch(d, stream);
     }
     if (impl == SCI_CONV_TC) {
         if (!fwd2_eligible(d)) return conv_fwd_tc_launch(d, stream);
-        if (d->Cout <= 128) return conv_fwd2_tc_launch(d, stream, 0, d->Cout);
-        // 256 columns: two passes of 128 (PixelShuffle layers: the two output-row parities); the activation rows are
-        // fetched twice, the tensor-core work is unchanged
-        rc = conv_fwd2_tc_launch(d, stream, 0, 128);
-        return rc ? rc : conv_fwd2_tc_launch(d, stream, 128, 128);
+        float* ord = need ? static_cast<float*>(d->workspace) : nullptr;
+        const int ncol = d->pixel_shuffle ? d->Cout / 4 : d->Cout;       // stored channels: the column sums' width
+        int grid = 0;
+        if (d->Cout <= 128) {
+            rc = conv_fwd2_tc_launch(d, stream, 0, d->Cout, ord, &grid);
+        } else {
+            // 256 columns: two passes of 128 (PixelShuffle layers: the two output-row parities); the activation rows are
+            // fetched twice, the tensor-core work is unchanged.  Ordered sums: the second pass has the slots after the first's
+            rc = conv_fwd2_tc_launch(d, stream, 0, 128, ord, &grid);
+            if (!rc) rc = conv_fwd2_tc_launch(d, stream, 128, 128, ord ? ord + (size_t)grid * 2 * ncol : nullptr);
+        }
+        if (rc || !ord) return rc;
+        return sci_ordered_slot_sum(ord, (d->Cout <= 128 ? 1 : 2) * grid, 2L * ncol, ncol, d->col_s1, d->col_s2, stream);
     }
     return sci_fail(SCI_EINVAL, "conv: unknown impl");
 }
@@ -1879,17 +1969,40 @@ extern "C" int sci_conv3x3_dgrad(const sci_conv_desc* d, int impl, void* stream)
     return sci_conv3x3_fwd(d, impl, stream);
 }
 
-extern "C" int sci_conv3x3_wgrad(const sci_wgrad_desc* d, int impl, void* stream) {
+static int check_wgrad_desc(const sci_wgrad_desc* d, int impl) {
     SCI_REQUIRE(d && d->x && d->dz && d->dw, "wgrad: null pointer");
     SCI_REQUIRE(d->N > 0 && d->H > 0 && d->W > 0 && d->Cin > 0 && d->Cout > 0 && (d->stride == 1 || d->stride == 2),
                 "wgrad: shape");
     SCI_REQUIRE(d->Cin % 4 == 0 && d->Cout % 4 == 0, "wgrad: channels % 4");
-    if (impl == SCI_CONV_REF) return sci_wgrad_ref_launch(d, stream);
-    if (impl == SCI_CONV_TC) {
-        if (d->Cin % 32 != 0 || d->Cout % 32 != 0 || d->Cin > 128 || d->Cout > 256)
-            return sci_fail(SCI_EUNSUPPORTED, "wgrad tc: needs Cin % 32 == 0 (<= 128), Cout % 32 == 0 (<= 256)");
-        if (wgrad3_eligible(d)) return conv_wgrad3_tc_launch(d, stream);
-        return conv_wgrad2_tc_launch(d, stream);
+    if (impl == SCI_CONV_TC && (d->Cin % 32 != 0 || d->Cout % 32 != 0 || d->Cin > 128 || d->Cout > 256))
+        return sci_fail(SCI_EUNSUPPORTED, "wgrad tc: needs Cin % 32 == 0 (<= 128), Cout % 32 == 0 (<= 256)");
+    if (impl != SCI_CONV_TC && impl != SCI_CONV_REF) return sci_fail(SCI_EINVAL, "wgrad: unknown impl");
+    return SCI_OK;
+}
+
+// CTA columns of the weight-gradient launch = slots of its ordered form (0: the descriptor is rejected)
+static int wgrad_slots(const sci_wgrad_desc* d, int impl) {
+    if (check_wgrad_desc(d, impl)) return 0;
+    if (impl == SCI_CONV_REF) return sci_wgrad_ref_slots(d);
+    int slots = 0;
+    const int rc = wgrad3_eligible(d) ? conv_wgrad3_tc_launch(d, nullptr, &slots) : conv_wgrad2_tc_launch(d, nullptr, &slots);
+    return rc ? 0 : slots;
+}
+
+extern "C" size_t sci_conv3x3_wgrad_workspace_bytes(const sci_wgrad_desc* d, int impl) {
+    const int slots = wgrad_slots(d, impl);
+    return slots ? (size_t)slots * 9 * (size_t)d->Cout * (size_t)d->Cin * sizeof(float) : 0;
+}
+
+extern "C" int sci_conv3x3_wgrad(const sci_wgrad_desc* d, int impl, void* stream) {
+    int rc = check_wgrad_desc(d, impl);
+    if (rc) return rc;
+    if (d->workspace || d->workspace_bytes) {
+        const size_t need = sci_conv3x3_wgrad_workspace_bytes(d, impl);
+        SCI_REQUIRE(d->workspace && d->workspace_bytes >= need, "wgrad ordered: workspace missing or too small");
+        SCI_REQUIRE(((uintptr_t)d->workspace & 15) == 0, "wgrad ordered: workspace must be 16-byte aligned");
     }
-    return sci_fail(SCI_EINVAL, "wgrad: unknown impl");
+    if (impl == SCI_CONV_REF) return sci_wgrad_ref_launch(d, stream);
+    if (wgrad3_eligible(d)) return conv_wgrad3_tc_launch(d, stream);
+    return conv_wgrad2_tc_launch(d, stream);
 }

@@ -107,6 +107,9 @@ __global__ void bn_fold_kernel(const float* __restrict__ gamma, const float* __r
 }
 
 // dz = dy * (y > 0); s1[c] += sum dz; s2[c] += sum dz*y.   blockDim = (C, rows)
+// ORDERED: the block's sums are stored, not added: s1 / s2 point at column 0 of slot 0 of a [grid][2][C] workspace
+// (sci_act_bwd_ordered), block b writes slot b, and sci_ordered_slot_sum adds the slots in slot order.
+template <bool ORDERED>
 __global__ void act_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ y, float* __restrict__ dz,
                                long n_pix, int C, int relu, float* __restrict__ s1, float* __restrict__ s2) {
     extern __shared__ float sm[];
@@ -125,10 +128,54 @@ __global__ void act_bwd_kernel(const float* __restrict__ dy, const float* __rest
         __syncthreads();
         if (row == 0) {
             for (int r = 1; r < rows; ++r) { a1 += sm[(r * C + c) * 2]; a2 += sm[(r * C + c) * 2 + 1]; }
-            if (s1) atomicAdd(s1 + c, a1);
-            if (s2) atomicAdd(s2 + c, a2);
+            if (ORDERED) {
+                const long o = (long)blockIdx.x * 2 * C + c;
+                if (s1) s1[o] = a1;
+                if (s2) s2[o] = a2;
+            } else {
+                if (s1) atomicAdd(s1 + c, a1);
+                if (s2) atomicAdd(s2 + c, a2);
+            }
         }
     }
+}
+
+// out0[i] = out0[i] + (((part[0][i] + part[1][i]) + part[2][i]) + ...), strictly in slot order, for i < n; out1 likewise over
+// part[b][n + i].  part holds `slots` slots of `width` floats.  blockIdx.y selects the output (NULL outputs are skipped).
+// The adds of one output form a chain, so what costs is waiting for its loads: G lanes serve one output, lane j loads slots
+// j, j + G, j + 2G, ... (G * K slots in flight per output), and every lane of the group adds the values, broadcast by
+// shuffles, in slot order (the group's first lane stores).  G = 32 for few outputs over many slots (column sums: up to
+// 2 x 1024 outputs, up to 1184 slots); G = 1 for weight gradients (10^4..10^5 outputs, 24..296 slots), where there are
+// threads enough and the shuffles would only add instructions.
+template <int G>
+__global__ void __launch_bounds__(256) ordered_slot_sum_kernel(const float* __restrict__ part, int slots, long width, long n,
+                                                               float* __restrict__ out0, float* __restrict__ out1) {
+    constexpr int K = 16;                                  // slots per lane and chunk: a chunk is G * K slots
+    const long i = ((long)blockIdx.x * blockDim.x + threadIdx.x) / G;
+    const int lane = threadIdx.x % G;
+    float* out = blockIdx.y ? out1 : out0;
+    const bool active = out != nullptr && i < n;
+    const float* pp = part + (blockIdx.y ? n : 0) + (active ? i : 0);
+    float s = 0.f;
+    for (int b0 = 0; b0 < slots; b0 += G * K) {
+        float t[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const int b = b0 + k * G + lane;
+            t[k] = (active && b < slots) ? pp[(long)b * width] : 0.f;
+        }
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+#pragma unroll
+            for (int j = 0; j < G; ++j) {
+                const float v = G == 1 ? t[k] : __shfl_sync(0xffffffffu, t[k], j, G);
+                const int b = b0 + k * G + j;
+                if (b == 0) s = v;
+                else if (b < slots) s += v;
+            }
+        }
+    }
+    if (active && lane == 0) out[i] = out[i] + s;
 }
 
 __global__ void bn_param_grad_kernel(const float* __restrict__ s1, const float* __restrict__ s2,
@@ -704,17 +751,59 @@ extern "C" int sci_bn_fold(const float* gamma, const float* beta, const float* m
     return SCI_OK;
 }
 
+int sci_ordered_slot_sum(const float* part, int slots, long width, long n, float* out0, float* out1, void* stream) {
+    if (!out0 && !out1) return SCI_OK;
+    const dim3 block(256);
+    if (n <= 2048)
+        ordered_slot_sum_kernel<32><<<dim3(grid1d(32 * n), out1 ? 2 : 1), block, 0, sci_stream(stream)>>>(part, slots, width, n,
+                                                                                                          out0, out1);
+    else
+        ordered_slot_sum_kernel<1><<<dim3(grid1d(n), out1 ? 2 : 1), block, 0, sci_stream(stream)>>>(part, slots, width, n, out0,
+                                                                                                    out1);
+    SCI_CHECK_LAUNCH("ordered slot sum");
+    return SCI_OK;
+}
+
+namespace {
+// launch shape of act_bwd_kernel: blocks of (C, rows) threads, at most 8 per SM
+int act_bwd_rows(int C) { return max(1, 256 / C); }
+int act_bwd_grid(long n_pix, int C) { return (int)min((long)SCI_NUM_SMS * 8, (n_pix + act_bwd_rows(C) - 1) / act_bwd_rows(C)); }
+
+int act_bwd_launch(bool ordered, const float* dy, const float* y, float* dz, long n_pix, int C, int relu, float* s1, float* s2,
+                   void* stream) {
+    const int rows = act_bwd_rows(C);
+    const dim3 block(C, rows);
+    const int grid = act_bwd_grid(n_pix, C);
+    const size_t smem = (size_t)rows * C * 2 * sizeof(float);
+    (ordered ? act_bwd_kernel<true> : act_bwd_kernel<false>)<<<grid, block, smem, sci_stream(stream)>>>(dy, y, dz, n_pix, C,
+                                                                                                         relu, s1, s2);
+    SCI_CHECK_LAUNCH("act_bwd");
+    return SCI_OK;
+}
+}  // namespace
+
 extern "C" int sci_act_bwd(const float* dy, const float* y, float* dz, long n_pix, int C, int relu, float* s1, float* s2,
                            void* stream) {
     SCI_REQUIRE(dy && dz && n_pix > 0 && C > 0 && C <= 1024, "act_bwd");
     SCI_REQUIRE(!(relu || s2) || y, "act_bwd: y needed for relu / s2");
-    const int rows = max(1, 256 / C);
-    const dim3 block(C, rows);
-    const int grid = (int)min((long)SCI_NUM_SMS * 8, (n_pix + rows - 1) / rows);
-    const size_t smem = (size_t)rows * C * 2 * sizeof(float);
-    act_bwd_kernel<<<grid, block, smem, sci_stream(stream)>>>(dy, y, dz, n_pix, C, relu, s1, s2);
-    SCI_CHECK_LAUNCH("act_bwd");
-    return SCI_OK;
+    return act_bwd_launch(false, dy, y, dz, n_pix, C, relu, s1, s2, stream);
+}
+
+extern "C" size_t sci_act_bwd_workspace_bytes(long n_pix, int C) {
+    if (n_pix <= 0 || C <= 0 || C > 1024) return 0;
+    return (size_t)act_bwd_grid(n_pix, C) * 2 * C * sizeof(float);
+}
+
+extern "C" int sci_act_bwd_ordered(const float* dy, const float* y, float* dz, long n_pix, int C, int relu, float* s1,
+                                   float* s2, void* workspace, size_t workspace_bytes, void* stream) {
+    SCI_REQUIRE(dy && dz && n_pix > 0 && C > 0 && C <= 1024, "act_bwd");
+    SCI_REQUIRE(!(relu || s2) || y, "act_bwd: y needed for relu / s2");
+    SCI_REQUIRE(workspace && workspace_bytes >= sci_act_bwd_workspace_bytes(n_pix, C), "act_bwd ordered: workspace missing or too small");
+    SCI_REQUIRE(((uintptr_t)workspace & 15) == 0, "act_bwd ordered: workspace must be 16-byte aligned");
+    float* ws = static_cast<float*>(workspace);
+    int rc = act_bwd_launch(true, dy, y, dz, n_pix, C, relu, s1 ? ws : nullptr, s2 ? ws + C : nullptr, stream);
+    if (rc) return rc;
+    return sci_ordered_slot_sum(ws, act_bwd_grid(n_pix, C), 2L * C, C, s1, s2, stream);
 }
 
 extern "C" int sci_bn_param_grad(const float* s1, const float* s2, const float* gamma, const float* beta, float* dgamma,

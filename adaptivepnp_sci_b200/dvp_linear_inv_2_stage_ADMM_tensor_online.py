@@ -326,6 +326,12 @@ def twoStageAdmm_denoise_bayer(y_bayer, Phi_bayer, _lambda=1, gamma=0.01,
     iteration, PSNR sums and the fine-tune gradients are all-reduced, and the returned arrays are the full frame (gathered
     on every rank).  The closed-form demosaic is pixel-wise and needs no halo.  DDnet needs strips and a width that are
     multiples of 8, and strips of at least 88 rows over several ranks (ValueError otherwise).
+
+    Reproducibility: the fine-tune's backward reductions (weight gradients, bias / BatchNorm column sums) run in a fixed
+    order, so the same inputs, the same numpy / torch seeds (``utilspy.worker_init_fn``), the same GPU model and the same
+    world size and transport give bit-identical reconstructions (``xbgr3``, ``x_bayer`` / ``theta``) and bit-identical fine-tuned weights.  Not covered: NCCL's
+    all-reduce in ``grad_sync`` (its algorithm choice; gloo is deterministic), DDnet's self-supervised update (never
+    run by the solvers), and the printed fp64 diagnostics (PSNR, SSIM, losses), which may vary at ~1e-16 relative.
     """
     name = denoiser if denoiser == 'tv' else str(denoiser).lower()
     if name not in ('tv', 'ffdnet_color', 'fastdvd_color'):
@@ -461,6 +467,12 @@ def twoStageAdmm_denoise_gray(y, Phi, denoiser='ffdnet_gray', iter_max=50, sigma
     against the derived oracles (``oracle.admm.twoStageAdmm_denoise_gray`` for 'ffdnet_gray',
     ``oracle.gray_fastdvd.twoStageAdmm_denoise_gray`` for 'fastdvd_gray') and reported as "parity vs derived oracle".
     'fastdvd_gray' needs H and W multiples of 4 (ValueError before any GPU work).
+
+    Reproducibility: the fine-tune's backward reductions (weight gradients, bias / BatchNorm column sums) run in a fixed
+    order, so the same inputs, the same numpy / torch seeds (``utilspy.worker_init_fn``), the same GPU model and the same
+    world size and transport give bit-identical reconstructions (``xhat``, ``theta``) and bit-identical fine-tuned weights.  Not covered: NCCL's
+    all-reduce in ``grad_sync`` (its algorithm choice; gloo is deterministic), DDnet's self-supervised update (never
+    run by the solvers), and the printed fp64 diagnostics (PSNR, SSIM, losses), which may vary at ~1e-16 relative.
 
     y [H,W], Phi [H,W,B], x0 [H,W,B] (warm start) -> (xhat_np[H,W,B], theta_np[H,W,B], psnr_, ssim_, psnr_all, model)."""
     name = str(denoiser).lower()

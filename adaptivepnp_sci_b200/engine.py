@@ -37,13 +37,15 @@ class ConvDesc(ctypes.Structure):
                 ("planar_in1", _f32p), ("planar_out", _f32p), ("pdl", ctypes.c_int),
                 ("half_io", ctypes.c_int), ("Cin_store", ctypes.c_int), ("Cout_store", ctypes.c_int),
                 ("mask_y", _f32p), ("col_s1", _f32p), ("col_s2", _f32p), ("mask_relu", ctypes.c_int), ("lo_channel0", ctypes.c_int),
-                ("K_used", ctypes.c_int), ("planar_planes", ctypes.c_int)]
+                ("K_used", ctypes.c_int), ("planar_planes", ctypes.c_int), ("workspace", ctypes.c_void_p),
+                ("workspace_bytes", ctypes.c_size_t)]
 
 
 class WgradDesc(ctypes.Structure):
     _fields_ = [("x", _f32p), ("dz", _f32p), ("oscale", _f32p), ("dw", _f32p),
                 ("N", ctypes.c_int), ("H", ctypes.c_int), ("W", ctypes.c_int), ("Cin", ctypes.c_int),
-                ("Cout", ctypes.c_int), ("stride", ctypes.c_int)]
+                ("Cout", ctypes.c_int), ("stride", ctypes.c_int), ("workspace", ctypes.c_void_p),
+                ("workspace_bytes", ctypes.c_size_t)]
 
 
 class LayerOp(ctypes.Structure):
@@ -281,6 +283,7 @@ class _EngineBase:
         self._tables = None
         self.s12_flat = None
         self.pdl_chain = False   # True inside an inference chain: weights are packed, consecutive convs may overlap (PDL)
+        self.red_buf = None      # scratch of the fixed-order reductions of the backward pass (grown on demand, see _red_ws)
         self.profile = None      # set to a list to record (start_event, end_event, algorithmic_flops, tag) per conv launch
 
     # ---- parameter state ------------------------------------------------------------------------------
@@ -351,6 +354,22 @@ class _EngineBase:
         self._table("grads").run()
         self.n_launch += 1
 
+    def _red_ws(self, nbytes, device):
+        """Scratch for the fixed-order (bit-reproducible) reductions of one backward call: each CTA stores its partial
+        weight gradient / column sums into its own slot, a second kernel adds the slots in slot order.  One buffer serves
+        every call of the stream in turn; it grows to the largest need seen (the widest layer's slots, 29 MB for the
+        128->128 FastDVDnet layers at 8x512x512), so nothing is allocated in steady state."""
+        if self.red_buf is None or self.red_buf.numel() < nbytes:
+            self.red_buf = torch.empty(nbytes, dtype=torch.uint8, device=device)
+        return self.red_buf.data_ptr()
+
+    def _ordered(self, d, query, dev):
+        """Give descriptor d (ConvDesc / WgradDesc) the reduction workspace its call needs (none: left NULL)."""
+        need = getattr(_lib.lib, query)(ctypes.byref(d), self.impl)
+        if need:
+            d.workspace = self._red_ws(need, dev)
+            d.workspace_bytes = need
+
     # ---- kernel wrappers ------------------------------------------------------------------------------
     def conv(self, L, x, N, H, W, y, residual=None, round_out=True, emit_lo=False, planar=None):
         """planar = (in1, out) planar [N,P,H,W] tensors (P = 3, or 1 for gray frames): tensor-core path only, fused
@@ -412,6 +431,8 @@ class _EngineBase:
         d = ConvDesc(_dp(dz), _dp(L.wpk_t), None, None, _dp(residual), _dp(dx), N, Ho, Wo, L.Co_pad, 4 * L.Ci_pad, 1, 0, 1,
                      int(self.tf32), 0, 0)
         self._mask_args(d, mask)
+        if mask is not None:
+            self._ordered(d, "sci_conv3x3_fwd_workspace_bytes", dz.device)
         call("sci_conv3x3_dgrad", ctypes.byref(d), self.impl, stream())
         self.n_launch += 1
 
@@ -420,22 +441,32 @@ class _EngineBase:
         d = ConvDesc(_dp(dz), _dp(L.wpk_t), None, None, _dp(residual), _dp(dx), N, Ho, Wo, L.Co_pad, L.Ci_pad, 1, 0, 0,
                      int(self.tf32), 0, 0)
         self._mask_args(d, mask)
+        if mask is not None:
+            self._ordered(d, "sci_conv3x3_fwd_workspace_bytes", dz.device)
         call("sci_conv3x3_dgrad", ctypes.byref(d), self.impl, stream())
         self.n_launch += 1
 
     def wgrad(self, L, x, dz, N, H, W):
+        """L.dwpk += packed weight gradient, reduced over the CTAs in a fixed order (bit-identical on every run)."""
         d = WgradDesc(_dp(x), _dp(dz), _dp(L.scale), _dp(L.dwpk), N, H, W, L.Ci_pad, L.Co_pad, L.stride)
+        self._ordered(d, "sci_conv3x3_wgrad_workspace_bytes", dz.device)
         call("sci_conv3x3_wgrad", ctypes.byref(d), self.impl, stream())
-        self.n_launch += 1
+        self.n_launch += 2
 
     def act_bwd(self, L, dy, y, n_pix, C):
-        """dz (in place over dy) = dy * relu'(y); accumulates the per-column sums needed for bias / BN grads."""
+        """dz (in place over dy) = dy * relu'(y); accumulates the per-column sums needed for bias / BN grads (fixed order)."""
         need = L.has_affine
         if not (L.relu or need):
             return dy
-        call("sci_act_bwd", ptr(dy), ptr(y) if (L.relu or L.bn is not None) else None, ptr(dy), n_pix, C, int(L.relu),
-             ptr(L.s1) if need else None, ptr(L.s2) if (need and L.bn is not None) else None, stream())
-        self.n_launch += 1
+        yp = ptr(y) if (L.relu or L.bn is not None) else None
+        if not need:
+            call("sci_act_bwd", ptr(dy), yp, ptr(dy), n_pix, C, int(L.relu), None, None, stream())
+            self.n_launch += 1
+            return dy
+        nb = _lib.lib.sci_act_bwd_workspace_bytes(n_pix, C)
+        call("sci_act_bwd_ordered", ptr(dy), yp, ptr(dy), n_pix, C, int(L.relu), ptr(L.s1),
+             ptr(L.s2) if L.bn is not None else None, self._red_ws(nb, dy.device), nb, stream())
+        self.n_launch += 2
         return dy
 
     def after_step(self):

@@ -329,7 +329,13 @@ def fastdvdnet_seqdenoise(seq, noise_std, windsize, model, train=None):
 def fastdvdnet_denoiser_full_tensor_v2(vnoisy, sigma, y_bayer=None, Phi=None, model=None,
                                        useGPU=True, lr_=0.000001, updata_=False, update_per_iter=1, gray=False,
                                        update_times=-1):
-    """vnoisy [H,W,3,B] CUDA, y_bayer [h,w,4], Phi [h,w,B,4] -> outv [H,W,3,B] (or ``(outv, model)``)."""
+    """vnoisy [H,W,3,B] CUDA, y_bayer [h,w,4], Phi [h,w,B,4] -> outv [H,W,3,B] (or ``(outv, model)``).
+
+    Reproducibility: the fine-tune's backward reductions (weight gradients, bias / BatchNorm column sums) run in a fixed
+    order, so the same inputs, the same numpy / torch seeds (``utilspy.worker_init_fn``), the same GPU model and the same
+    world size and transport give bit-identical outputs and bit-identical fine-tuned weights.  Not covered: NCCL's
+    all-reduce in ``grad_sync`` (its algorithm choice; gloo is deterministic), DDnet's self-supervised update (never
+    run by the solvers), and the printed fp64 diagnostics (PSNR, SSIM, losses), which may vary at ~1e-16 relative."""
     from .utils_image import fourCh2OneCh
     if gray:
         raise NotImplementedError("the full-tensor adapter serves the Bayer solvers (colour cube [H,W,3,B]); the gray model "

@@ -82,7 +82,13 @@ def denoise_planar(u, pb, sigma, model, lr, do_update, update_per_iter, grad_syn
 def ffdnet_rgb_denoise_full_tensor(x, yall, Phiall, sigma, model, useGPU=True, lr_=0.000001, updata_=False,
                                    update_per_iter=4, device=0):
     """x [H,W,3,B] CUDA, yall [h,w,4], Phiall [h,w,B,4], sigma float -> outv [H,W,3,B]
-    (or ``(outv, model)`` when ``updata_``), exactly the reference's convention (:356-359)."""
+    (or ``(outv, model)`` when ``updata_``), exactly the reference's convention (:356-359).
+
+    Reproducibility: the fine-tune's backward reductions (weight gradients, bias / BatchNorm column sums) run in a fixed
+    order, so the same inputs, the same numpy / torch seeds (``utilspy.worker_init_fn``), the same GPU model and the same
+    world size and transport give bit-identical outputs and bit-identical fine-tuned weights.  Not covered: NCCL's
+    all-reduce in ``grad_sync`` (its algorithm choice; gloo is deterministic), DDnet's self-supervised update (never
+    run by the solvers), and the printed fp64 diagnostics (PSNR, SSIM, losses), which may vary at ~1e-16 relative."""
     from .utils_image import fourCh2OneCh
     x = x.contiguous().float()
     H, W, _, B = x.shape

@@ -273,6 +273,12 @@ typedef struct sci_conv_desc {
     int planar_planes;      /* TC only, with planar_out: planes P per frame of planar_in1 / planar_out, 3 (colour) or 1 (the
                                gray FastDVDnet: columns 1 and 2 of the layer, all-zero weights in the colour-shaped embedding,
                                are not written).  0 = 3 */
+    void* workspace;        /* with mask_y and col_s1: NULL = the column sums are added with atomics (their low bits depend on
+                               the order in which CTAs finish); non-NULL = FIXED-ORDER column sums, bit-identical on every run:
+                               each CTA stores its sums (epilogue warps added in warp order) into its own slot of this
+                               workspace, and a second kernel of the same call adds the slots in slot order into col_s1 /
+                               col_s2.  Size: sci_conv3x3_fwd_workspace_bytes (SCI_EINVAL when smaller).  16-byte aligned */
+    size_t workspace_bytes;
 } sci_conv_desc;
 
 /* 1 if this build contains the tcgen05 tensor-core convolution kernels. */
@@ -281,6 +287,11 @@ int sci_conv_tc_available(void);
  * of a stride-1 layer is the same call with weights packed in transposed+flipped form. */
 int sci_conv3x3_fwd(const sci_conv_desc* d, int impl, void* stream);
 int sci_conv3x3_dgrad(const sci_conv_desc* d, int impl, void* stream);
+/* Bytes of sci_conv_desc.workspace the fixed-order column sums of this call need with this impl: 0 unless the call is a
+ * fused data gradient (mask_y) with column sums (col_s1) on the tensor-core path.  Otherwise slots x 2 x C x 4, C = the
+ * stored output channels (Cout, Cout/4 with pixel_shuffle), one slot [col_s1 part | col_s2 part] per CTA of each launch
+ * (a 256-column layer runs as two launches of the same grid).  Host arithmetic only. */
+size_t sci_conv3x3_fwd_workspace_bytes(const sci_conv_desc* d, int impl);
 
 typedef struct sci_wgrad_desc {
     const float* x;         /* layer input  [N][H][W][Cin]                          */
@@ -288,9 +299,19 @@ typedef struct sci_wgrad_desc {
     const float* oscale;    /* per output column scale (folded BN), NULL = 1        */
     float* dw;              /* packed weight gradient [9][Cout][Cin], ACCUMULATED   */
     int N, H, W, Cin, Cout, stride;
+    void* workspace;        /* NULL = every CTA adds its partial gradient into dw with atomics (low bits depend on the order
+                               in which CTAs finish); non-NULL = FIXED ORDER, bit-identical on every run: CTA column b stores
+                               its scaled partial into slot b (a [9][Cout][Cin] block) of this workspace, and a second kernel
+                               of the same call computes dw[i] = dw[i] + (((slot0[i] + slot1[i]) + slot2[i]) + ...).  Size:
+                               sci_conv3x3_wgrad_workspace_bytes (SCI_EINVAL when smaller).  16-byte aligned */
+    size_t workspace_bytes;
 } sci_wgrad_desc;
 /* dw[tap][co][ci] += oscale[co] * sum_{n,ho,wo} dz[n,ho,wo,co] * x[n, ho*s+r-1, wo*s+q-1, ci] */
 int sci_conv3x3_wgrad(const sci_wgrad_desc* d, int impl, void* stream);
+/* Bytes of sci_wgrad_desc.workspace for this impl: slots x 9 x Cout x Cin x 4, slots = the CTA columns of the launch (a
+ * function of the shape only: tensor-core v3 min(tiles, 148), v2 min(tiles, 148 / (3 m_tiles)), fp32 reference its pixel
+ * chunks).  0 for a descriptor the impl rejects.  Host arithmetic only. */
+size_t sci_conv3x3_wgrad_workspace_bytes(const sci_wgrad_desc* d, int impl);
 
 /* PyTorch weight [Co][Ci/groups][3][3] -> packed [9][Co_pad][Ci_pad] (zero padded; grouped convs become
  * block-diagonal; ps != 0 permutes output columns for PixelShuffle(2): column q*(Co/4)+c <- channel c*4+q).
@@ -351,6 +372,13 @@ int sci_bn_fold(const float* gamma, const float* beta, const float* mean, const 
  * s1[c] += sum dz, s2[c] += sum dz*y  (either may be NULL).  n_pix pixels of C channels (NHWC). */
 int sci_act_bwd(const float* dy, const float* y, float* dz, long n_pix, int C, int relu, float* s1, float* s2,
                 void* stream);
+/* The same with FIXED-ORDER column sums (bit-identical on every run; dz is the same as sci_act_bwd's): block b stores its
+ * (s1, s2) partials into slot b = [C floats of s1 | C floats of s2] of the workspace, a second kernel adds the slots in slot
+ * order into s1 / s2.  workspace: sci_act_bwd_workspace_bytes(n_pix, C) bytes, 16-byte aligned; missing or smaller ->
+ * SCI_EINVAL before any launch. */
+size_t sci_act_bwd_workspace_bytes(long n_pix, int C);
+int sci_act_bwd_ordered(const float* dy, const float* y, float* dz, long n_pix, int C, int relu, float* s1, float* s2,
+                        void* workspace, size_t workspace_bytes, void* stream);
 /* BatchNorm affine gradients from the two sums: dbeta = s1, dgamma = (s2 - beta*s1)/gamma (0 where gamma == 0). */
 int sci_bn_param_grad(const float* s1, const float* s2, const float* gamma, const float* beta, float* dgamma,
                       float* dbeta, int C, void* stream);
